@@ -1,7 +1,7 @@
 # Builds the product library (CUDA, sm_100a only) and the test-only artefacts.
 #   make lib       -> libgoldilocks_b200/libgoldilocks_b200.so   (the C ABI of include/goldilocks_b200.h)
 #   make hostsim   -> tests/hostsim/_hostsim.so                  (device math compiled for the host; tests only)
-#   make oracle    -> oracle/liboracle.so (+ oracle/_ref/*.so when /root/reference is present; tests/bench baseline only)
+#   make oracle    -> oracle/liboracle.so (+ oracle/_ref/*.so with REF=<libgoldilocks source tree>; tests/bench baseline only)
 NVCC      ?= nvcc
 CXX       ?= g++
 ARCH      := -gencode arch=compute_100a,code=sm_100a

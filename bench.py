@@ -3,7 +3,7 @@
 configs ride along in `extra`: field / point ops (config 1), fixed-base comb (2), X448 (3), decaf + Elligator (5),
 sign, variable-base multiplications, and ONE batch sharded over all N GPUs by the library (`extra.strong`).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W]          our arm  (under torchrun for N > 1)
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]   our arm  (under torchrun for N > 1)
   python bench.py --impl reference [...]                        the reference's CPU path on all host cores
 
 A step = one pass of the hot path over one batch of 2^20 synthetic signatures per GPU.  Two multi-GPU readings:
@@ -32,6 +32,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -49,7 +50,9 @@ MAC32 = {"verify": 981120, "verify_finish": 800300, "x448": 870208, "comb": 1426
 METRIC = "Ed448 verifies/s at batch 2^20 per GPU (X448 and comb ops/s in extra)"
 UNIT = "verifies/s"
 DTYPE = "u32 limbs (448-bit integers)"
-CACHE = os.environ.get("GOLDILOCKS_B200_BENCH_CACHE", "/tmp/goldilocks_b200_bench_cache")
+# per user: on a shared machine another user's cache directory is not writable
+CACHE = os.environ.get("GOLDILOCKS_B200_BENCH_CACHE", os.path.join(tempfile.gettempdir(), "goldilocks_b200_bench_cache_%d" % os.getuid()))
+DUMP_BYTES = 64 << 20
 
 
 # ------------------------------------------------------------------------------------------------
@@ -399,6 +402,8 @@ def run_ours(args):
     launches = eng.launch_count() - l0
     clocks = sampler.stop()
     t_step = max_over_ranks(e0.elapsed_time(e1) / 1e3 / K)
+    if args.dump_outputs and rank == 0:
+        dump_output(args.dump_outputs, "verify_status", d_st.cpu().numpy())    # the legs below reuse d_st
     dominant = "SlotEdVerifyFinishShared" if "SlotEdVerifyFinishShared" in kavg else "SlotEdVerifyFinish"
     t_finish = kavg.get(dominant, 0.0) / 1e3
     # signatures whose key occurs at least twice in the batch go through the per-key tables (what the device-side grouping finds)
@@ -927,6 +932,17 @@ def strong_leg(lib, torch, world, n, corpus, peak, ops, reps):
     return out
 
 
+def dump_output(out_dir, name, a):
+    """<out_dir>/<name>.npy in float32 (statuses -1 / 0 are exact), at most DUMP_BYTES: a larger array keeps a sample
+    at sorted indices drawn with a fixed seed, the same for every build"""
+    os.makedirs(out_dir, exist_ok=True)
+    a = np.asarray(a).reshape(-1)
+    keep = DUMP_BYTES // 4 - 64
+    if a.size > keep:
+        a = a[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+    np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
+
+
 def emit(line):
     """the ONE JSON line on the real stdout (library banners are kept off it)"""
     os.write(_REAL_STDOUT, (json.dumps(line) + "\n").encode())
@@ -952,7 +968,11 @@ def main():
     ap.add_argument("--no-strong", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-peak", action="store_true", help="skip the on-box IMAD.WIDE peak measurement (use the committed figure)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps write the statuses of the last one (rank 0's batch) "
+                    "as DIR/verify_status.npy, float32, for comparing two builds on the same inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

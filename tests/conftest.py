@@ -27,7 +27,7 @@ def oracle():
 
 @pytest.fixture(scope="session")
 def ref():
-    """the unmodified reference compiled from /root/reference (oracle/_ref); skipped when not built"""
+    """the unmodified reference built by `make -C oracle ref REF=<its source tree>` (oracle/_ref); skipped when not built"""
     import util
     lib = util.ref_lib()
     if lib is None:

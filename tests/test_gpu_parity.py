@@ -69,6 +69,10 @@ def test_eddsa_vectors(gpu, vectors):
     parity.check_eddsa_vectors(gpu, vectors)
 
 
+def test_openssl_golden(gpu):
+    parity.check_openssl_golden(gpu, util.openssl_golden())
+
+
 def test_eddsa_random(gpu, chk):
     parity.check_eddsa_random(gpu, chk, 1 << 12)
 

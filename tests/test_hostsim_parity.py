@@ -79,6 +79,10 @@ def test_shake(sim):
     parity.check_shake(sim)
 
 
+def test_openssl_golden(sim):
+    parity.check_openssl_golden(sim, util.openssl_golden())
+
+
 def test_widened(sim, chk):
     parity.check_widened(sim, chk, 96)
 

@@ -30,7 +30,13 @@ def test_reference_build_reproduces_vectors(ref, vectors):
     parity.check_x448_vectors(ref, vectors, iters=1000)
 
 
-def test_oracle_vs_reference(oracle, ref):
+def test_oracle_vs_reference(oracle):
+    """the reference's Ed448 / X448 outputs stored as golden data always; everything else against the reference build
+    where it exists"""
+    parity.check_openssl_golden(oracle, util.openssl_golden())
+    ref = util.ref_lib()
+    if ref is None:
+        return
     t = os.cpu_count() or 1
     util.set_threads(oracle, t)
     util.set_threads(ref, t)

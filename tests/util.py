@@ -37,8 +37,8 @@ def oracle_lib():
 
 
 def ref_lib(arch="x86_64"):
-    build = ["make", "-C", "oracle", "ref"] if os.path.exists("/root/reference/src/goldilocks.c") else None
-    return _load("ref_" + arch, os.path.join(ROOT, "oracle", "_ref", "libgoldilocks_ref_%s.so" % arch), build)
+    """the original libgoldilocks as `make -C oracle ref REF=<its source tree>` built it; None when it was not built"""
+    return _load("ref_" + arch, os.path.join(ROOT, "oracle", "_ref", "libgoldilocks_ref_%s.so" % arch))
 
 
 def checker_lib():
@@ -60,6 +60,12 @@ def set_threads(lib, t):
 def golden_vectors():
     with open(os.path.join(ROOT, "tests", "golden", "reference_vectors.json")) as f:
         return json.load(f)
+
+
+def openssl_golden():
+    """Ed448 / X448 outputs of OpenSSL on seeded inputs (tools/openssl_vectors.py)"""
+    with np.load(os.path.join(ROOT, "tests", "golden", "openssl_ed448_x448.npz")) as z:
+        return {k: z[k] for k in z.files}
 
 
 def stream_bytes(label, n):

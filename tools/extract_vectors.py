@@ -1,8 +1,8 @@
 #!/usr/bin/env python3
 """Extracts the reference's own known-answer vectors into tests/golden/reference_vectors.json.
 
-Run in the build container only (reads /root/reference/test/*.inc.cxx, which does not exist on the
-GPU box).  The JSON it writes is committed; the tests read only the JSON.
+Usage: tools/extract_vectors.py <libgoldilocks source tree> (reads its test/*.inc.cxx).  The JSON it writes is
+committed; the tests read only the JSON.
 
 Sources (SURVEY.md section 8(c)):
   test/vectors.inc.cxx:3-29       RFC 7748 X448 iterated ladder after 1 / 1000 / 10^6 iterations
@@ -12,7 +12,9 @@ Sources (SURVEY.md section 8(c)):
 """
 import json, os, re, sys
 
-REF = sys.argv[1] if len(sys.argv) > 1 else "/root/reference"
+if len(sys.argv) != 2:
+    sys.exit(__doc__)
+REF = sys.argv[1]
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "tests", "golden", "reference_vectors.json")
 
 
