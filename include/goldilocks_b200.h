@@ -258,6 +258,21 @@ GOLDILOCKS_B200_API size_t goldilocks_b200_keyset_size(const goldilocks_b200_key
  * sets of up to 93 000 keys); larger sets keep the 41 KB per key layout (ten columns, forty doublings per signature).  0 = never flat. */
 GOLDILOCKS_B200_API void goldilocks_b200_keyset_policy(unsigned long long max_table_bytes);
 GOLDILOCKS_B200_API goldilocks_error_t goldilocks_ed448_verify_keyset_batch(goldilocks_error_t *status, const goldilocks_b200_keyset *keyset, const uint32_t *key_index /*n*/, const uint8_t *signature /*n*114*/, const uint8_t *msg, const size_t *msg_off /*n+1*/, uint8_t prehashed, const uint8_t *context, uint8_t context_len, size_t n);
+/* X448 peer sets (our extension; the 2014 API's "ECDH with a precomputed partner key", BASELINE.md section 1).  A caller whose
+ * fresh secret scalars keep meeting the same public u-coordinates -- HPKE / ECIES to a known recipient, onion packets to a fixed
+ * relay set -- builds a set of m peers once: each peer on the curve gets the reference's (5,5,18) comb table of a point that
+ * multiplies like u (15 KB per peer in HBM), and an X448 against it costs a comb instead of a ladder.  Any 56 bytes are accepted as
+ * a peer, exactly as goldilocks_x448 accepts them (u >= p is taken mod p; twist points, u = 0 and u = p - 1 keep the ladder).  out[i], status[i] are
+ * exactly what goldilocks_x448(out, peers[peer_index[i]], scalar + 56 i) returns; peer_index[i] >= m yields FAILURE and 56 zero
+ * bytes.  Constant time in the scalars; the peer indices are public.  The handle belongs to the CUDA device that was current at
+ * creation and is never sharded over goldilocks_b200_set_devices.  Order a batch by peer: the lanes of a
+ * warp then read one table (with many peers in random order goldilocks_x448_batch's ladder is faster; DESIGN.md decision 20). */
+typedef struct goldilocks_b200_x448_peerset_s goldilocks_b200_x448_peerset;
+GOLDILOCKS_B200_API goldilocks_error_t goldilocks_b200_x448_peerset_create(goldilocks_b200_x448_peerset **set, const uint8_t *peers /*m*56*/, size_t m);
+GOLDILOCKS_B200_API void goldilocks_b200_x448_peerset_destroy(goldilocks_b200_x448_peerset *set);
+GOLDILOCKS_B200_API size_t goldilocks_b200_x448_peerset_size(const goldilocks_b200_x448_peerset *set);
+GOLDILOCKS_B200_API goldilocks_error_t goldilocks_x448_peerset_batch(uint8_t *out /*n*56*/, goldilocks_error_t *status, const goldilocks_b200_x448_peerset *set,
+                                                                     const uint32_t *peer_index /*n*/, const uint8_t *scalar /*n*56*/, size_t n);
 /* Random-linear-combination batch verification (SURVEY 8(f)3; csrc/rlc.cuh): an OPTIONAL fast path for batches in which
  * (nearly) every signature is expected to be valid.  Same arguments and per-element statuses as
  * goldilocks_ed448_verify_batch (eddsa.c:253-306).  Signatures whose R or public key does not decode are rejected up
@@ -306,6 +321,8 @@ GOLDILOCKS_B200_API goldilocks_error_t goldilocks_ed448_verify_batch_dev(goldilo
  * synchronises `stream` (it needs the number of distinct keys and the verdict on the host) */
 GOLDILOCKS_B200_API goldilocks_error_t goldilocks_ed448_verify_rlc_batch_dev(goldilocks_error_t *status, const uint8_t *signature, const uint8_t *pubkey, const uint8_t *msg, const size_t *msg_off, uint8_t prehashed, const uint8_t *context /*device or NULL*/, uint8_t context_len, size_t n, void *stream, int *fast_path);
 GOLDILOCKS_B200_API goldilocks_error_t goldilocks_x448_batch_dev(uint8_t *out, goldilocks_error_t *status, const uint8_t *base, const uint8_t *scalar, size_t n, void *stream);
+GOLDILOCKS_B200_API goldilocks_error_t goldilocks_x448_peerset_batch_dev(uint8_t *out, goldilocks_error_t *status, const goldilocks_b200_x448_peerset *set,
+                                                                         const uint32_t *peer_index, const uint8_t *scalar, size_t n, void *stream);
 GOLDILOCKS_B200_API goldilocks_error_t goldilocks_448_precomputed_scalarmul_batch_dev(goldilocks_448_point_s *out, const goldilocks_448_scalar_s *scalar, size_t n, void *stream);
 GOLDILOCKS_B200_API goldilocks_error_t goldilocks_448_gf_mul_batch_dev(uint8_t *out, const uint8_t *a, const uint8_t *b, size_t n, void *stream);
 GOLDILOCKS_B200_API goldilocks_error_t goldilocks_448_point_add_batch_dev(goldilocks_448_point_s *out, const goldilocks_448_point_s *a, const goldilocks_448_point_s *b, size_t n, void *stream);

@@ -328,6 +328,30 @@ class BatchLib:
         self._call("goldilocks_ed448_verify_keyset_batch", st, handle, key_index, sig, arena, off, C.c_uint8(1 if prehashed else 0), ctx, C.c_uint8(ctx_len), _Z(len(sig)))
         return st
 
+    # ---- X448 peer sets: per-peer comb tables kept on the device across calls ----
+    def x448_peerset_create(self, peers):
+        """handle for m peer u-coordinates ((m,56) u8); free it with x448_peerset_destroy"""
+        peers = _u8(peers, 56)
+        h = C.c_void_p()
+        self._call("goldilocks_b200_x448_peerset_create", C.byref(h), peers, _Z(len(peers)))
+        return h
+
+    def x448_peerset_destroy(self, handle):
+        self.lib.goldilocks_b200_x448_peerset_destroy.restype = None
+        self.lib.goldilocks_b200_x448_peerset_destroy(handle)
+
+    def x448_peerset_size(self, handle):
+        f = self.lib.goldilocks_b200_x448_peerset_size
+        f.restype = _Z
+        return int(f(handle))
+
+    def x448_peerset(self, handle, peer_index, scalar):
+        """(out (n,56) u8, status int32[n]): X448 of scalar i against peer peer_index[i] of the set"""
+        scalar = _u8(scalar, 56); peer_index = np.ascontiguousarray(peer_index, np.uint32).reshape(-1)
+        out = np.empty_like(scalar); st = np.zeros(len(scalar), np.int32)
+        self._call("goldilocks_x448_peerset_batch", out, st, handle, peer_index, scalar, _Z(len(scalar)))
+        return out, st
+
     def ed448_verify(self, sig, pk, msgs, prehashed=False, context=b""):
         sig, pk = _u8(sig, 114), _u8(pk, 57)
         arena, off = pack_messages(msgs) if isinstance(msgs, list) else msgs

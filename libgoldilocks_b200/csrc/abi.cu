@@ -1581,6 +1581,65 @@ goldilocks_error_t goldilocks_ed448_verify_keyset_batch(goldilocks_error_t *stat
     return k.finish();
 }
 
+// ---- X448 peer sets: per-peer comb tables for key agreement with recurring public keys (slot_lanes.cuh SlotX448Peer) -------
+struct goldilocks_b200_x448_peerset_s {
+    int dev; size_t m;
+    uint8_t *peers;     /* m x 56 u bytes: what the ladder reads for the peers that keep it */
+    int32_t *table_ok;  /* per peer: SUCCESS = the comb table is valid (public) */
+    niels *tables;      /* m tables of COMB_ENTRIES affine niels, 15 360 bytes each */
+};
+goldilocks_error_t goldilocks_b200_x448_peerset_create(goldilocks_b200_x448_peerset **out, const uint8_t *peers, size_t m) {
+    if (!out) return GOLDILOCKS_FAILURE;
+    *out = nullptr;
+    Call k;
+    if (!k.ok) return k.finish();
+    const size_t mm = m ? m : 1;
+    goldilocks_b200_x448_peerset_s *ps = new goldilocks_b200_x448_peerset_s{k.c->dev, m, nullptr, nullptr, nullptr};
+    bool ok = m <= UINT32_MAX && cudaMalloc(&ps->peers, 56 * mm) == cudaSuccess && cudaMalloc(&ps->table_ok, sizeof(int32_t) * mm) == cudaSuccess &&
+              cudaMalloc(&ps->tables, mm * COMB_ENTRIES * sizeof(niels)) == cudaSuccess;
+    if (ok && m) {
+        ok = cudaMemcpyAsync(ps->peers, peers, 56 * m, cudaMemcpyHostToDevice, k.c->stream) == cudaSuccess;
+        abi_pt *pts = k.out<abi_pt>(m);
+        LaneX448PeerLift fl = {pts, ps->table_ok, ps->peers};
+        k.run(fl, m);
+        LanePrecompute fp = {k.out<abi_niels>(COMB_ENTRIES * m), pts, k.out<niels>(16 * COMB_N * m)};
+        k.run(fp, COMB_N * m);
+        LaneNielsFromAbi fc = {ps->tables, fp.tables};
+        k.run(fc, COMB_ENTRIES * m);
+    }
+    goldilocks_error_t r = k.finish();
+    if (!ok || r != GOLDILOCKS_SUCCESS) {
+        if (!ok) g_err = "goldilocks_b200_x448_peerset_create: device allocation or copy failed";
+        cudaFree(ps->peers); cudaFree(ps->table_ok); cudaFree(ps->tables);
+        delete ps;
+        return GOLDILOCKS_FAILURE;
+    }
+    *out = ps;
+    return GOLDILOCKS_SUCCESS;
+}
+void goldilocks_b200_x448_peerset_destroy(goldilocks_b200_x448_peerset *ps) {
+    if (!ps) return;
+    int cur = 0;
+    const bool sw = cudaGetDevice(&cur) == cudaSuccess && cur != ps->dev && cudaSetDevice(ps->dev) == cudaSuccess;
+    cudaFree(ps->peers); cudaFree(ps->table_ok); cudaFree(ps->tables);
+    if (sw) cudaSetDevice(cur);
+    delete ps;
+}
+size_t goldilocks_b200_x448_peerset_size(const goldilocks_b200_x448_peerset *ps) { return ps ? ps->m : 0; }
+goldilocks_error_t goldilocks_x448_peerset_batch(uint8_t *out, goldilocks_error_t *status, const goldilocks_b200_x448_peerset *ps, const uint32_t *peer_index,
+                                                 const uint8_t *scalar, size_t n) {
+    if (n == 0) return GOLDILOCKS_SUCCESS;
+    Call k;
+    if (!k.ok) return k.finish();
+    if (!ps || ps->dev != k.c->dev) { g_err = "goldilocks_x448_peerset_batch: the peer set lives on another device"; return GOLDILOCKS_FAILURE; }
+    SlotX448Peer f = {k.secret(k.out<uint8_t>(56 * n), 56 * n), k.out<int32_t>(n), ps->tables, ps->table_ok, ps->peers, k.in(peer_index, n),
+                      k.secret(k.in(scalar, 56 * n), 56 * n), (uint32_t)ps->m};
+    k.run_sm(f, n);
+    k.fetch(out, f.out, 56 * n);
+    k.fetch((int32_t *)status, f.status, n);
+    return k.finish();
+}
+
 // ---- device-resident variants -------------------------------------------------------------------------------
 goldilocks_error_t goldilocks_ed448_verify_batch_dev(goldilocks_error_t *status, const uint8_t *signature, const uint8_t *pubkey, const uint8_t *msg, const size_t *msg_off,
                                                      uint8_t prehashed, const uint8_t *context, uint8_t context_len, size_t n, void *scratch, void *stream) {
@@ -1600,6 +1659,15 @@ goldilocks_error_t goldilocks_x448_batch_dev(uint8_t *out, goldilocks_error_t *s
     Ctx *c = dev_ctx();
     if (!c) return GOLDILOCKS_FAILURE;
     SlotX448 f = {out, (int32_t *)status, base, scalar};
+    return launch_slots(*c, f, n, as_stream(stream)) ? GOLDILOCKS_SUCCESS : GOLDILOCKS_FAILURE;
+}
+goldilocks_error_t goldilocks_x448_peerset_batch_dev(uint8_t *out, goldilocks_error_t *status, const goldilocks_b200_x448_peerset *ps, const uint32_t *peer_index,
+                                                     const uint8_t *scalar, size_t n, void *stream) {
+    if (n == 0) return GOLDILOCKS_SUCCESS;
+    Ctx *c = dev_ctx();
+    if (!c) return GOLDILOCKS_FAILURE;
+    if (!ps || ps->dev != c->dev) { g_err = "goldilocks_x448_peerset_batch_dev: the peer set lives on another device"; return GOLDILOCKS_FAILURE; }
+    SlotX448Peer f = {out, (int32_t *)status, ps->tables, ps->table_ok, ps->peers, peer_index, scalar, (uint32_t)ps->m};
     return launch_slots(*c, f, n, as_stream(stream)) ? GOLDILOCKS_SUCCESS : GOLDILOCKS_FAILURE;
 }
 goldilocks_error_t goldilocks_448_precomputed_scalarmul_batch_dev(hpt *out, const hsc *scalar, size_t n, void *stream) {

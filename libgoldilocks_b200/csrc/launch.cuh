@@ -44,6 +44,7 @@ cudaError_t launch_lanes(const F &f, size_t n, cudaStream_t s) {
 #define SLOT7_MIN_BLOCKS 4 /* 7 slots = 56 KB per block: four blocks (16 warps) per SM, 128 registers */
 #endif
 template <> struct slot_min_blocks<SlotX448> { static constexpr int value = 4; };
+template <> struct slot_min_blocks<SlotX448Peer> { static constexpr int value = 4; };
 template <> struct slot_min_blocks<SlotNielsDebug> { static constexpr int value = 4; };
 template <> struct slot_min_blocks<SlotComb> { static constexpr int value = SLOT7_MIN_BLOCKS; };
 template <> struct slot_min_blocks<SlotX448DerivePk> { static constexpr int value = SLOT7_MIN_BLOCKS; };
@@ -106,12 +107,12 @@ cudaError_t launch_sm_persist(const F &f, size_t n, int grid, cudaStream_t s, un
     X(LaneFromHash<false>) X(LaneFromHash<true>) X(LaneInvertElligator<false>) X(LaneInvertElligator<true>)                                                    \
     X(LaneEncodeEddsa) X(LaneDecodeEddsa) X(LaneEncodeX448)                                         \
     X(LaneSc<SCOP_ADD>) X(LaneSc<SCOP_SUB>) X(LaneSc<SCOP_MUL>) X(LaneSc<SCOP_HALVE>)               \
-    X(LaneScDecodeLong) X(LaneScInvert) X(LaneShake256) X(LaneSpongeUpdate) X(LaneSpongeOutput) X(LaneEdPkToX448) X(LaneEdSkToX448) X(LanePrecompute) X(LaneNielsFromAbi)                                                             \
+    X(LaneScDecodeLong) X(LaneScInvert) X(LaneShake256) X(LaneSpongeUpdate) X(LaneSpongeOutput) X(LaneEdPkToX448) X(LaneEdSkToX448) X(LanePrecompute) X(LaneNielsFromAbi) X(LaneX448PeerLift)                                                             \
     X(LaneEdSecretScalar) X(LaneEdSignExpand) X(LaneEdSignNonce) X(LaneEdSignFinish)   \
     X(LaneEdVerifyDecode) X(LaneEdVerifyScalars) X(LaneVerifySign) X(LaneVerifyHalf) X(LaneKeysetNormalize) X(LaneBuildTables) X(LaneBuildWide) \
     X(LaneRlcDecode) X(LaneRlcZ) X(LaneRlcWeights) X(LaneRlcLate) X(LaneRlcKeyScalars) X(LaneRlcDigits) X(LaneRlcBucketRuns) X(LaneRlcSegments) X(LaneRlcNodes) X(LaneRlcWindows) X(LaneRlcTotal) X(LaneRlcVerdict) X(LaneRlcPackPlan) X(LaneRlcPack) X(LaneRlcUnpack) X(LanePtNiels)
 
-#define LANES_SM(X) X(SlotNielsDebug) X(SlotX448) X(SlotComb) X(SlotCombTable) X(SlotX448DerivePk) X(SlotEdDerivePk) X(SlotEdSignR) X(SlotRlcBucket)
+#define LANES_SM(X) X(SlotNielsDebug) X(SlotX448) X(SlotX448Peer) X(SlotComb) X(SlotCombTable) X(SlotX448DerivePk) X(SlotEdDerivePk) X(SlotEdSignR) X(SlotRlcBucket)
 #define INSTANTIATE_SM(F) template cudaError_t launch_sm<F>(const F &, size_t, cudaStream_t);
 #define DECLARE_SM(F) extern INSTANTIATE_SM(F)
 #define LANES_SMP(X) X(SlotEdVerifyFinish) X(SlotEdVerifyFinishShared) X(SlotKeyChain) X(SlotKeyColumns) X(SlotKeysetTables) X(SlotKeysetChain) X(SlotKeysetColumns) X(SlotEdVerifyFinishKeyset) X(SlotEdVerifyFinishKeysetFlat) X(SlotBaseDoubleScalarmul) X(SlotScalarmul) X(SlotDoubleScalarmul) X(SlotDualScalarmul) X(SlotDirectScalarmul)

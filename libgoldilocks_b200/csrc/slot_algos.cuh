@@ -43,7 +43,8 @@ GD void s_block_invert4(sref sb, int zin, int zout) {
 // 1 mulw+add = 14 slot operations on 7 slots; the two conditional swaps exchange handles only.
 // ---------------------------------------------------------------------------------------------
 #define X448_NSLOTS 7
-GD gmask_t x448_ladder_slots(uint32_t out[14], const uint32_t base[14], const uint32_t scalar[14], sref sb) {
+// The ladder proper: on return x_out / z_out name the slots (two of 1..4) that hold the projective result.
+GD void x448_ladder_xz(sref &x_out, sref &z_out, const uint32_t base[14], const uint32_t scalar[14], sref sb) {
     sref x1 = s_slot(sb, 0), x2 = s_slot(sb, 1), z2 = s_slot(sb, 2), x3 = s_slot(sb, 3), z3 = s_slot(sb, 4), t1 = s_slot(sb, 5), t2 = s_slot(sb, 6);
     {
         gf v;
@@ -97,19 +98,24 @@ GD gmask_t x448_ladder_slots(uint32_t out[14], const uint32_t base[14], const ui
         const sref nz2 = s_sel(z2, z3, swap), nz3 = s_sel(z3, z2, swap);
         x2 = nx2; x3 = nx3; z2 = nz2; z3 = nz3;
     }
-    /* u = x2 / z2 with 0 for z2 = 0 (goldilocks.c:69-80 gf_invert(0) = 0).  On the device the inversion is
-     * shared by the four lanes of a block that have the same lane index (s_block_invert4 below): one
-     * addition chain per four elements instead of one per element. */
+    x_out = x2;
+    z_out = z2;
+}
+// out = canonical bytes of num / den, 0 for den = 0 (goldilocks.c:69-80 gf_invert(0) = 0); all-ones iff out != 0.
+// num: any slot but 5, den: any slot; every slot is clobbered.  On the device the inversion is
+// shared by the four lanes of a block that have the same lane index (s_block_invert4 below): one addition chain
+// per four elements instead of one per element -- so every lane of the block has to get here.
+GD gmask_t x448_finish(uint32_t out[14], sref sb, sref num, sref den) {
     const sref zi = s_slot(sb, 5), xs = s_slot(sb, 6), res = s_slot(sb, 0);
     gmask_t nz;
     {
         gf z, one;
-        s_ld(z, z2);
+        s_ld(z, den);
         nz = ~gf_is_zero(z);
         gf_set_ui(one, 1);
         gf_cond_sel(z, one, z, nz);             /* 0 -> 1 so it cannot poison the shared product */
         s_st(zi, z);
-        s_copy(xs, x2);
+        s_copy(xs, num);
     }
 #if defined(__CUDA_ARCH__)
     s_block_invert4(sb, 5, 4);                  /* slot 5 -> its inverse in slot 4 */
@@ -124,6 +130,11 @@ GD gmask_t x448_ladder_slots(uint32_t out[14], const uint32_t base[14], const ui
     gf_cond_sel(r, zero, r, nz);
     gf_to_words(out, r);
     return ~gf_is_zero(r);
+}
+GD gmask_t x448_ladder_slots(uint32_t out[14], const uint32_t base[14], const uint32_t scalar[14], sref sb) {
+    sref x2, z2;
+    x448_ladder_xz(x2, z2, base, scalar, sb);
+    return x448_finish(out, sb, x2, z2);
 }
 
 // ---------------------------------------------------------------------------------------------

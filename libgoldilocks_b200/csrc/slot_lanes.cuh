@@ -371,6 +371,99 @@ struct SlotX448DerivePk { /* goldilocks.c:1117-1141 */
         if (live) words_store56(out + 56 * i, wo);
     }
 };
+// X448 peer sets (include/goldilocks_b200.h, goldilocks_b200_x448_peerset_*; DESIGN.md decision 20).  A recurring public u gets
+// the reference's (5,5,18) comb table (LanePrecompute) of an Edwards point Q with X448(u, k) = encode_like_x448((k / 8) Q):
+// 17 doublings and 90 additions instead of 448 ladder steps.  The dual of RFC 7748's 4-isogeny sends (u, v) on curve448 to
+// edwards448 with a y that depends on u alone,
+//     y = -(u^5 - 2u^3 - 4u v^2 + u) / (u^5 - 2u^2 v^2 - 2u^3 - 2v^2 + u),   v^2 = u^3 + 156326 u^2 + u,
+// and Q = that y decoded like an EdDSA key with sign 0 (the sign of x never reaches a u-coordinate).  psi_hat(psi) = [4], the
+// decode has ratio 1 and the X448 encoder ratio 2: the composite is [+-8], hence k / 8, and it kills the torsion of u as the
+// clamped k does in the ladder.  A peer takes the table only if v^2 is a non-zero square (checked here, not left to the
+// decoder), u mod p is neither 0 (the denominator vanishes and gf_invert(0) = 0 would hide it) nor p - 1 (y = 1, which the
+// decoder rejects), and the decode succeeds; every other peer keeps the ladder.  The flag is public.
+struct LaneX448PeerLift {
+    abi_pt *pts; int32_t *table_ok; const uint8_t *peers;
+    GDM void operator()(size_t i) const {
+        uint32_t w[14];
+        words_load56(w, peers + 56 * i);
+        gf u, u2, v2, a, b, num, den, one;
+        (void)gf_from_words(u, w);                       /* u >= p is taken mod p, like the ladder does */
+        gf_set_ui(one, 1);
+        gf_sqr(u2, u);
+        gf_mulw(a, u, 156326);
+        gf_add(a, a, u2);
+        gf_add(a, a, one);
+        gf_mul(v2, a, u);                                /* v^2 = u (u^2 + 156326 u + 1) */
+        gf_sub(a, u2, one);
+        gf_sqr(a, a);                                    /* (u^2 - 1)^2 */
+        gf_add(b, v2, v2);
+        gf_add(b, b, b);
+        gf_sub(num, a, b);
+        gf_mul(num, num, u);                             /* u ((u^2 - 1)^2 - 4 v^2) */
+        gf_mul(den, a, u);
+        gf_add(b, u2, one);
+        gf_mul(b, b, v2);
+        gf_add(b, b, b);
+        gf_sub(den, den, b);                             /* u (u^2 - 1)^2 - 2 v^2 (u^2 + 1) */
+        gmask_t ok = gf_isr(a, v2);                      /* v^2 a non-zero square: u is on the curve, not on its twist */
+        ok &= ~gf_is_zero(u);
+        gf_add(b, u, one);
+        ok &= ~gf_is_zero(b);                            /* u != p - 1 */
+        ok &= ~gf_is_zero(den);
+        gf_invert(den, den);
+        gf_mul(a, num, den);
+        gf_neg(a, a);
+        uint32_t yw[14];
+        gf_to_words(yw, a);
+        pt q;
+        ok &= pt_decode_like_eddsa(q, yw, 0);
+        if (!ok) pt_set_identity(q);                     /* a ladder peer's table is built from the identity and never read */
+        pt_to_abi(pts + i, q);
+        table_ok[i] = ST_OK(ok);
+    }
+};
+// Element i = goldilocks_x448(peers[peer_index[i]], scalar i): the comb over the peer's table or the ladder, by the peer's
+// public flag.  Both leave a fraction num / den -- (y^2, x^2) of the comb result (goldilocks.c:1104-1115 u = (y/x)^2), the
+// ladder's (x2, z2) -- and meet in ONE x448_finish, because its inversion is shared across the block (s_block_invert4) and
+// every lane has to reach it, whichever branch its warp took.  A missing peer is 0 / 0: zeros and FAILURE.
+struct SlotX448Peer {
+    static constexpr int NSLOTS = 7;
+    static_assert(COMB_NSLOTS == NSLOTS && X448_NSLOTS == NSLOTS, "the comb and the ladder share the slots");
+    uint8_t *out; int32_t *status; const niels *tables; const int32_t *table_ok; const uint8_t *peers;
+    const uint32_t *peer_index; const uint8_t *scalar; uint32_t n_peers;
+    GDM void operator()(size_t i, sref sb, bool live) const {
+        uint32_t ws[14], wo[14];
+        words_load56(ws, scalar + 56 * i);
+        const uint32_t t = peer_index[i];
+        sref num = s_slot(sb, 6), den = s_slot(sb, 5);
+        if (t >= n_peers) {
+            gf z;
+            gf_set_zero(z);
+            s_st(num, z);
+            s_st(den, z);
+        } else if (table_ok[t]) {
+            ws[0] &= ~3u;
+            ws[13] |= 0x80000000u;                       /* clamped exactly as the ladder clamps (SlotX448DerivePk) */
+            sc s, h;
+            ByteAtWords at = {ws};
+            sc_decode_long(s, at, 56);
+            sc_halve(h, s);
+            sc_halve(s, h);
+            sc_halve(h, s);                              /* k / 8 */
+            s_comb_scalarmul_table(sb, tables + (size_t)COMB_ENTRIES * t, h);
+            s_sqr(num, s_slot(sb, 1));
+            s_sqr(den, s_slot(sb, 0));
+        } else {
+            uint32_t wu[14];
+            words_load56(wu, peers + 56 * (size_t)t);
+            x448_ladder_xz(num, den, wu, ws, sb);
+        }
+        const gmask_t nz = x448_finish(wo, sb, num, den);
+        if (!live) return;
+        words_store56(out + 56 * i, wo);
+        status[i] = ST_OK(nz);
+    }
+};
 struct SlotEdDerivePk { /* eddsa.c:129-144 */
     static constexpr int NSLOTS = COMB_NSLOTS;
     uint8_t *pk; const uint8_t *sk; const fixed_tables *ft;

@@ -93,6 +93,11 @@ class DeviceEngine:
     def x448(self, out, status, base, scalar):
         self._call("goldilocks_x448_batch_dev", self._p(out), self._p(status), self._p(base), self._p(scalar), _Z(status.numel()), self._stream())
 
+    def x448_peerset(self, out, status, handle, peer_index, scalar):
+        """X448 of scalar i against peer peer_index[i] (uint32 tensor viewed as int32) of a set made by capi x448_peerset_create"""
+        self._call("goldilocks_x448_peerset_batch_dev", self._p(out), self._p(status), handle, self._p(peer_index), self._p(scalar),
+                   _Z(status.numel()), self._stream())
+
     def precomputed_scalarmul(self, out_pts, scalars):
         self._call("goldilocks_448_precomputed_scalarmul_batch_dev", self._p(out_pts), self._p(scalars), _Z(scalars.numel() // 56), self._stream())
 
