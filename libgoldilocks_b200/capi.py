@@ -352,6 +352,31 @@ class BatchLib:
         self._call("goldilocks_x448_peerset_batch", out, st, handle, peer_index, scalar, _Z(len(scalar)))
         return out, st
 
+    # ---- decaf peer sets: per-peer comb tables for direct_scalarmul against recurring points ----
+    def decaf_peerset_create(self, encodings, allow_identity=False):
+        """handle for m peer encodings ((m,56) u8) decoded under allow_identity; free it with decaf_peerset_destroy"""
+        enc = _u8(encodings, 56)
+        h = C.c_void_p()
+        self._call("goldilocks_b200_decaf_peerset_create", C.byref(h), enc, C.c_uint64(ALL if allow_identity else 0), _Z(len(enc)))
+        return h
+
+    def decaf_peerset_destroy(self, handle):
+        self.lib.goldilocks_b200_decaf_peerset_destroy.restype = None
+        self.lib.goldilocks_b200_decaf_peerset_destroy(handle)
+
+    def decaf_peerset_size(self, handle):
+        f = self.lib.goldilocks_b200_decaf_peerset_size
+        f.restype = _Z
+        return int(f(handle))
+
+    def decaf_peerset(self, handle, peer_index, scalars, short_circuit=True, prefill=0):
+        """(scaled (n,56) u8, status int32[n]): direct_scalarmul of scalar struct i against peer peer_index[i] of the set;
+        `prefill` is what short-circuited elements keep, as in direct_scalarmul"""
+        s = _u8(scalars, 56); peer_index = np.ascontiguousarray(peer_index, np.uint32).reshape(-1)
+        out = np.full((len(s), 56), prefill, np.uint8); st = np.zeros(len(s), np.int32)
+        self._call("goldilocks_448_direct_scalarmul_peerset_batch", out, st, handle, peer_index, s, C.c_uint64(ALL if short_circuit else 0), _Z(len(s)))
+        return out, st
+
     def ed448_verify(self, sig, pk, msgs, prehashed=False, context=b""):
         sig, pk = _u8(sig, 114), _u8(pk, 57)
         arena, off = pack_messages(msgs) if isinstance(msgs, list) else msgs

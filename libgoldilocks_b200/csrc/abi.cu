@@ -1640,6 +1640,98 @@ goldilocks_error_t goldilocks_x448_peerset_batch(uint8_t *out, goldilocks_error_
     return k.finish();
 }
 
+// ---- decaf peer sets: per-peer comb tables for goldilocks_448_direct_scalarmul against recurring points (slot_lanes.cuh SlotDecafPeer)
+struct goldilocks_b200_decaf_peerset_s {
+    int dev; size_t m;
+    int32_t *peer_ok;   /* m + 1 decode statuses (public); entry m, the base point with FAILURE, stands for every index >= m */
+    niels *tables;      /* m + 1 tables of COMB_ENTRIES affine niels, 15 360 bytes each */
+};
+/* the scratch of one call, carved from `base` (null: sizes only): sort keys and values in and out, CUB's temporary storage */
+struct DecafPeerScratch { uint32_t *keys, *vals, *keys_s, *order; void *sort_tmp; size_t sort_bytes; };
+static size_t decaf_peer_scratch(DecafPeerScratch *s, void *base, size_t n) {
+    auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
+    const size_t words = al(sizeof(uint32_t) * n), sort_bytes = pair_sort_scratch_bytes(n);
+    if (s) {
+        char *p = (char *)base;
+        s->keys = (uint32_t *)p; s->vals = (uint32_t *)(p + words); s->keys_s = (uint32_t *)(p + 2 * words); s->order = (uint32_t *)(p + 3 * words);
+        s->sort_tmp = p + 4 * words; s->sort_bytes = sort_bytes;
+    }
+    return 4 * words + al(sort_bytes);
+}
+/* keys (min(peer_index[j], m), j) -> stable radix sort by peer -> the comb kernel over the elements in that order.  The sort is
+ * bracketed like a launch when profiling is on, so goldilocks_b200_profile_timeline shows its share of the call. */
+static bool decaf_peer_enqueue(Ctx &c, uint8_t *scaled, int32_t *status, const goldilocks_b200_decaf_peerset_s *ps, const uint32_t *peer_index,
+                               const abi_sc *scalar, bool short_circuit, size_t n, const DecafPeerScratch &s, cudaStream_t st) {
+    const uint32_t m = (uint32_t)ps->m;
+    LaneDecafPeerKeys fk = {s.keys, s.vals, peer_index, m};
+    if (!launch(c, fk, n, st)) return false;
+    int key_bits = 1;
+    while (key_bits < 32 && (m >> key_bits)) key_bits++;   /* the bit length of m, the largest key */
+    cudaEvent_t a = nullptr, b = nullptr;
+    const bool prof = g_prof_on.load() != 0;
+    if (prof) a = prof_begin("pair_sort", st, &b);
+    const cudaError_t e = pair_sort(s.sort_tmp, s.sort_bytes, s.keys, s.keys_s, s.vals, s.order, n, key_bits, st);
+    if (prof) prof_end("pair_sort", st, a, b);
+    if (e != cudaSuccess) return fail("pair_sort (decaf peer set)", e);
+    SlotDecafPeer f = {scaled, status, ps->tables, ps->peer_ok, peer_index, s.order, scalar, m, short_circuit ? ~0u : 0u};
+    return launch_slots(c, f, n, st);
+}
+goldilocks_error_t goldilocks_b200_decaf_peerset_create(goldilocks_b200_decaf_peerset **out, const uint8_t *peers, goldilocks_bool_t allow_identity, size_t m) {
+    if (!out) return GOLDILOCKS_FAILURE;
+    *out = nullptr;
+    Call k;
+    if (!k.ok) return k.finish();
+    if (m >= UINT32_MAX) { g_err = "goldilocks_b200_decaf_peerset_create: at most 2^32 - 2 peers"; return GOLDILOCKS_FAILURE; }
+    const size_t mm = m + 1;
+    goldilocks_b200_decaf_peerset_s *ps = new goldilocks_b200_decaf_peerset_s{k.c->dev, m, nullptr, nullptr};
+    bool ok = cudaMalloc(&ps->peer_ok, sizeof(int32_t) * mm) == cudaSuccess && cudaMalloc(&ps->tables, mm * COMB_ENTRIES * sizeof(niels)) == cudaSuccess;
+    if (ok) {
+        abi_pt *pts = k.out<abi_pt>(mm);
+        LaneDecafPeerDecode fd = {pts, ps->peer_ok, k.in(peers, 56 * m), k.c->ft, (uint32_t)m, allow_identity ? 1u : 0u};
+        k.run(fd, mm);
+        LanePrecompute fp = {k.out<abi_niels>(COMB_ENTRIES * mm), pts, k.out<niels>(16 * COMB_N * mm)};
+        k.run(fp, COMB_N * mm);
+        LaneNielsFromAbi fc = {ps->tables, fp.tables};
+        k.run(fc, COMB_ENTRIES * mm);
+    }
+    goldilocks_error_t r = k.finish();
+    if (!ok || r != GOLDILOCKS_SUCCESS) {
+        if (!ok) g_err = "goldilocks_b200_decaf_peerset_create: device allocation failed";
+        cudaFree(ps->peer_ok); cudaFree(ps->tables);
+        delete ps;
+        return GOLDILOCKS_FAILURE;
+    }
+    *out = ps;
+    return GOLDILOCKS_SUCCESS;
+}
+void goldilocks_b200_decaf_peerset_destroy(goldilocks_b200_decaf_peerset *ps) {
+    if (!ps) return;
+    int cur = 0;
+    const bool sw = cudaGetDevice(&cur) == cudaSuccess && cur != ps->dev && cudaSetDevice(ps->dev) == cudaSuccess;
+    cudaFree(ps->peer_ok); cudaFree(ps->tables);
+    if (sw) cudaSetDevice(cur);
+    delete ps;
+}
+size_t goldilocks_b200_decaf_peerset_size(const goldilocks_b200_decaf_peerset *ps) { return ps ? ps->m : 0; }
+goldilocks_error_t goldilocks_448_direct_scalarmul_peerset_batch(uint8_t *scaled, goldilocks_error_t *status, const goldilocks_b200_decaf_peerset *ps,
+                                                                 const uint32_t *peer_index, const hsc *scalar, goldilocks_bool_t short_circuit, size_t n) {
+    if (n == 0) return GOLDILOCKS_SUCCESS;
+    Call k;
+    if (!k.ok) return k.finish();
+    if (!ps || ps->dev != k.c->dev) { g_err = "goldilocks_448_direct_scalarmul_peerset_batch: the peer set lives on another device"; return GOLDILOCKS_FAILURE; }
+    if (n > (size_t)INT32_MAX) { g_err = "goldilocks_448_direct_scalarmul_peerset_batch: n >= 2^31"; return GOLDILOCKS_FAILURE; }
+    uint8_t *dout = k.secret(k.in(scaled, 56 * n), 56 * n); /* short-circuited elements keep the caller's bytes */
+    int32_t *dst = k.out<int32_t>(n);
+    const uint32_t *didx = k.in(peer_index, n);
+    const abi_sc *dsc = k.secret(k.in(S(scalar), n), n);
+    DecafPeerScratch s;
+    decaf_peer_scratch(&s, k.alloc(decaf_peer_scratch(nullptr, nullptr, n)), n);
+    if (k.ok) k.ok = decaf_peer_enqueue(*k.c, dout, dst, ps, didx, dsc, short_circuit != 0, n, s, k.c->stream);
+    k.fetch(scaled, dout, 56 * n);
+    k.fetch((int32_t *)status, dst, n);
+    return k.finish();
+}
+
 // ---- device-resident variants -------------------------------------------------------------------------------
 goldilocks_error_t goldilocks_ed448_verify_batch_dev(goldilocks_error_t *status, const uint8_t *signature, const uint8_t *pubkey, const uint8_t *msg, const size_t *msg_off,
                                                      uint8_t prehashed, const uint8_t *context, uint8_t context_len, size_t n, void *scratch, void *stream) {
@@ -1669,6 +1761,25 @@ goldilocks_error_t goldilocks_x448_peerset_batch_dev(uint8_t *out, goldilocks_er
     if (!ps || ps->dev != c->dev) { g_err = "goldilocks_x448_peerset_batch_dev: the peer set lives on another device"; return GOLDILOCKS_FAILURE; }
     SlotX448Peer f = {out, (int32_t *)status, ps->tables, ps->table_ok, ps->peers, peer_index, scalar, (uint32_t)ps->m};
     return launch_slots(*c, f, n, as_stream(stream)) ? GOLDILOCKS_SUCCESS : GOLDILOCKS_FAILURE;
+}
+size_t goldilocks_b200_decaf_peerset_scratch_bytes(size_t n) {
+    if (!dev_ctx()) return 0;
+    return decaf_peer_scratch(nullptr, nullptr, n);
+}
+goldilocks_error_t goldilocks_448_direct_scalarmul_peerset_batch_dev(uint8_t *scaled, goldilocks_error_t *status, const goldilocks_b200_decaf_peerset *ps,
+                                                                     const uint32_t *peer_index, const hsc *scalar, goldilocks_bool_t short_circuit, size_t n,
+                                                                     void *scratch, void *stream) {
+    if (n == 0) return GOLDILOCKS_SUCCESS;
+    Ctx *c = dev_ctx();
+    if (!c) return GOLDILOCKS_FAILURE;
+    if (!ps || ps->dev != c->dev) { g_err = "goldilocks_448_direct_scalarmul_peerset_batch_dev: the peer set lives on another device"; return GOLDILOCKS_FAILURE; }
+    if (n > (size_t)INT32_MAX) { g_err = "goldilocks_448_direct_scalarmul_peerset_batch_dev: n >= 2^31"; return GOLDILOCKS_FAILURE; }
+    if (!scratch) { g_err = "goldilocks_448_direct_scalarmul_peerset_batch_dev: no scratch"; return GOLDILOCKS_FAILURE; }
+    /* everything the call writes besides scaled / status lives in the caller's scratch: calls on different streams do not interfere */
+    DecafPeerScratch s;
+    decaf_peer_scratch(&s, scratch, n);
+    return decaf_peer_enqueue(*c, scaled, (int32_t *)status, ps, peer_index, S(scalar), short_circuit != 0, n, s, as_stream(stream)) ? GOLDILOCKS_SUCCESS
+                                                                                                                                      : GOLDILOCKS_FAILURE;
 }
 goldilocks_error_t goldilocks_448_precomputed_scalarmul_batch_dev(hpt *out, const hsc *scalar, size_t n, void *stream) {
     Ctx *c = dev_ctx();

@@ -51,6 +51,7 @@ template <> struct slot_min_blocks<SlotX448DerivePk> { static constexpr int valu
 template <> struct slot_min_blocks<SlotEdDerivePk> { static constexpr int value = SLOT7_MIN_BLOCKS; };
 template <> struct slot_min_blocks<SlotEdSignR> { static constexpr int value = SLOT7_MIN_BLOCKS; };
 template <> struct slot_min_blocks<SlotCombTable> { static constexpr int value = SLOT7_MIN_BLOCKS; };
+template <> struct slot_min_blocks<SlotDecafPeer> { static constexpr int value = SLOT7_MIN_BLOCKS; };
 template <> struct slot_min_blocks<SlotDualScalarmul> { static constexpr int value = SLOT7_MIN_BLOCKS; };
 template <> struct slot_min_blocks<SlotDirectScalarmul> { static constexpr int value = SLOT7_MIN_BLOCKS; };
 template <> struct slot_min_blocks<SlotScalarmul> { static constexpr int value = SLOT7_MIN_BLOCKS; };
@@ -107,12 +108,12 @@ cudaError_t launch_sm_persist(const F &f, size_t n, int grid, cudaStream_t s, un
     X(LaneFromHash<false>) X(LaneFromHash<true>) X(LaneInvertElligator<false>) X(LaneInvertElligator<true>)                                                    \
     X(LaneEncodeEddsa) X(LaneDecodeEddsa) X(LaneEncodeX448)                                         \
     X(LaneSc<SCOP_ADD>) X(LaneSc<SCOP_SUB>) X(LaneSc<SCOP_MUL>) X(LaneSc<SCOP_HALVE>)               \
-    X(LaneScDecodeLong) X(LaneScInvert) X(LaneShake256) X(LaneSpongeUpdate) X(LaneSpongeOutput) X(LaneEdPkToX448) X(LaneEdSkToX448) X(LanePrecompute) X(LaneNielsFromAbi) X(LaneX448PeerLift)                                                             \
+    X(LaneScDecodeLong) X(LaneScInvert) X(LaneShake256) X(LaneSpongeUpdate) X(LaneSpongeOutput) X(LaneEdPkToX448) X(LaneEdSkToX448) X(LanePrecompute) X(LaneNielsFromAbi) X(LaneX448PeerLift) X(LaneDecafPeerDecode) X(LaneDecafPeerKeys)                                                             \
     X(LaneEdSecretScalar) X(LaneEdSignExpand) X(LaneEdSignNonce) X(LaneEdSignFinish)   \
     X(LaneEdVerifyDecode) X(LaneEdVerifyScalars) X(LaneVerifySign) X(LaneVerifyHalf) X(LaneKeysetNormalize) X(LaneBuildTables) X(LaneBuildWide) \
     X(LaneRlcDecode) X(LaneRlcZ) X(LaneRlcWeights) X(LaneRlcLate) X(LaneRlcKeyScalars) X(LaneRlcDigits) X(LaneRlcBucketRuns) X(LaneRlcSegments) X(LaneRlcNodes) X(LaneRlcWindows) X(LaneRlcTotal) X(LaneRlcVerdict) X(LaneRlcPackPlan) X(LaneRlcPack) X(LaneRlcUnpack) X(LanePtNiels)
 
-#define LANES_SM(X) X(SlotNielsDebug) X(SlotX448) X(SlotX448Peer) X(SlotComb) X(SlotCombTable) X(SlotX448DerivePk) X(SlotEdDerivePk) X(SlotEdSignR) X(SlotRlcBucket)
+#define LANES_SM(X) X(SlotNielsDebug) X(SlotX448) X(SlotX448Peer) X(SlotComb) X(SlotCombTable) X(SlotDecafPeer) X(SlotX448DerivePk) X(SlotEdDerivePk) X(SlotEdSignR) X(SlotRlcBucket)
 #define INSTANTIATE_SM(F) template cudaError_t launch_sm<F>(const F &, size_t, cudaStream_t);
 #define DECLARE_SM(F) extern INSTANTIATE_SM(F)
 #define LANES_SMP(X) X(SlotEdVerifyFinish) X(SlotEdVerifyFinishShared) X(SlotKeyChain) X(SlotKeyColumns) X(SlotKeysetTables) X(SlotKeysetChain) X(SlotKeysetColumns) X(SlotEdVerifyFinishKeyset) X(SlotEdVerifyFinishKeysetFlat) X(SlotBaseDoubleScalarmul) X(SlotScalarmul) X(SlotDoubleScalarmul) X(SlotDualScalarmul) X(SlotDirectScalarmul)

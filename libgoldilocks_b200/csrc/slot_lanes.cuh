@@ -464,6 +464,74 @@ struct SlotX448Peer {
         status[i] = ST_OK(nz);
     }
 };
+// Decaf peer sets (include/goldilocks_b200.h, goldilocks_b200_decaf_peerset_*; DESIGN.md decision 21): a recurring peer of
+// goldilocks_448_direct_scalarmul (goldilocks.c:888-903) is decoded once and gets the reference's (5,5,18) comb table, so a call
+// runs the comb instead of the signed-window multiplication.  Both recode the scalar with the same sc_recode_signed and add up
+// the same signed digits (every one of the 450 bit positions contributes +-2^k), so they multiply the point by the same
+// integer 2 s' - (2^450 - 1): the same point, and the same encoding.  Lane t < m decodes peer t; a peer that fails to decode
+// is the base point with FAILURE, exactly as SlotDirectScalarmul selects it.  Entry m is the base point with FAILURE: an index
+// >= m is clamped to it, which is what 56 undecodable bytes give.  The status is public.
+struct LaneDecafPeerDecode {
+    abi_pt *pts; int32_t *peer_ok; const uint8_t *peers; const fixed_tables *ft; uint32_t m, allow_identity;
+    GDM void operator()(size_t t) const {
+        pt p;
+        pt_set_identity(p);
+        gmask_t ok = 0;
+        if (t < m) {
+            uint32_t wd[14];
+            words_load56(wd, peers + 56 * t);
+            ok = pt_decode(p, wd, allow_identity ? ~0u : 0u);
+        }
+        pt q; /* point_cond_sel(basep, point_base, basep, succ) */
+        gf_cond_sel(q.x, ft->base.x, p.x, ok);
+        gf_cond_sel(q.y, ft->base.y, p.y, ok);
+        gf_cond_sel(q.z, ft->base.z, p.z, ok);
+        gf_cond_sel(q.t, ft->base.t, p.t, ok);
+        pt_to_abi(pts + t, q);
+        peer_ok[t] = ST_OK(ok);
+    }
+};
+// The sort keys of a call: (min(peer_index[j], m), j).  Sorted by peer, the values are the order SlotDecafPeer takes the
+// elements in, so the lanes of a warp read one or two tables instead of up to 32.  Only public data goes through the sort.
+struct LaneDecafPeerKeys {
+    uint32_t *keys, *vals; const uint32_t *peer_index; uint32_t m;
+    GDM void operator()(size_t j) const {
+        const uint32_t t = peer_index[j];
+        keys[j] = t < m ? t : m;
+        vals[j] = (uint32_t)j;
+    }
+};
+// Lane j: element i = order[j] of goldilocks_448_direct_scalarmul(scaled_i, peers[peer_index[i]], scalar i, allow_identity of
+// the set, short_circuit).  The comb over table min(peer_index[i], m), the decaf encoding, the peer's status; with short_circuit
+// a failed element keeps the caller's bytes through SlotDirectScalarmul's masked merge.  Reads and writes element i in place.
+struct SlotDecafPeer {
+    static constexpr int NSLOTS = COMB_NSLOTS;
+    uint8_t *scaled; int32_t *status; const niels *tables; const int32_t *peer_ok; const uint32_t *peer_index; const uint32_t *order;
+    const abi_sc *scalar; uint32_t n_peers, short_circuit;
+    GDM void operator()(size_t j, sref sb, bool live) const {
+        const size_t i = order[j];
+        const uint32_t ti = peer_index[i];
+        const size_t t = ti < n_peers ? ti : n_peers;
+        sc s;
+        sc_from_abi(s, scalar + i);
+        s_comb_scalarmul_table(sb, tables + (size_t)COMB_ENTRIES * t, s);
+        pt q;
+        s_ld(q.x, s_slot(sb, 0)); s_ld(q.y, s_slot(sb, 1)); s_ld(q.z, s_slot(sb, 2)); s_ld(q.t, s_slot(sb, 3));
+        gf e;
+        pt_deisogenize(e, q);
+        uint32_t wd[14];
+        gf_to_words(wd, e);
+        if (!live) return;
+        const int32_t st = peer_ok[t];
+        status[i] = st;
+        uint32_t keep[14];
+        words_load56(keep, scaled + 56 * i);
+        const gmask_t wr = (gmask_t)st | (short_circuit ? 0u : ~0u);
+#pragma unroll
+        for (int k = 0; k < 14; k++) wd[k] = (wd[k] & wr) | (keep[k] & ~wr);
+        words_store56(scaled + 56 * i, wd);
+    }
+};
 struct SlotEdDerivePk { /* eddsa.c:129-144 */
     static constexpr int NSLOTS = COMB_NSLOTS;
     uint8_t *pk; const uint8_t *sk; const fixed_tables *ft;

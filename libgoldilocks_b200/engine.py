@@ -98,6 +98,19 @@ class DeviceEngine:
         self._call("goldilocks_x448_peerset_batch_dev", self._p(out), self._p(status), handle, self._p(peer_index), self._p(scalar),
                    _Z(status.numel()), self._stream())
 
+    def decaf_peerset_scratch_bytes(self, n):
+        f = self.lib.goldilocks_b200_decaf_peerset_scratch_bytes
+        f.restype = _Z
+        f.argtypes = [_Z]
+        return int(f(n))
+
+    def decaf_peerset(self, scaled, status, handle, peer_index, scalars, scratch, short_circuit=True):
+        """direct_scalarmul of scalar struct i against peer peer_index[i] (uint32 tensor viewed as int32) of a set made by capi
+        decaf_peerset_create; `scaled` is read (short-circuited elements keep it) and written in place; `scratch` holds
+        decaf_peerset_scratch_bytes(n)"""
+        self._call("goldilocks_448_direct_scalarmul_peerset_batch_dev", self._p(scaled), self._p(status), handle, self._p(peer_index), self._p(scalars),
+                   C.c_uint64((1 << 64) - 1 if short_circuit else 0), _Z(status.numel()), self._p(scratch), self._stream())
+
     def precomputed_scalarmul(self, out_pts, scalars):
         self._call("goldilocks_448_precomputed_scalarmul_batch_dev", self._p(out_pts), self._p(scalars), _Z(scalars.numel() // 56), self._stream())
 
