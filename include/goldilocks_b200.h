@@ -253,9 +253,10 @@ typedef struct goldilocks_b200_keyset_s goldilocks_b200_keyset;
 GOLDILOCKS_B200_API goldilocks_error_t goldilocks_b200_keyset_create(goldilocks_b200_keyset **keyset, const uint8_t *pubkeys /*m*57*/, size_t m);
 GOLDILOCKS_B200_API void goldilocks_b200_keyset_destroy(goldilocks_b200_keyset *keyset);
 GOLDILOCKS_B200_API size_t goldilocks_b200_keyset_size(const goldilocks_b200_keyset *keyset);
-/* Table layout of the key sets created from now on: a set whose FLAT tables -- 369 KB per key, one 16-entry table of affine multiples per
- * digit position, so a signature under the key costs additions only and no doubling -- fit max_table_bytes gets them (default 32 GB:
- * sets of up to 93 000 keys); larger sets keep the 41 KB per key layout (ten columns, forty doublings per signature).  0 = never flat. */
+/* Table layout of the key sets and point sets created from now on: a set whose FLAT tables -- 369 KB per key or point, one 16-entry
+ * table of affine multiples per digit position, so a multiplication by the key costs additions only and no doubling -- fit
+ * max_table_bytes gets them (default 32 GB: sets of up to 93 000 keys or points); larger sets keep the 41 KB per key layout (ten
+ * columns, forty doublings per call).  0 = never flat. */
 GOLDILOCKS_B200_API void goldilocks_b200_keyset_policy(unsigned long long max_table_bytes);
 GOLDILOCKS_B200_API goldilocks_error_t goldilocks_ed448_verify_keyset_batch(goldilocks_error_t *status, const goldilocks_b200_keyset *keyset, const uint32_t *key_index /*n*/, const uint8_t *signature /*n*114*/, const uint8_t *msg, const size_t *msg_off /*n+1*/, uint8_t prehashed, const uint8_t *context, uint8_t context_len, size_t n);
 /* X448 peer sets (our extension; the 2014 API's "ECDH with a precomputed partner key", BASELINE.md section 1).  A caller whose
@@ -292,6 +293,29 @@ GOLDILOCKS_B200_API size_t goldilocks_b200_decaf_peerset_size(const goldilocks_b
 GOLDILOCKS_B200_API goldilocks_error_t goldilocks_448_direct_scalarmul_peerset_batch(uint8_t *scaled /*n*56*/, goldilocks_error_t *status,
                                                                                      const goldilocks_b200_decaf_peerset *set, const uint32_t *peer_index /*n*/,
                                                                                      const goldilocks_448_scalar_s *scalar, goldilocks_bool_t short_circuit, size_t n);
+/* Point sets (our extension): goldilocks_448_base_double_scalarmul_non_secret, s1 B + s2 P on public inputs, against recurring
+ * points P -- the participant keys a FROST coordinator checks signature shares against, an OPRF server's public key, the long-term
+ * keys of ring and SMP proofs.  A set of m points gets the tables a key set keeps for its keys (goldilocks_b200_keyset_policy
+ * picks the layout: flat, 369 KB per point and no doubling per call, or 41 KB per point and forty doublings), so a call costs
+ * additions against them instead of a window table and 445 doublings.
+ *   Result: out[i] is the group element goldilocks_448_base_double_scalarmul_non_secret(scalar1 + i, points[point_index[i]],
+ *   scalar2 + i) returns: goldilocks_448_point_eq holds and goldilocks_448_point_encode gives the same bytes.  out[i] has canonical
+ *   limbs and all four coordinates valid.  Scalars are below q, as goldilocks_448_scalar_s requires.  The reference's scalar2 = 0
+ *   case is kept: the result is the identity, without scalar1 B.
+ *   Indices: point_index[i] >= m behaves as if the point were the identity (scalar1 B, or the identity when scalar2 = 0).
+ *   Variable time in all of its inputs, like the reference's _non_secret; never pass secrets.
+ *   Points passed to create must satisfy goldilocks_448_point_valid; weakly reduced limbs below 2^60 are accepted.
+ * The call orders the batch by point on the device (a radix sort of the indices), so the lanes of a warp read one table whatever
+ * order the caller used.  The handle belongs to the CUDA device that was current at creation and is never sharded over
+ * goldilocks_b200_set_devices; another device gets FAILURE.  An empty set is valid, n = 0 succeeds, m < 2^32 - 1, n < 2^31
+ * (DESIGN.md decision 22). */
+typedef struct goldilocks_b200_pointset_s goldilocks_b200_pointset;
+GOLDILOCKS_B200_API goldilocks_error_t goldilocks_b200_pointset_create(goldilocks_b200_pointset **set, const goldilocks_448_point_s *points /*m*/, size_t m);
+GOLDILOCKS_B200_API void goldilocks_b200_pointset_destroy(goldilocks_b200_pointset *set);
+GOLDILOCKS_B200_API size_t goldilocks_b200_pointset_size(const goldilocks_b200_pointset *set);
+GOLDILOCKS_B200_API goldilocks_error_t goldilocks_448_base_double_scalarmul_non_secret_pointset_batch(goldilocks_448_point_s *out, const goldilocks_b200_pointset *set,
+                                                                                                      const uint32_t *point_index /*n*/, const goldilocks_448_scalar_s *scalar1,
+                                                                                                      const goldilocks_448_scalar_s *scalar2, size_t n);
 /* Random-linear-combination batch verification (SURVEY 8(f)3; csrc/rlc.cuh): an OPTIONAL fast path for batches in which
  * (nearly) every signature is expected to be valid.  Same arguments and per-element statuses as
  * goldilocks_ed448_verify_batch (eddsa.c:253-306).  Signatures whose R or public key does not decode are rejected up
@@ -349,6 +373,13 @@ GOLDILOCKS_B200_API size_t goldilocks_b200_decaf_peerset_scratch_bytes(size_t n)
 GOLDILOCKS_B200_API goldilocks_error_t goldilocks_448_direct_scalarmul_peerset_batch_dev(uint8_t *scaled, goldilocks_error_t *status, const goldilocks_b200_decaf_peerset *set,
                                                                                          const uint32_t *peer_index, const goldilocks_448_scalar_s *scalar,
                                                                                          goldilocks_bool_t short_circuit, size_t n, void *scratch, void *stream);
+/* scratch of a device-resident point-set call: the sort keys, the order and the sort's temporary storage, about 16 bytes per
+ * element.  The call writes only there and into out, so calls in flight on different streams with different scratch buffers are
+ * independent.  Returns 0 without a usable GPU. */
+GOLDILOCKS_B200_API size_t goldilocks_b200_pointset_scratch_bytes(size_t n);
+GOLDILOCKS_B200_API goldilocks_error_t goldilocks_448_base_double_scalarmul_non_secret_pointset_batch_dev(goldilocks_448_point_s *out, const goldilocks_b200_pointset *set,
+                                                                                                          const uint32_t *point_index, const goldilocks_448_scalar_s *scalar1,
+                                                                                                          const goldilocks_448_scalar_s *scalar2, size_t n, void *scratch, void *stream);
 GOLDILOCKS_B200_API goldilocks_error_t goldilocks_448_precomputed_scalarmul_batch_dev(goldilocks_448_point_s *out, const goldilocks_448_scalar_s *scalar, size_t n, void *stream);
 GOLDILOCKS_B200_API goldilocks_error_t goldilocks_448_gf_mul_batch_dev(uint8_t *out, const uint8_t *a, const uint8_t *b, size_t n, void *stream);
 GOLDILOCKS_B200_API goldilocks_error_t goldilocks_448_point_add_batch_dev(goldilocks_448_point_s *out, const goldilocks_448_point_s *a, const goldilocks_448_point_s *b, size_t n, void *stream);

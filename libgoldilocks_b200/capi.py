@@ -377,6 +377,31 @@ class BatchLib:
         self._call("goldilocks_448_direct_scalarmul_peerset_batch", out, st, handle, peer_index, s, C.c_uint64(ALL if short_circuit else 0), _Z(len(s)))
         return out, st
 
+    # ---- point sets: key-set tables for base_double_scalarmul_non_secret against recurring points ----
+    def pointset_create(self, points):
+        """handle for m point structs ((m,256) u8, each goldilocks_448_point_valid); free it with pointset_destroy"""
+        pts = _u8(points, 256)
+        h = C.c_void_p()
+        self._call("goldilocks_b200_pointset_create", C.byref(h), pts, _Z(len(pts)))
+        return h
+
+    def pointset_destroy(self, handle):
+        self.lib.goldilocks_b200_pointset_destroy.restype = None
+        self.lib.goldilocks_b200_pointset_destroy(handle)
+
+    def pointset_size(self, handle):
+        f = self.lib.goldilocks_b200_pointset_size
+        f.restype = _Z
+        return int(f(handle))
+
+    def pointset(self, handle, point_index, s1, s2):
+        """(n,256) u8: base_double_scalarmul_non_secret(s1[i], point point_index[i] of the set, s2[i]); an index >= m stands for
+        the identity"""
+        s1, s2 = _u8(s1, 56), _u8(s2, 56); point_index = np.ascontiguousarray(point_index, np.uint32).reshape(-1)
+        out = np.empty((len(s1), 256), np.uint8)
+        self._call("goldilocks_448_base_double_scalarmul_non_secret_pointset_batch", out, handle, point_index, s1, s2, _Z(len(s1)))
+        return out
+
     def ed448_verify(self, sig, pk, msgs, prehashed=False, context=b""):
         sig, pk = _u8(sig, 114), _u8(pk, 57)
         arena, off = pack_messages(msgs) if isinstance(msgs, list) else msgs

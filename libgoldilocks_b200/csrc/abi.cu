@@ -1499,13 +1499,32 @@ struct goldilocks_b200_keyset_s {
 /* A set whose flat tables (369 KB per key) fit this many bytes gets them; larger sets keep the 41 KB layout (goldilocks_b200_keyset_policy) */
 std::atomic<unsigned long long> g_keyset_flat_bytes{32ull << 30};
 void goldilocks_b200_keyset_policy(unsigned long long max_table_bytes) { g_keyset_flat_bytes.store(max_table_bytes); }
+static bool keyset_flat(size_t tables) { return (unsigned long long)tables * KSET_QUADS * sizeof(uint4) <= g_keyset_flat_bytes.load(); }
+/* the per-key tables of `count` points into ktabs (key sets and point sets): the flat layout's doubling chain and 90 column tables, or
+ * the ten-column layout; then affine entries -- the set pays one inversion per column once, every call saves a multiplication per addition */
+static void keyset_tables(Call &k, const abi_pt *pts, uint4 *ktabs, size_t count, bool flat) {
+    if (flat) {
+        int grid = k.smp_grid_for<SlotKeysetChain>();
+        SlotKeysetChain fc = {pts, ktabs};
+        k.run_smp(fc, count, grid);
+        grid = k.smp_grid_for<SlotKeysetColumns>();
+        SlotKeysetColumns fcol = {ktabs, k.slots((size_t)grid * SLOT_BLOCK, 1)};
+        k.run_smp(fcol, count * KSET_COLS, grid);
+    } else {
+        int grid = k.smp_grid_for<SlotKeysetTables>();
+        SlotKeysetTables ft = {pts, ktabs};
+        k.run_smp(ft, count, grid);
+    }
+    LaneKeysetNormalize fn = {ktabs, flat ? (uint32_t)KSET_COLS : (uint32_t)VSH_CHUNKS, flat ? (uint32_t)KSET_QUADS : (uint32_t)KTAB_QUADS};
+    k.run(fn, count * (flat ? KSET_COLS : VSH_CHUNKS));
+}
 goldilocks_error_t goldilocks_b200_keyset_create(goldilocks_b200_keyset **out, const uint8_t *pubkeys, size_t m) {
     if (!out) return GOLDILOCKS_FAILURE;
     *out = nullptr;
     Call k;
     if (!k.ok) return k.finish();
     const size_t mm = m ? m : 1;
-    const bool flat = (unsigned long long)mm * KSET_QUADS * sizeof(uint4) <= g_keyset_flat_bytes.load();
+    const bool flat = keyset_flat(mm);
     goldilocks_b200_keyset_s *ks = new goldilocks_b200_keyset_s{k.c->dev, m, nullptr, nullptr, nullptr, flat};
     bool ok = cudaMalloc(&ks->pk, 57 * mm) == cudaSuccess && cudaMalloc(&ks->key_ok, sizeof(int32_t) * mm) == cudaSuccess &&
               cudaMalloc(&ks->ktabs, mm * (flat ? KSET_QUADS : KTAB_QUADS) * sizeof(uint4)) == cudaSuccess;
@@ -1514,21 +1533,7 @@ goldilocks_error_t goldilocks_b200_keyset_create(goldilocks_b200_keyset **out, c
         abi_pt *pts = k.out<abi_pt>(m);
         LaneDecodeEddsa fd = {pts, ks->key_ok, ks->pk};
         k.run(fd, m);
-        if (flat) {
-            int grid = k.smp_grid_for<SlotKeysetChain>();
-            SlotKeysetChain fc = {pts, ks->ktabs};
-            k.run_smp(fc, m, grid);
-            grid = k.smp_grid_for<SlotKeysetColumns>();
-            SlotKeysetColumns fcol = {ks->ktabs, k.slots((size_t)grid * SLOT_BLOCK, 1)};
-            k.run_smp(fcol, m * KSET_COLS, grid);
-        } else {
-            int grid = k.smp_grid_for<SlotKeysetTables>();
-            SlotKeysetTables ft = {pts, ks->ktabs};
-            k.run_smp(ft, m, grid);
-        }
-        /* affine entries: the set pays one inversion per column once, every call saves a multiplication per addition */
-        LaneKeysetNormalize fn = {ks->ktabs, flat ? (uint32_t)KSET_COLS : (uint32_t)VSH_CHUNKS, flat ? (uint32_t)KSET_QUADS : (uint32_t)KTAB_QUADS};
-        k.run(fn, m * (flat ? KSET_COLS : VSH_CHUNKS));
+        keyset_tables(k, pts, ks->ktabs, m, flat);
     }
     goldilocks_error_t r = k.finish();
     if (!ok || r != GOLDILOCKS_SUCCESS) {
@@ -1658,11 +1663,10 @@ static size_t decaf_peer_scratch(DecafPeerScratch *s, void *base, size_t n) {
     }
     return 4 * words + al(sort_bytes);
 }
-/* keys (min(peer_index[j], m), j) -> stable radix sort by peer -> the comb kernel over the elements in that order.  The sort is
- * bracketed like a launch when profiling is on, so goldilocks_b200_profile_timeline shows its share of the call. */
-static bool decaf_peer_enqueue(Ctx &c, uint8_t *scaled, int32_t *status, const goldilocks_b200_decaf_peerset_s *ps, const uint32_t *peer_index,
-                               const abi_sc *scalar, bool short_circuit, size_t n, const DecafPeerScratch &s, cudaStream_t st) {
-    const uint32_t m = (uint32_t)ps->m;
+/* s.order = the elements sorted by set entry: keys (min(peer_index[j], m), j) -> stable radix sort.  Decaf peer sets and point sets
+ * order every call this way.  The sort is bracketed like a launch when profiling is on, so goldilocks_b200_profile_timeline shows
+ * its share of the call. */
+static bool peer_order(Ctx &c, const uint32_t *peer_index, uint32_t m, size_t n, const DecafPeerScratch &s, cudaStream_t st, const char *what) {
     LaneDecafPeerKeys fk = {s.keys, s.vals, peer_index, m};
     if (!launch(c, fk, n, st)) return false;
     int key_bits = 1;
@@ -1672,7 +1676,14 @@ static bool decaf_peer_enqueue(Ctx &c, uint8_t *scaled, int32_t *status, const g
     if (prof) a = prof_begin("pair_sort", st, &b);
     const cudaError_t e = pair_sort(s.sort_tmp, s.sort_bytes, s.keys, s.keys_s, s.vals, s.order, n, key_bits, st);
     if (prof) prof_end("pair_sort", st, a, b);
-    if (e != cudaSuccess) return fail("pair_sort (decaf peer set)", e);
+    if (e != cudaSuccess) return fail(what, e);
+    return true;
+}
+/* the sort by peer, then the comb kernel over the elements in that order */
+static bool decaf_peer_enqueue(Ctx &c, uint8_t *scaled, int32_t *status, const goldilocks_b200_decaf_peerset_s *ps, const uint32_t *peer_index,
+                               const abi_sc *scalar, bool short_circuit, size_t n, const DecafPeerScratch &s, cudaStream_t st) {
+    const uint32_t m = (uint32_t)ps->m;
+    if (!peer_order(c, peer_index, m, n, s, st, "pair_sort (decaf peer set)")) return false;
     SlotDecafPeer f = {scaled, status, ps->tables, ps->peer_ok, peer_index, s.order, scalar, m, short_circuit ? ~0u : 0u};
     return launch_slots(c, f, n, st);
 }
@@ -1732,6 +1743,78 @@ goldilocks_error_t goldilocks_448_direct_scalarmul_peerset_batch(uint8_t *scaled
     return k.finish();
 }
 
+// ---- point sets: key-set tables for goldilocks_448_base_double_scalarmul_non_secret against recurring points (slot_lanes.cuh SlotPointset)
+struct goldilocks_b200_pointset_s {
+    int dev; size_t m;
+    uint4 *ktabs;   /* m + 1 key-set tables (KSET_QUADS each when flat, else KTAB_QUADS); table m, the identity's, stands for every index >= m */
+    bool flat;
+};
+/* the sort by point (as decaf peer sets), then the point-set kernel of the set's layout over the elements in that order */
+static bool pointset_enqueue(Ctx &c, abi_pt *out, const goldilocks_b200_pointset_s *ps, const uint32_t *point_index, const abi_sc *scalar1,
+                             const abi_sc *scalar2, size_t n, const DecafPeerScratch &s, cudaStream_t st, unsigned *counter) {
+    const uint32_t m = (uint32_t)ps->m;
+    if (!peer_order(c, point_index, m, n, s, st, "pair_sort (point set)")) return false;
+    int grid = 1;
+    if (ps->flat) {
+        SlotPointset<true> f = {out, scalar1, scalar2, c.wide, ps->ktabs, point_index, s.order, m};
+        return smp_grid<SlotPointset<true>>(c, &grid) && launch_smp(c, f, n, grid, st, counter);
+    }
+    SlotPointset<false> f = {out, scalar1, scalar2, c.wide, ps->ktabs, point_index, s.order, m};
+    return smp_grid<SlotPointset<false>>(c, &grid) && launch_smp(c, f, n, grid, st, counter);
+}
+goldilocks_error_t goldilocks_b200_pointset_create(goldilocks_b200_pointset **out, const hpt *points, size_t m) {
+    if (!out) return GOLDILOCKS_FAILURE;
+    *out = nullptr;
+    Call k;
+    if (!k.ok) return k.finish();
+    if (m >= UINT32_MAX) { g_err = "goldilocks_b200_pointset_create: at most 2^32 - 2 points"; return GOLDILOCKS_FAILURE; }
+    const size_t mm = m + 1;
+    const bool flat = keyset_flat(mm);
+    goldilocks_b200_pointset_s *ps = new goldilocks_b200_pointset_s{k.c->dev, m, nullptr, flat};
+    bool ok = cudaMalloc(&ps->ktabs, mm * (flat ? KSET_QUADS : KTAB_QUADS) * sizeof(uint4)) == cudaSuccess;
+    if (ok) {
+        static const abi_pt identity = {{{0}}, {{1}}, {{1}}, {{0}}};
+        abi_pt *pts = k.out<abi_pt>(mm);
+        ok = k.ok && (m == 0 || cudaMemcpyAsync(pts, points, sizeof(abi_pt) * m, cudaMemcpyHostToDevice, k.c->stream) == cudaSuccess) &&
+             cudaMemcpyAsync(pts + m, &identity, sizeof(abi_pt), cudaMemcpyHostToDevice, k.c->stream) == cudaSuccess;
+        if (ok) keyset_tables(k, pts, ps->ktabs, mm, flat);
+    }
+    goldilocks_error_t r = k.finish();
+    if (!ok || r != GOLDILOCKS_SUCCESS) {
+        if (!ok) g_err = "goldilocks_b200_pointset_create: device allocation or copy failed";
+        cudaFree(ps->ktabs);
+        delete ps;
+        return GOLDILOCKS_FAILURE;
+    }
+    *out = ps;
+    return GOLDILOCKS_SUCCESS;
+}
+void goldilocks_b200_pointset_destroy(goldilocks_b200_pointset *ps) {
+    if (!ps) return;
+    int cur = 0;
+    const bool sw = cudaGetDevice(&cur) == cudaSuccess && cur != ps->dev && cudaSetDevice(ps->dev) == cudaSuccess;
+    cudaFree(ps->ktabs);
+    if (sw) cudaSetDevice(cur);
+    delete ps;
+}
+size_t goldilocks_b200_pointset_size(const goldilocks_b200_pointset *ps) { return ps ? ps->m : 0; }
+goldilocks_error_t goldilocks_448_base_double_scalarmul_non_secret_pointset_batch(hpt *out, const goldilocks_b200_pointset *ps, const uint32_t *point_index,
+                                                                              const hsc *scalar1, const hsc *scalar2, size_t n) {
+    if (n == 0) return GOLDILOCKS_SUCCESS;
+    Call k;
+    if (!k.ok) return k.finish();
+    if (!ps || ps->dev != k.c->dev) { g_err = "goldilocks_448_base_double_scalarmul_non_secret_pointset_batch: the point set lives on another device"; return GOLDILOCKS_FAILURE; }
+    if (n > (size_t)INT32_MAX) { g_err = "goldilocks_448_base_double_scalarmul_non_secret_pointset_batch: n >= 2^31"; return GOLDILOCKS_FAILURE; }
+    abi_pt *dout = k.out<abi_pt>(n);
+    const uint32_t *didx = k.in(point_index, n);
+    const abi_sc *ds1 = k.in(S(scalar1), n), *ds2 = k.in(S(scalar2), n);
+    DecafPeerScratch s;
+    decaf_peer_scratch(&s, k.alloc(decaf_peer_scratch(nullptr, nullptr, n)), n);
+    if (k.ok) k.ok = pointset_enqueue(*k.c, dout, ps, didx, ds1, ds2, n, s, k.c->stream, nullptr);
+    k.fetch(P(out), dout, n);
+    return k.finish();
+}
+
 // ---- device-resident variants -------------------------------------------------------------------------------
 goldilocks_error_t goldilocks_ed448_verify_batch_dev(goldilocks_error_t *status, const uint8_t *signature, const uint8_t *pubkey, const uint8_t *msg, const size_t *msg_off,
                                                      uint8_t prehashed, const uint8_t *context, uint8_t context_len, size_t n, void *scratch, void *stream) {
@@ -1780,6 +1863,24 @@ goldilocks_error_t goldilocks_448_direct_scalarmul_peerset_batch_dev(uint8_t *sc
     decaf_peer_scratch(&s, scratch, n);
     return decaf_peer_enqueue(*c, scaled, (int32_t *)status, ps, peer_index, S(scalar), short_circuit != 0, n, s, as_stream(stream)) ? GOLDILOCKS_SUCCESS
                                                                                                                                       : GOLDILOCKS_FAILURE;
+}
+size_t goldilocks_b200_pointset_scratch_bytes(size_t n) {
+    if (!dev_ctx()) return 0;
+    return decaf_peer_scratch(nullptr, nullptr, n);
+}
+goldilocks_error_t goldilocks_448_base_double_scalarmul_non_secret_pointset_batch_dev(hpt *out, const goldilocks_b200_pointset *ps, const uint32_t *point_index,
+                                                                                  const hsc *scalar1, const hsc *scalar2, size_t n, void *scratch, void *stream) {
+    if (n == 0) return GOLDILOCKS_SUCCESS;
+    Ctx *c = dev_ctx();
+    if (!c) return GOLDILOCKS_FAILURE;
+    if (!ps || ps->dev != c->dev) { g_err = "goldilocks_448_base_double_scalarmul_non_secret_pointset_batch_dev: the point set lives on another device"; return GOLDILOCKS_FAILURE; }
+    if (n > (size_t)INT32_MAX) { g_err = "goldilocks_448_base_double_scalarmul_non_secret_pointset_batch_dev: n >= 2^31"; return GOLDILOCKS_FAILURE; }
+    if (!scratch) { g_err = "goldilocks_448_base_double_scalarmul_non_secret_pointset_batch_dev: no scratch"; return GOLDILOCKS_FAILURE; }
+    /* the sort lives in the caller's scratch and the kernel takes a fixed grid-stride assignment (no hand-out counter of the
+     * context): calls on different streams do not interfere */
+    DecafPeerScratch s;
+    decaf_peer_scratch(&s, scratch, n);
+    return pointset_enqueue(*c, P(out), ps, point_index, S(scalar1), S(scalar2), n, s, as_stream(stream), GRID_STRIDE) ? GOLDILOCKS_SUCCESS : GOLDILOCKS_FAILURE;
 }
 goldilocks_error_t goldilocks_448_precomputed_scalarmul_batch_dev(hpt *out, const hsc *scalar, size_t n, void *stream) {
     Ctx *c = dev_ctx();

@@ -67,6 +67,7 @@ template <> struct slot_min_blocks<SlotEdVerifyFinishKeyset> { static constexpr 
 template <> struct slot_min_blocks<SlotEdVerifyFinishKeysetFlat> { static constexpr int value = 4; };
 template <> struct slot_min_blocks<SlotKeysetChain> { static constexpr int value = 4; };
 template <> struct slot_min_blocks<SlotKeysetColumns> { static constexpr int value = 4; };
+template <bool FLAT> struct slot_min_blocks<SlotPointset<FLAT>> { static constexpr int value = 4; };
 template <class F>
 cudaError_t launch_sm(const F &f, size_t n, cudaStream_t s) {
     const int smem = F::NSLOTS * 64 * SLOT_BLOCK;
@@ -116,7 +117,7 @@ cudaError_t launch_sm_persist(const F &f, size_t n, int grid, cudaStream_t s, un
 #define LANES_SM(X) X(SlotNielsDebug) X(SlotX448) X(SlotX448Peer) X(SlotComb) X(SlotCombTable) X(SlotDecafPeer) X(SlotX448DerivePk) X(SlotEdDerivePk) X(SlotEdSignR) X(SlotRlcBucket)
 #define INSTANTIATE_SM(F) template cudaError_t launch_sm<F>(const F &, size_t, cudaStream_t);
 #define DECLARE_SM(F) extern INSTANTIATE_SM(F)
-#define LANES_SMP(X) X(SlotEdVerifyFinish) X(SlotEdVerifyFinishShared) X(SlotKeyChain) X(SlotKeyColumns) X(SlotKeysetTables) X(SlotKeysetChain) X(SlotKeysetColumns) X(SlotEdVerifyFinishKeyset) X(SlotEdVerifyFinishKeysetFlat) X(SlotBaseDoubleScalarmul) X(SlotScalarmul) X(SlotDoubleScalarmul) X(SlotDualScalarmul) X(SlotDirectScalarmul)
+#define LANES_SMP(X) X(SlotEdVerifyFinish) X(SlotEdVerifyFinishShared) X(SlotKeyChain) X(SlotKeyColumns) X(SlotKeysetTables) X(SlotKeysetChain) X(SlotKeysetColumns) X(SlotEdVerifyFinishKeyset) X(SlotEdVerifyFinishKeysetFlat) X(SlotPointset<true>) X(SlotPointset<false>) X(SlotBaseDoubleScalarmul) X(SlotScalarmul) X(SlotDoubleScalarmul) X(SlotDualScalarmul) X(SlotDirectScalarmul)
 #define INSTANTIATE_SMP(F)                                                                          \
     template cudaError_t sm_configure<F>(int *);                                                    \
     template cudaError_t launch_sm_persist<F>(const F &, size_t, int, cudaStream_t, unsigned *);

@@ -441,7 +441,8 @@ GD void s_build_key_column(sref sb, const wtab<1> &t, int c, const wtab<1> &scra
 #define KSET_COLS 90
 #define KSET_QUADS (KSET_COLS * WINDOW_NTABLE * 16)
 GD wtab<1> kset_of(uint4 *ktabs, size_t table) { wtab<1> t; t.base = ktabs + table * KSET_QUADS; return t; }
-GD void s_verify_flat_key(sref sb, const sc &scalar1, const sc &scalar2, const niels *wide, const wtab<1> &kt) {
+// need_t: T of the result too (point sets return the point; verification only compares it).
+GD void s_verify_flat_key(sref sb, const sc &scalar1, const sc &scalar2, const niels *wide, const wtab<1> &kt, bool need_t = false) {
     const spt p = {s_slot(sb, 0), s_slot(sb, 1), s_slot(sb, 2), s_slot(sb, 3)};
     const swk w = {s_slot(sb, 4), s_slot(sb, 5), s_slot(sb, 6)};
     sc s1x, s2x;
@@ -458,12 +459,14 @@ GD void s_verify_flat_key(sref sb, const sc &scalar1, const sc &scalar2, const n
         const int e2 = k * WINDOW_NTABLE + (int)(bits2 & (WINDOW_NTABLE - 1));
         s_pt_add_niels_g<1>(p, w, kt.coord(e2, 0), kt.coord(e2, 1), kt.coord(e2, 2), inv2, ~inv2, false);
     }
-    s_add_fixed_base(p, w, s1x, wide, false);
+    s_add_fixed_base(p, w, s1x, wide, need_t);
 }
 // combo (slots 0..3) = scalar1*B + scalar2*A with A's tables in `kt`; `wide` = the init-time tables of the fixed base.
 // AFFINE: the entries have been divided by their z (key sets, LaneKeysetNormalize): 7 multiplications per addition instead of 8.
+// need_t as in s_verify_flat_key.
 template <bool AFFINE = false>
-GD void s_verify_shared_key(sref sb, const sc &scalar1, const sc &scalar2, const niels *wide, const wtab<1> &kt, int rows = VSH_ROWS, int chunks = VSH_CHUNKS) {
+GD void s_verify_shared_key(sref sb, const sc &scalar1, const sc &scalar2, const niels *wide, const wtab<1> &kt, int rows = VSH_ROWS, int chunks = VSH_CHUNKS,
+                            bool need_t = false) {
     const spt p = {s_slot(sb, 0), s_slot(sb, 1), s_slot(sb, 2), s_slot(sb, 3)};
     const swk w = {s_slot(sb, 4), s_slot(sb, 5), s_slot(sb, 6)};
     sc s1x, s2x;
@@ -499,7 +502,7 @@ GD void s_verify_shared_key(sref sb, const sc &scalar1, const sc &scalar2, const
             else s_pt_add_pniels_g<1>(p, w, kt, e2, inv2, ~inv2, row_ends);
         }
     }
-    s_add_fixed_base(p, w, s1x, wide, false);
+    s_add_fixed_base(p, w, s1x, wide, need_t);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -532,6 +532,30 @@ struct SlotDecafPeer {
         words_store56(scaled + 56 * i, wd);
     }
 };
+// Point sets (include/goldilocks_b200.h, goldilocks_b200_pointset_*; DESIGN.md decision 22): goldilocks_448_base_double_scalarmul_non_secret
+// (goldilocks.c:1260-1330) against a recurring point, from the tables a key set keeps for its keys (flat: FLAT = true, or the compact
+// ten-column layout).  Both evaluations add the same sc_recode_signed digits of scalar2 times the same multiples of the point as
+// s_base_double_scalarmul, and scalar1 B from the same fixed-base tables, so they give the same point, torsion included.  Table m of
+// the set is the identity's: an index >= m is clamped to it, so the kernel never branches on the index.  Lane j handles element
+// i = order[j] (the batch sorted by point, LaneDecafPeerKeys) and writes out[i] in place.  Variable time, like the reference's _non_secret.
+template <bool FLAT>
+struct SlotPointset {
+    static constexpr int NSLOTS = BDSM_NSLOTS;
+    abi_pt *out; const abi_sc *scalar1, *scalar2; const niels *wide; const uint4 *ktabs; const uint32_t *point_index, *order; uint32_t n_points;
+    GDM void operator()(size_t j, sref sb, size_t slot) const {
+        (void)slot;
+        const size_t i = order[j];
+        const uint32_t ti = point_index[i];
+        const size_t t = ti < n_points ? ti : n_points;
+        sc s1, s2;
+        sc_from_abi(s1, scalar1 + i);
+        sc_from_abi(s2, scalar2 + i);
+        if (FLAT) s_verify_flat_key(sb, s1, s2, wide, kset_of(const_cast<uint4 *>(ktabs), t), true);
+        else s_verify_shared_key<true>(sb, s1, s2, wide, ktab_of(const_cast<uint4 *>(ktabs), t), VSH_ROWS, VSH_CHUNKS, true);   /* affine entries */
+        s_bdsm_quirk(sb, s2);
+        s_pt_to_abi(out + i, sb);
+    }
+};
 struct SlotEdDerivePk { /* eddsa.c:129-144 */
     static constexpr int NSLOTS = COMB_NSLOTS;
     uint8_t *pk; const uint8_t *sk; const fixed_tables *ft;

@@ -111,6 +111,18 @@ class DeviceEngine:
         self._call("goldilocks_448_direct_scalarmul_peerset_batch_dev", self._p(scaled), self._p(status), handle, self._p(peer_index), self._p(scalars),
                    C.c_uint64((1 << 64) - 1 if short_circuit else 0), _Z(status.numel()), self._p(scratch), self._stream())
 
+    def pointset_scratch_bytes(self, n):
+        f = self.lib.goldilocks_b200_pointset_scratch_bytes
+        f.restype = _Z
+        f.argtypes = [_Z]
+        return int(f(n))
+
+    def pointset(self, out, handle, point_index, s1, s2, scratch):
+        """base_double_scalarmul_non_secret of scalar structs s1[i], s2[i] against point point_index[i] (uint32 tensor viewed as int32)
+        of a set made by capi pointset_create, into the point structs `out`; `scratch` holds pointset_scratch_bytes(n)"""
+        self._call("goldilocks_448_base_double_scalarmul_non_secret_pointset_batch_dev", self._p(out), handle, self._p(point_index), self._p(s1), self._p(s2),
+                   _Z(point_index.numel()), self._p(scratch), self._stream())
+
     def precomputed_scalarmul(self, out_pts, scalars):
         self._call("goldilocks_448_precomputed_scalarmul_batch_dev", self._p(out_pts), self._p(scalars), _Z(scalars.numel() // 56), self._stream())
 
