@@ -259,6 +259,19 @@ GOLDILOCKS_B200_API size_t goldilocks_b200_keyset_size(const goldilocks_b200_key
  * columns, forty doublings per call).  0 = never flat. */
 GOLDILOCKS_B200_API void goldilocks_b200_keyset_policy(unsigned long long max_table_bytes);
 GOLDILOCKS_B200_API goldilocks_error_t goldilocks_ed448_verify_keyset_batch(goldilocks_error_t *status, const goldilocks_b200_keyset *keyset, const uint32_t *key_index /*n*/, const uint8_t *signature /*n*114*/, const uint8_t *msg, const size_t *msg_off /*n+1*/, uint8_t prehashed, const uint8_t *context, uint8_t context_len, size_t n);
+/* Verification by public-key bytes against a key set (our extension; DESIGN.md decision 23): the arguments of
+ * goldilocks_ed448_verify_batch plus a key set, for a verifier that knows most of its signers but gets (signature, key, message)
+ * rather than key indices.  status[i] is exactly what goldilocks_ed448_verify(signature i, pubkey i, message i, prehashed,
+ * context) returns, for every i.  Signatures whose 57 key bytes equal a key of the set use its tables; the others go through
+ * goldilocks_ed448_verify_batch's path (grouped by key within the call when there are 64 or more of them).  key_index (may be
+ * NULL) receives, per element, the lowest set index whose 57 bytes equal pubkey i, or m when there is none.  A key of the set
+ * that does not decode is still a hit and rejects its signatures, as goldilocks_ed448_verify does; duplicate keys in a set are
+ * allowed.  The lookup is a binary search over the set's keys in byte order (kept by goldilocks_b200_keyset_create, 4 bytes per
+ * key), so its cost does not depend on which keys the set holds.  Everything is public and the call is variable time.  The
+ * handle belongs to the CUDA device that was current at creation (another device gets FAILURE) and is never sharded over
+ * goldilocks_b200_set_devices.  An empty set is valid: every element misses and the result is goldilocks_ed448_verify_batch's.
+ * n = 0 succeeds, n < 2^31. */
+GOLDILOCKS_B200_API goldilocks_error_t goldilocks_ed448_verify_keyset_lookup_batch(goldilocks_error_t *status, uint32_t *key_index /*n, or NULL*/, const goldilocks_b200_keyset *keyset, const uint8_t *signature /*n*114*/, const uint8_t *pubkey /*n*57*/, const uint8_t *msg, const size_t *msg_off /*n+1*/, uint8_t prehashed, const uint8_t *context, uint8_t context_len, size_t n);
 /* X448 peer sets (our extension; the 2014 API's "ECDH with a precomputed partner key", BASELINE.md section 1).  A caller whose
  * fresh secret scalars keep meeting the same public u-coordinates -- HPKE / ECIES to a known recipient, onion packets to a fixed
  * relay set -- builds a set of m peers once: each peer on the curve gets the reference's (5,5,18) comb table of a point that
@@ -380,6 +393,21 @@ GOLDILOCKS_B200_API size_t goldilocks_b200_pointset_scratch_bytes(size_t n);
 GOLDILOCKS_B200_API goldilocks_error_t goldilocks_448_base_double_scalarmul_non_secret_pointset_batch_dev(goldilocks_448_point_s *out, const goldilocks_b200_pointset *set,
                                                                                                           const uint32_t *point_index, const goldilocks_448_scalar_s *scalar1,
                                                                                                           const goldilocks_448_scalar_s *scalar2, size_t n, void *scratch, void *stream);
+/* scratch of the device-resident key-set calls below, for n signatures and msg_bytes (= msg_off[n]) bytes of messages: the
+ * looked-up indices and their order, scalars, the sign-check records, the misses packed, and goldilocks_b200_verify_scratch_bytes(n)
+ * for them.  Returns 0 without a usable GPU. */
+GOLDILOCKS_B200_API size_t goldilocks_b200_keyset_scratch_bytes(size_t n, size_t msg_bytes);
+/* device-pointer form of goldilocks_ed448_verify_keyset_lookup_batch; scratch >= goldilocks_b200_keyset_scratch_bytes(n, msg_off[n]).
+ * The call synchronises `stream` ONCE, after the lookup (it needs the number of misses on the host), then queues the rest and
+ * returns: the statuses are written when `stream` reaches that point.  It writes only into scratch, status and key_index. */
+GOLDILOCKS_B200_API goldilocks_error_t goldilocks_ed448_verify_keyset_lookup_batch_dev(goldilocks_error_t *status, uint32_t *key_index /*or NULL*/, const goldilocks_b200_keyset *keyset,
+                                                                                       const uint8_t *signature, const uint8_t *pubkey, const uint8_t *msg, const size_t *msg_off,
+                                                                                       uint8_t prehashed, const uint8_t *context /*device or NULL*/, uint8_t context_len, size_t n,
+                                                                                       void *scratch, void *stream);
+/* device-pointer form of goldilocks_ed448_verify_keyset_batch (indices already known); asynchronous on `stream`, scratch as above */
+GOLDILOCKS_B200_API goldilocks_error_t goldilocks_ed448_verify_keyset_batch_dev(goldilocks_error_t *status, const goldilocks_b200_keyset *keyset, const uint32_t *key_index,
+                                                                                const uint8_t *signature, const uint8_t *msg, const size_t *msg_off, uint8_t prehashed,
+                                                                                const uint8_t *context /*device or NULL*/, uint8_t context_len, size_t n, void *scratch, void *stream);
 GOLDILOCKS_B200_API goldilocks_error_t goldilocks_448_precomputed_scalarmul_batch_dev(goldilocks_448_point_s *out, const goldilocks_448_scalar_s *scalar, size_t n, void *stream);
 GOLDILOCKS_B200_API goldilocks_error_t goldilocks_448_gf_mul_batch_dev(uint8_t *out, const uint8_t *a, const uint8_t *b, size_t n, void *stream);
 GOLDILOCKS_B200_API goldilocks_error_t goldilocks_448_point_add_batch_dev(goldilocks_448_point_s *out, const goldilocks_448_point_s *a, const goldilocks_448_point_s *b, size_t n, void *stream);

@@ -328,6 +328,19 @@ class BatchLib:
         self._call("goldilocks_ed448_verify_keyset_batch", st, handle, key_index, sig, arena, off, C.c_uint8(1 if prehashed else 0), ctx, C.c_uint8(ctx_len), _Z(len(sig)))
         return st
 
+    def ed448_verify_keyset_lookup(self, handle, sig, pk, msgs, prehashed=False, context=b"", return_index=False):
+        """status int32[n] of signature i under public key pk[i] ((n,57) u8), exactly goldilocks_ed448_verify's; keys found in the set
+        use its tables, the rest the ordinary path.  With return_index: (status, key_index uint32[n]), the lowest set index whose
+        57 bytes equal pk[i], or m"""
+        sig, pk = _u8(sig, 114), _u8(pk, 57)
+        arena, off = pack_messages(msgs) if isinstance(msgs, list) else msgs
+        ctx, ctx_len = self._ctx(context)
+        st = np.zeros(len(sig), np.int32)
+        idx = np.zeros(len(sig), np.uint32) if return_index else None
+        self._call("goldilocks_ed448_verify_keyset_lookup_batch", st, idx, handle, sig, pk, arena, off, C.c_uint8(1 if prehashed else 0), ctx, C.c_uint8(ctx_len),
+                   _Z(len(sig)))
+        return (st, idx) if return_index else st
+
     # ---- X448 peer sets: per-peer comb tables kept on the device across calls ----
     def x448_peerset_create(self, peers):
         """handle for m peer u-coordinates ((m,56) u8); free it with x448_peerset_destroy"""

@@ -1495,6 +1495,7 @@ struct goldilocks_b200_keyset_s {
     int32_t *key_ok;  /* decode status per key */
     uint4 *ktabs;     /* m tables of KTAB_QUADS quads (10 columns x 9 rows), or of KSET_QUADS (flat: a column per digit position) */
     bool flat;
+    uint32_t *sorted; /* the m indices ordered by key bytes (memcmp), ties by index: the lookup calls' binary search (LaneKeysetLookup) */
 };
 /* A set whose flat tables (369 KB per key) fit this many bytes gets them; larger sets keep the 41 KB layout (goldilocks_b200_keyset_policy) */
 std::atomic<unsigned long long> g_keyset_flat_bytes{32ull << 30};
@@ -1525,11 +1526,17 @@ goldilocks_error_t goldilocks_b200_keyset_create(goldilocks_b200_keyset **out, c
     if (!k.ok) return k.finish();
     const size_t mm = m ? m : 1;
     const bool flat = keyset_flat(mm);
-    goldilocks_b200_keyset_s *ks = new goldilocks_b200_keyset_s{k.c->dev, m, nullptr, nullptr, nullptr, flat};
+    goldilocks_b200_keyset_s *ks = new goldilocks_b200_keyset_s{k.c->dev, m, nullptr, nullptr, nullptr, flat, nullptr};
     bool ok = cudaMalloc(&ks->pk, 57 * mm) == cudaSuccess && cudaMalloc(&ks->key_ok, sizeof(int32_t) * mm) == cudaSuccess &&
-              cudaMalloc(&ks->ktabs, mm * (flat ? KSET_QUADS : KTAB_QUADS) * sizeof(uint4)) == cudaSuccess;
+              cudaMalloc(&ks->ktabs, mm * (flat ? KSET_QUADS : KTAB_QUADS) * sizeof(uint4)) == cudaSuccess &&
+              cudaMalloc(&ks->sorted, sizeof(uint32_t) * mm) == cudaSuccess;
+    /* the bytes are on the host already: sort there (a byte order, not a hash order -- nobody can make the search longer) */
+    std::vector<uint32_t> sorted(m);
+    for (size_t i = 0; i < m; i++) sorted[i] = (uint32_t)i;
+    std::stable_sort(sorted.begin(), sorted.end(), [pubkeys](uint32_t a, uint32_t b) { return memcmp(pubkeys + 57 * (size_t)a, pubkeys + 57 * (size_t)b, 57) < 0; });
     if (ok && m) {
-        ok = cudaMemcpyAsync(ks->pk, pubkeys, 57 * m, cudaMemcpyHostToDevice, k.c->stream) == cudaSuccess;
+        ok = cudaMemcpyAsync(ks->pk, pubkeys, 57 * m, cudaMemcpyHostToDevice, k.c->stream) == cudaSuccess &&
+             cudaMemcpyAsync(ks->sorted, sorted.data(), sizeof(uint32_t) * m, cudaMemcpyHostToDevice, k.c->stream) == cudaSuccess;
         abi_pt *pts = k.out<abi_pt>(m);
         LaneDecodeEddsa fd = {pts, ks->key_ok, ks->pk};
         k.run(fd, m);
@@ -1538,7 +1545,7 @@ goldilocks_error_t goldilocks_b200_keyset_create(goldilocks_b200_keyset **out, c
     goldilocks_error_t r = k.finish();
     if (!ok || r != GOLDILOCKS_SUCCESS) {
         if (!ok) g_err = "goldilocks_b200_keyset_create: device allocation or copy failed";
-        cudaFree(ks->pk); cudaFree(ks->key_ok); cudaFree(ks->ktabs);
+        cudaFree(ks->pk); cudaFree(ks->key_ok); cudaFree(ks->ktabs); cudaFree(ks->sorted);
         delete ks;
         return GOLDILOCKS_FAILURE;
     }
@@ -1549,11 +1556,28 @@ void goldilocks_b200_keyset_destroy(goldilocks_b200_keyset *ks) {
     if (!ks) return;
     int cur = 0;
     const bool sw = cudaGetDevice(&cur) == cudaSuccess && cur != ks->dev && cudaSetDevice(ks->dev) == cudaSuccess;
-    cudaFree(ks->pk); cudaFree(ks->key_ok); cudaFree(ks->ktabs);
+    cudaFree(ks->pk); cudaFree(ks->key_ok); cudaFree(ks->ktabs); cudaFree(ks->sorted);
     if (sw) cudaSetDevice(cur);
     delete ks;
 }
 size_t goldilocks_b200_keyset_size(const goldilocks_b200_keyset *ks) { return ks ? ks->m : 0; }
+/* the index form on device buffers: challenges under the set's key bytes, the finish kernel of the set's layout, the sign check */
+static bool keyset_enqueue(Ctx &c, int32_t *status, const goldilocks_b200_keyset_s *ks, const uint32_t *key_index, const uint8_t *sig, const uint8_t *msg,
+                           const size_t *off, uint8_t prehashed, const uint8_t *ctx, uint8_t ctx_len, size_t n, abi_sc *chal, abi_sc *resp, verify_aux *aux,
+                           cudaStream_t st, unsigned *counter) {
+    LaneEdVerifyScalars f2 = {chal, resp, sig, ks->pk, msg, off, prehashed, ctx, ctx_len, 0, key_index, (uint32_t)ks->m};
+    if (!launch(c, f2, n, st)) return false;
+    int grid = 1;
+    if (ks->flat) {
+        SlotEdVerifyFinishKeysetFlat f3 = {aux, ks->key_ok, chal, resp, c.wide, ks->ktabs, key_index, (uint32_t)ks->m, sig};
+        if (!smp_grid<SlotEdVerifyFinishKeysetFlat>(c, &grid) || !launch_smp(c, f3, n, grid, st, counter)) return false;
+    } else {
+        SlotEdVerifyFinishKeyset f3 = {aux, ks->key_ok, chal, resp, c.wide, ks->ktabs, key_index, (uint32_t)ks->m, sig};
+        if (!smp_grid<SlotEdVerifyFinishKeyset>(c, &grid) || !launch_smp(c, f3, n, grid, st, counter)) return false;
+    }
+    LaneVerifySign fv = {status, aux, 1, n};
+    return launch(c, fv, (n + VSIGN_BATCH - 1) / VSIGN_BATCH, st);
+}
 goldilocks_error_t goldilocks_ed448_verify_keyset_batch(goldilocks_error_t *status, const goldilocks_b200_keyset *ks, const uint32_t *key_index,
                                                         const uint8_t *signature, const uint8_t *msg, const size_t *msg_off, uint8_t prehashed,
                                                         const uint8_t *context, uint8_t context_len, size_t n) {
@@ -1568,20 +1592,8 @@ goldilocks_error_t goldilocks_ed448_verify_keyset_batch(goldilocks_error_t *stat
     const uint8_t *dsig = k.in(signature, 114 * n), *dmsg = k.in(msg, total);
     int32_t *dst = k.out<int32_t>(n);
     abi_sc *chal = k.out<abi_sc>(n), *resp = k.out<abi_sc>(n);
-    LaneEdVerifyScalars f2 = {chal, resp, dsig, ks->pk, dmsg, doff, prehashed, dctx, context_len, 0, dki, (uint32_t)ks->m};
-    k.run(f2, n);
     verify_aux *aux = k.out<verify_aux>(n);
-    if (ks->flat) {
-        int grid = k.smp_grid_for<SlotEdVerifyFinishKeysetFlat>();
-        SlotEdVerifyFinishKeysetFlat f3 = {aux, ks->key_ok, chal, resp, k.ok ? k.c->wide : nullptr, ks->ktabs, dki, (uint32_t)ks->m, dsig};
-        k.run_smp(f3, n, grid);
-    } else {
-        int grid = k.smp_grid_for<SlotEdVerifyFinishKeyset>();
-        SlotEdVerifyFinishKeyset f3 = {aux, ks->key_ok, chal, resp, k.ok ? k.c->wide : nullptr, ks->ktabs, dki, (uint32_t)ks->m, dsig};
-        k.run_smp(f3, n, grid);
-    }
-    LaneVerifySign fv = {dst, aux, 1, n};
-    k.run(fv, (n + VSIGN_BATCH - 1) / VSIGN_BATCH);
+    if (k.ok) k.ok = keyset_enqueue(*k.c, dst, ks, dki, dsig, dmsg, doff, prehashed, dctx, context_len, n, chal, resp, aux, k.c->stream, nullptr);
     k.fetch((int32_t *)status, dst, n);
     return k.finish();
 }
@@ -1815,6 +1827,124 @@ goldilocks_error_t goldilocks_448_base_double_scalarmul_non_secret_pointset_batc
     return k.finish();
 }
 
+// ---- key-set lookup: verification by public-key bytes against a key set, the keys outside it through the ordinary path --------
+// Looked-up index per element (LaneKeysetLookup) -> the order of the decaf peer sets (hits grouped by key, the misses as one tail)
+// -> the miss count, read back once -> the hits through the ordered key-set finish kernel, the misses packed and through verify_dev
+// unchanged -> every status scattered back to its element.
+struct KeysetLookupScratch {
+    DecafPeerScratch peer;
+    uint32_t *idx, *hits;
+    abi_sc *chal, *resp;
+    verify_aux *aux;
+    int32_t *st;                 /* statuses in sorted order: the hits', then the misses' */
+    uint8_t *sig2, *pk2;         /* the misses, packed */
+    size_t *len, *off2;
+    void *scan_tmp; size_t scan_bytes;
+    void *verify; uint4 *slots;  /* verify_dev's scratch and window tables, sized for n misses */
+    uint8_t *msg2;               /* last: msg_bytes of it */
+};
+static size_t keyset_lookup_scratch(KeysetLookupScratch *s, void *base, size_t n, size_t msg_bytes, const VerifyGrids &g) {
+    auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
+    char *p = (char *)base;
+    size_t used = 0;
+    auto take = [&](size_t bytes) { void *r = p ? p + used : nullptr; used += al(bytes); return r; };
+    DecafPeerScratch peer;
+    void *pb = take(decaf_peer_scratch(nullptr, nullptr, n));
+    if (s) decaf_peer_scratch(&peer, pb, n);
+    uint32_t *idx = (uint32_t *)take(sizeof(uint32_t) * n), *hits = (uint32_t *)take(sizeof(uint32_t));
+    abi_sc *chal = (abi_sc *)take(sizeof(abi_sc) * n), *resp = (abi_sc *)take(sizeof(abi_sc) * n);
+    verify_aux *aux = (verify_aux *)take(sizeof(verify_aux) * n);
+    int32_t *st = (int32_t *)take(sizeof(int32_t) * n);
+    uint8_t *sig2 = (uint8_t *)take(114 * n), *pk2 = (uint8_t *)take(57 * n);
+    size_t *len = (size_t *)take(sizeof(size_t) * (n + 1)), *off2 = (size_t *)take(sizeof(size_t) * (n + 1));
+    const size_t scan_bytes = length_scan_scratch_bytes(n + 1);
+    void *scan_tmp = take(scan_bytes);
+    void *verify = take(verify_core_scratch_bytes(n));
+    uint4 *slots = (uint4 *)take(verify_slot_bytes(g, n));
+    uint8_t *msg2 = (uint8_t *)take(msg_bytes);
+    if (s) *s = {peer, idx, hits, chal, resp, aux, st, sig2, pk2, len, off2, scan_tmp, scan_bytes, verify, slots, msg2};
+    return used;
+}
+/* the first half: looked-up indices into idx, the order, the number of hits on the host (synchronises st) */
+static bool keyset_lookup_order(Ctx &c, uint32_t *idx, const goldilocks_b200_keyset_s *ks, const uint8_t *pk, size_t n, const KeysetLookupScratch &s,
+                                cudaStream_t st, size_t *hits) {
+    const uint32_t m = (uint32_t)ks->m;
+    LaneKeysetLookup fl = {idx, pk, ks->pk, ks->sorted, m};
+    if (!launch(c, fl, n, st) || !peer_order(c, idx, m, n, s.peer, st, "pair_sort (key set lookup)")) return false;
+    LaneKeysetHits fh = {s.hits, s.peer.keys_s, m, n};
+    if (!launch(c, fh, n, st)) return false;
+    uint32_t h = 0;
+    CU(cudaMemcpyAsync(&h, s.hits, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    *hits = h;
+    return true;
+}
+/* the second half: hits through the key set, misses through verify_dev (on `side` beside it where verify_dev forks), statuses back */
+static bool keyset_lookup_verify(Ctx &c, int32_t *status, const goldilocks_b200_keyset_s *ks, const uint32_t *idx, const uint8_t *sig, const uint8_t *pk,
+                                 const uint8_t *msg, const size_t *off, uint8_t prehashed, const uint8_t *ctx, uint8_t ctx_len, size_t n, size_t hits,
+                                 const KeysetLookupScratch &s, const VerifyGrids &grids, cudaStream_t st, unsigned *counter, cudaStream_t side, cudaEvent_t *side_evt) {
+    if (hits) {
+        LaneEdVerifyScalars f2 = {s.chal, s.resp, sig, pk, msg, off, prehashed, ctx, ctx_len, 0};   /* a hit's key bytes are its set key's */
+        if (!launch(c, f2, n, st)) return false;
+        int grid = 1;
+        if (ks->flat) {
+            SlotEdVerifyFinishKeysetOrdered<true> f3 = {s.aux, ks->key_ok, s.chal, s.resp, c.wide, ks->ktabs, idx, s.peer.order, sig};
+            if (!smp_grid<SlotEdVerifyFinishKeysetOrdered<true>>(c, &grid) || !launch_smp(c, f3, hits, grid, st, counter)) return false;
+        } else {
+            SlotEdVerifyFinishKeysetOrdered<false> f3 = {s.aux, ks->key_ok, s.chal, s.resp, c.wide, ks->ktabs, idx, s.peer.order, sig};
+            if (!smp_grid<SlotEdVerifyFinishKeysetOrdered<false>>(c, &grid) || !launch_smp(c, f3, hits, grid, st, counter)) return false;
+        }
+        LaneVerifySign fv = {s.st, s.aux, 1, hits};
+        if (!launch(c, fv, (hits + VSIGN_BATCH - 1) / VSIGN_BATCH, st)) return false;
+    }
+    const size_t misses = n - hits;
+    if (misses) {
+        LaneKeysetMissLengths fl = {s.len, off, s.peer.order, hits, misses};
+        if (!launch(c, fl, misses + 1, st)) return false;
+        CU(length_scan(s.scan_tmp, s.scan_bytes, s.len, s.off2, misses + 1, st));
+        LaneKeysetMissGather fg = {s.sig2, s.pk2, s.msg2, s.off2, sig, pk, msg, off, s.peer.order, hits};
+        if (!launch(c, fg, misses, st)) return false;
+        if (!verify_dev(c, s.st + hits, s.sig2, s.pk2, s.msg2, s.off2, prehashed, ctx, ctx_len, misses, s.verify, s.slots, grids, st, nullptr, side, side_evt))
+            return false;
+    }
+    LaneKeysetScatter fs = {status, s.st, s.peer.order};
+    return launch(c, fs, n, st);
+}
+goldilocks_error_t goldilocks_ed448_verify_keyset_lookup_batch(goldilocks_error_t *status, uint32_t *key_index, const goldilocks_b200_keyset *ks, const uint8_t *signature,
+                                                               const uint8_t *pubkey, const uint8_t *msg, const size_t *msg_off, uint8_t prehashed,
+                                                               const uint8_t *context, uint8_t context_len, size_t n) {
+    if (n == 0) return GOLDILOCKS_SUCCESS;
+    Call k;
+    if (!k.ok) return k.finish();
+    if (!ks || ks->dev != k.c->dev) { g_err = "goldilocks_ed448_verify_keyset_lookup_batch: the key set lives on another device"; return GOLDILOCKS_FAILURE; }
+    if (n > (size_t)INT32_MAX) { g_err = "goldilocks_ed448_verify_keyset_lookup_batch: n >= 2^31"; return GOLDILOCKS_FAILURE; }
+    /* the keys first, as goldilocks_ed448_verify_batch: the lookup, the sort and the read-back of the miss count run while the
+     * signatures and messages still cross PCIe on the copy stream */
+    const size_t total = msg_off[n];
+    const size_t *doff = k.in(msg_off, n + 1);
+    const uint8_t *dctx = k.in(context, context_len);
+    const uint8_t *dpk = k.in(pubkey, 57 * n);
+    uint8_t *dsig = k.out<uint8_t>(114 * n), *dmsg = k.out<uint8_t>(total);
+    int32_t *dst = k.out<int32_t>(n);
+    k.push(dsig, signature, 114 * n);
+    k.push(dmsg, msg, total);
+    if (k.ok && cudaEventRecord(k.c->copy_done[0], k.c->copy_stream) != cudaSuccess) k.ok = false;
+    VerifyGrids grids;
+    if (k.ok) k.ok = verify_grids(*k.c, &grids);
+    KeysetLookupScratch s = {};
+    void *base = k.alloc(keyset_lookup_scratch(nullptr, nullptr, n, total, grids));
+    if (k.ok) keyset_lookup_scratch(&s, base, n, total, grids);
+    size_t hits = 0;
+    if (k.ok) k.ok = keyset_lookup_order(*k.c, s.idx, ks, dpk, n, s, k.c->stream, &hits);
+    if (k.ok) k.ok = cudaStreamWaitEvent(k.c->stream, k.c->copy_done[0], 0) == cudaSuccess;
+    if (k.ok) k.ok = keyset_lookup_verify(*k.c, dst, ks, s.idx, dsig, dpk, dmsg, doff, prehashed, dctx, context_len, n, hits, s, grids, k.c->stream, nullptr,
+                                          k.c->side_stream, k.c->side_evt);
+    k.fetch((int32_t *)status, dst, n);
+    if (key_index) k.fetch(key_index, s.idx, n);
+    if (!k.ok && k.c) cudaStreamSynchronize(k.c->copy_stream); /* never leave copies in flight behind an error */
+    return k.finish();
+}
+
 // ---- device-resident variants -------------------------------------------------------------------------------
 goldilocks_error_t goldilocks_ed448_verify_batch_dev(goldilocks_error_t *status, const uint8_t *signature, const uint8_t *pubkey, const uint8_t *msg, const size_t *msg_off,
                                                      uint8_t prehashed, const uint8_t *context, uint8_t context_len, size_t n, void *scratch, void *stream) {
@@ -1881,6 +2011,51 @@ goldilocks_error_t goldilocks_448_base_double_scalarmul_non_secret_pointset_batc
     DecafPeerScratch s;
     decaf_peer_scratch(&s, scratch, n);
     return pointset_enqueue(*c, P(out), ps, point_index, S(scalar1), S(scalar2), n, s, as_stream(stream), GRID_STRIDE) ? GOLDILOCKS_SUCCESS : GOLDILOCKS_FAILURE;
+}
+size_t goldilocks_b200_keyset_scratch_bytes(size_t n, size_t msg_bytes) {
+    Ctx *c = dev_ctx();
+    VerifyGrids grids;
+    if (!c || !verify_grids(*c, &grids)) return 0;
+    return keyset_lookup_scratch(nullptr, nullptr, n, msg_bytes, grids);
+}
+goldilocks_error_t goldilocks_ed448_verify_keyset_batch_dev(goldilocks_error_t *status, const goldilocks_b200_keyset *ks, const uint32_t *key_index,
+                                                            const uint8_t *signature, const uint8_t *msg, const size_t *msg_off, uint8_t prehashed,
+                                                            const uint8_t *context, uint8_t context_len, size_t n, void *scratch, void *stream) {
+    if (n == 0) return GOLDILOCKS_SUCCESS;
+    Ctx *c = dev_ctx();
+    if (!c) return GOLDILOCKS_FAILURE;
+    if (!ks || ks->dev != c->dev) { g_err = "goldilocks_ed448_verify_keyset_batch_dev: the key set lives on another device"; return GOLDILOCKS_FAILURE; }
+    if (n > (size_t)INT32_MAX) { g_err = "goldilocks_ed448_verify_keyset_batch_dev: n >= 2^31"; return GOLDILOCKS_FAILURE; }
+    if (!scratch) { g_err = "goldilocks_ed448_verify_keyset_batch_dev: no scratch"; return GOLDILOCKS_FAILURE; }
+    VerifyGrids grids;
+    if (!verify_grids(*c, &grids)) return GOLDILOCKS_FAILURE;
+    KeysetLookupScratch s = {};
+    keyset_lookup_scratch(&s, scratch, n, 0, grids);
+    /* fixed grid-stride assignment (no hand-out counter of the context): calls on different streams do not interfere */
+    return keyset_enqueue(*c, (int32_t *)status, ks, key_index, signature, msg, msg_off, prehashed, context, context_len, n, s.chal, s.resp, s.aux,
+                          as_stream(stream), GRID_STRIDE) ? GOLDILOCKS_SUCCESS : GOLDILOCKS_FAILURE;
+}
+goldilocks_error_t goldilocks_ed448_verify_keyset_lookup_batch_dev(goldilocks_error_t *status, uint32_t *key_index, const goldilocks_b200_keyset *ks,
+                                                                   const uint8_t *signature, const uint8_t *pubkey, const uint8_t *msg, const size_t *msg_off,
+                                                                   uint8_t prehashed, const uint8_t *context, uint8_t context_len, size_t n, void *scratch, void *stream) {
+    if (n == 0) return GOLDILOCKS_SUCCESS;
+    Ctx *c = dev_ctx();
+    if (!c) return GOLDILOCKS_FAILURE;
+    if (!ks || ks->dev != c->dev) { g_err = "goldilocks_ed448_verify_keyset_lookup_batch_dev: the key set lives on another device"; return GOLDILOCKS_FAILURE; }
+    if (n > (size_t)INT32_MAX) { g_err = "goldilocks_ed448_verify_keyset_lookup_batch_dev: n >= 2^31"; return GOLDILOCKS_FAILURE; }
+    if (!scratch) { g_err = "goldilocks_ed448_verify_keyset_lookup_batch_dev: no scratch"; return GOLDILOCKS_FAILURE; }
+    VerifyGrids grids;
+    if (!verify_grids(*c, &grids)) return GOLDILOCKS_FAILURE;
+    KeysetLookupScratch s = {};
+    keyset_lookup_scratch(&s, scratch, n, 0, grids);   /* the packed messages sit last, so the layout does not depend on msg_bytes */
+    cudaStream_t st = as_stream(stream);
+    uint32_t *idx = key_index ? key_index : s.idx;
+    size_t hits = 0;
+    if (!keyset_lookup_order(*c, idx, ks, pubkey, n, s, st, &hits)) return GOLDILOCKS_FAILURE;
+    /* everything from here on lives in the caller's scratch, as in goldilocks_ed448_verify_batch_dev */
+    std::lock_guard<std::mutex> g(c->dev_side_mu); /* held while the launches are queued, not while they run */
+    return keyset_lookup_verify(*c, (int32_t *)status, ks, idx, signature, pubkey, msg, msg_off, prehashed, context, context_len, n, hits, s, grids, st, GRID_STRIDE,
+                                c->dev_side, c->dev_evt) ? GOLDILOCKS_SUCCESS : GOLDILOCKS_FAILURE;
 }
 goldilocks_error_t goldilocks_448_precomputed_scalarmul_batch_dev(hpt *out, const hsc *scalar, size_t n, void *stream) {
     Ctx *c = dev_ctx();

@@ -638,6 +638,65 @@ struct LaneVerifySign {
         }
     }
 };
+// ---- key-set lookup (goldilocks_ed448_verify_keyset_lookup_batch; DESIGN.md decision 23).  Public data only, variable time.
+GD int key57_cmp(const uint8_t *a, const uint8_t *b) { /* memcmp order of two 57-byte keys */
+    for (int k = 0; k < 57; k++)
+        if (a[k] != b[k]) return a[k] < b[k] ? -1 : 1;
+    return 0;
+}
+// Lane j: key_index[j] = the lowest index of the set whose 57 bytes equal pk j, or m.  `sorted` holds the set's indices ordered by
+// key bytes, ties by index (made on the host at creation), so the lower bound of pk j in it is its lowest equal index.  A byte
+// order rather than a hash order: ceil(log2 m) + 1 comparisons whatever keys the set holds.
+struct LaneKeysetLookup {
+    uint32_t *key_index; const uint8_t *pk, *set_pk; const uint32_t *sorted; uint32_t m;
+    GDM void operator()(size_t j) const {
+        const uint8_t *q = pk + 57 * j;
+        uint32_t lo = 0, hi = m;
+        while (lo < hi) {
+            const uint32_t mid = lo + (hi - lo) / 2;
+            if (key57_cmp(set_pk + 57 * (size_t)sorted[mid], q) < 0) lo = mid + 1;
+            else hi = mid;
+        }
+        key_index[j] = (lo < m && key57_cmp(set_pk + 57 * (size_t)sorted[lo], q) == 0) ? sorted[lo] : m;
+    }
+};
+// *hits = the number of sort keys below m (keys_s: the looked-up indices, clamped to m and sorted; LaneDecafPeerKeys).  One lane
+// writes: the first miss, or the last lane when there is none.
+struct LaneKeysetHits {
+    uint32_t *hits; const uint32_t *keys_s; uint32_t m; size_t n;
+    GDM void operator()(size_t j) const {
+        const bool miss = keys_s[j] >= m;
+        if (miss && (j == 0 || keys_s[j - 1] < m)) *hits = (uint32_t)j;
+        if (!miss && j + 1 == n) *hits = (uint32_t)n;
+    }
+};
+// The misses (elements order[hits + q], q < misses) packed for goldilocks_ed448_verify_batch's path: their message lengths (lane
+// `misses` writes 0, so an exclusive scan over misses + 1 entries gives the new offsets and the total) ...
+struct LaneKeysetMissLengths {
+    size_t *len; const size_t *off; const uint32_t *order; size_t hits, misses;
+    GDM void operator()(size_t q) const {
+        if (q >= misses) { len[q] = 0; return; }
+        const size_t i = order[hits + q];
+        len[q] = off[i + 1] - off[i];
+    }
+};
+// ... then their signatures, keys and messages
+struct LaneKeysetMissGather {
+    uint8_t *sig2, *pk2, *msg2; const size_t *off2; const uint8_t *sig, *pk, *msg; const size_t *off; const uint32_t *order; size_t hits;
+    GDM void operator()(size_t q) const {
+        const size_t i = order[hits + q];
+        for (int k = 0; k < 114; k++) sig2[114 * q + k] = sig[114 * i + k];
+        for (int k = 0; k < 57; k++) pk2[57 * q + k] = pk[57 * i + k];
+        const size_t lo = off[i], len = off[i + 1] - lo;
+        uint8_t *d = msg2 + off2[q];
+        for (size_t k = 0; k < len; k++) d[k] = msg[lo + k];
+    }
+};
+// status[order[j]] = st_sorted[j]: the hits' statuses (j < hits) and the misses' (j >= hits) back to the caller's positions
+struct LaneKeysetScatter {
+    int32_t *status; const int32_t *st_sorted; const uint32_t *order;
+    GDM void operator()(size_t j) const { status[order[j]] = st_sorted[j]; }
+};
 struct LaneBuildWide { /* verification table, WIDE_LANES lanes */
     niels *wide; pniels *tmp; gf *pre; const fixed_tables *ft;
     GDM void operator()(size_t lane) const { build_wide_lane(wide, tmp, pre, ft->comb, (int)lane); }

@@ -68,6 +68,7 @@ template <> struct slot_min_blocks<SlotEdVerifyFinishKeysetFlat> { static conste
 template <> struct slot_min_blocks<SlotKeysetChain> { static constexpr int value = 4; };
 template <> struct slot_min_blocks<SlotKeysetColumns> { static constexpr int value = 4; };
 template <bool FLAT> struct slot_min_blocks<SlotPointset<FLAT>> { static constexpr int value = 4; };
+template <bool FLAT> struct slot_min_blocks<SlotEdVerifyFinishKeysetOrdered<FLAT>> { static constexpr int value = 4; };
 template <class F>
 cudaError_t launch_sm(const F &f, size_t n, cudaStream_t s) {
     const int smem = F::NSLOTS * 64 * SLOT_BLOCK;
@@ -112,12 +113,13 @@ cudaError_t launch_sm_persist(const F &f, size_t n, int grid, cudaStream_t s, un
     X(LaneScDecodeLong) X(LaneScInvert) X(LaneShake256) X(LaneSpongeUpdate) X(LaneSpongeOutput) X(LaneEdPkToX448) X(LaneEdSkToX448) X(LanePrecompute) X(LaneNielsFromAbi) X(LaneX448PeerLift) X(LaneDecafPeerDecode) X(LaneDecafPeerKeys)                                                             \
     X(LaneEdSecretScalar) X(LaneEdSignExpand) X(LaneEdSignNonce) X(LaneEdSignFinish)   \
     X(LaneEdVerifyDecode) X(LaneEdVerifyScalars) X(LaneVerifySign) X(LaneVerifyHalf) X(LaneKeysetNormalize) X(LaneBuildTables) X(LaneBuildWide) \
-    X(LaneRlcDecode) X(LaneRlcZ) X(LaneRlcWeights) X(LaneRlcLate) X(LaneRlcKeyScalars) X(LaneRlcDigits) X(LaneRlcBucketRuns) X(LaneRlcSegments) X(LaneRlcNodes) X(LaneRlcWindows) X(LaneRlcTotal) X(LaneRlcVerdict) X(LaneRlcPackPlan) X(LaneRlcPack) X(LaneRlcUnpack) X(LanePtNiels)
+    X(LaneRlcDecode) X(LaneRlcZ) X(LaneRlcWeights) X(LaneRlcLate) X(LaneRlcKeyScalars) X(LaneRlcDigits) X(LaneRlcBucketRuns) X(LaneRlcSegments) X(LaneRlcNodes) X(LaneRlcWindows) X(LaneRlcTotal) X(LaneRlcVerdict) X(LaneRlcPackPlan) X(LaneRlcPack) X(LaneRlcUnpack) X(LanePtNiels) \
+    X(LaneKeysetLookup) X(LaneKeysetHits) X(LaneKeysetMissLengths) X(LaneKeysetMissGather) X(LaneKeysetScatter)
 
 #define LANES_SM(X) X(SlotNielsDebug) X(SlotX448) X(SlotX448Peer) X(SlotComb) X(SlotCombTable) X(SlotDecafPeer) X(SlotX448DerivePk) X(SlotEdDerivePk) X(SlotEdSignR) X(SlotRlcBucket)
 #define INSTANTIATE_SM(F) template cudaError_t launch_sm<F>(const F &, size_t, cudaStream_t);
 #define DECLARE_SM(F) extern INSTANTIATE_SM(F)
-#define LANES_SMP(X) X(SlotEdVerifyFinish) X(SlotEdVerifyFinishShared) X(SlotKeyChain) X(SlotKeyColumns) X(SlotKeysetTables) X(SlotKeysetChain) X(SlotKeysetColumns) X(SlotEdVerifyFinishKeyset) X(SlotEdVerifyFinishKeysetFlat) X(SlotPointset<true>) X(SlotPointset<false>) X(SlotBaseDoubleScalarmul) X(SlotScalarmul) X(SlotDoubleScalarmul) X(SlotDualScalarmul) X(SlotDirectScalarmul)
+#define LANES_SMP(X) X(SlotEdVerifyFinish) X(SlotEdVerifyFinishShared) X(SlotKeyChain) X(SlotKeyColumns) X(SlotKeysetTables) X(SlotKeysetChain) X(SlotKeysetColumns) X(SlotEdVerifyFinishKeyset) X(SlotEdVerifyFinishKeysetFlat) X(SlotPointset<true>) X(SlotPointset<false>) X(SlotEdVerifyFinishKeysetOrdered<true>) X(SlotEdVerifyFinishKeysetOrdered<false>) X(SlotBaseDoubleScalarmul) X(SlotScalarmul) X(SlotDoubleScalarmul) X(SlotDualScalarmul) X(SlotDirectScalarmul)
 #define INSTANTIATE_SMP(F)                                                                          \
     template cudaError_t sm_configure<F>(int *);                                                    \
     template cudaError_t launch_sm_persist<F>(const F &, size_t, int, cudaStream_t, unsigned *);

@@ -335,6 +335,27 @@ struct SlotEdVerifyFinishKeyset { /* signature i under key key_index[i] of the s
         s_verify_accept_prep(aux + i, sb, sig + 114 * i, (gmask_t)key_ok[t]);
     }
 };
+// Key-set lookup calls (goldilocks_ed448_verify_keyset_lookup_batch; DESIGN.md decision 23): lane j < hits verifies element
+// i = order[j] (the batch sorted by looked-up key, so the lanes of a warp read one or two tables) under key key_index[i] < m of a
+// set of either layout, with the evaluations of the two kernels above, and leaves its aux record at aux[j].
+template <bool FLAT>
+struct SlotEdVerifyFinishKeysetOrdered {
+    static constexpr int NSLOTS = BDSM_NSLOTS;
+    verify_aux *aux; const int32_t *key_ok; const abi_sc *challenge, *response; const niels *wide; const uint4 *ktabs;
+    const uint32_t *key_index, *order; const uint8_t *sig;
+    GDM void operator()(size_t j, sref sb, size_t slot) const {
+        (void)slot;
+        const size_t i = order[j];
+        const uint32_t t = key_index[i];
+        sc c, r;
+        sc_from_abi(c, challenge + i);
+        sc_from_abi(r, response + i);
+        if (FLAT) s_verify_flat_key(sb, r, c, wide, kset_of(const_cast<uint4 *>(ktabs), t));
+        else s_verify_shared_key<true>(sb, r, c, wide, ktab_of(const_cast<uint4 *>(ktabs), t));   /* affine entries */
+        s_bdsm_quirk(sb, c);
+        s_verify_accept_prep(aux + j, sb, sig + 114 * i, (gmask_t)key_ok[t]);
+    }
+};
 
 GD void s_pt_to_abi(abi_pt *o, sref sb) { /* slots 0..3 -> canonical host limbs */
     gf v;

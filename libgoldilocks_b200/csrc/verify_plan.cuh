@@ -27,5 +27,7 @@ cudaError_t key_chunks(uint32_t *kchunk, const key_groups *g, uint32_t m, uint32
 size_t pair_sort_scratch_bytes(size_t npairs);
 cudaError_t pair_sort(void *tmp, size_t tmp_bytes, const uint32_t *keys_in, uint32_t *keys_out, const uint32_t *vals_in, uint32_t *vals_out, size_t npairs,
                       int key_bits, cudaStream_t s);
+size_t length_scan_scratch_bytes(size_t count);
+cudaError_t length_scan(void *tmp, size_t tmp_bytes, const size_t *len, size_t *off, size_t count, cudaStream_t s);
 cudaError_t group_keys(const uint8_t *pk, size_t n, uint32_t cap, void *scratch, verify_plan *plan, cudaStream_t s, uint64_t *launches);
 #endif

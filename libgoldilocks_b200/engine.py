@@ -90,6 +90,24 @@ class DeviceEngine:
                    C.c_uint8(prehashed), self._p(ctx), C.c_uint8(ctx_len), _Z(status.numel()), self._stream(), C.byref(fast))
         return fast.value
 
+    def keyset_scratch_bytes(self, n, msg_bytes):
+        f = self.lib.goldilocks_b200_keyset_scratch_bytes
+        f.restype = _Z
+        f.argtypes = [_Z, _Z]
+        return int(f(n, msg_bytes))
+
+    def ed448_verify_keyset_lookup(self, status, key_index, handle, sig, pk, msg, msg_off, scratch, prehashed=0, ctx=None, ctx_len=0):
+        """goldilocks_ed448_verify_keyset_lookup_batch_dev against a set made by capi keyset_create; key_index (int32 tensor read as
+        uint32, or None) receives the looked-up indices; `scratch` holds keyset_scratch_bytes(n, msg_off[n]).  Synchronises the current
+        stream once, after the lookup."""
+        self._call("goldilocks_ed448_verify_keyset_lookup_batch_dev", self._p(status), self._p(key_index), handle, self._p(sig), self._p(pk), self._p(msg),
+                   self._p(msg_off), C.c_uint8(prehashed), self._p(ctx), C.c_uint8(ctx_len), _Z(status.numel()), self._p(scratch), self._stream())
+
+    def ed448_verify_keyset(self, status, handle, key_index, sig, msg, msg_off, scratch, prehashed=0, ctx=None, ctx_len=0):
+        """goldilocks_ed448_verify_keyset_batch_dev: signature i under key key_index[i] (int32 tensor read as uint32) of the set"""
+        self._call("goldilocks_ed448_verify_keyset_batch_dev", self._p(status), handle, self._p(key_index), self._p(sig), self._p(msg), self._p(msg_off),
+                   C.c_uint8(prehashed), self._p(ctx), C.c_uint8(ctx_len), _Z(status.numel()), self._p(scratch), self._stream())
+
     def x448(self, out, status, base, scalar):
         self._call("goldilocks_x448_batch_dev", self._p(out), self._p(status), self._p(base), self._p(scalar), _Z(status.numel()), self._stream())
 
