@@ -1488,9 +1488,110 @@ goldilocks_error_t goldilocks_ed448_verify_rlc_batch_dev(goldilocks_error_t *sta
     return k.finish();
 }
 
-// ---- key sets: per-key verification tables that outlive a call (SURVEY 8(f)4) ---------------------------------------
-struct goldilocks_b200_keyset_s {
+// ---- device-resident sets: tables built once on one device and used by many calls (key, X448 peer, decaf peer and point sets) --
+extern "C++" {   /* the helpers shared by the sets are templates */
+/* What every set struct inherits: the device it belongs to, its size m and the device buffers it owns.  The handles are opaque in
+ * the header, so each *_destroy is `delete`; the destructor frees the buffers on the set's own device, whichever is current. */
+struct DeviceSet {
+    static constexpr int MAX_BUFFERS = 4;   /* a key set's pk, key_ok, ktabs and sorted */
     int dev; size_t m;
+    void *owned[MAX_BUFFERS] = {};
+    int n_owned = 0;
+    DeviceSet(int dev, size_t m) : dev(dev), m(m) {}
+    DeviceSet(const DeviceSet &) = delete;
+    DeviceSet &operator=(const DeviceSet &) = delete;
+    ~DeviceSet() {
+        int cur = 0;
+        const bool sw = cudaGetDevice(&cur) == cudaSuccess && cur != dev && cudaSetDevice(dev) == cudaSuccess;
+        for (int i = 0; i < n_owned; i++) cudaFree(owned[i]);
+        if (sw) cudaSetDevice(cur);
+    }
+    template <class T> bool alloc(T **p, size_t count) {
+        if (n_owned == MAX_BUFFERS || cudaMalloc(p, sizeof(T) * count) != cudaSuccess) return false;
+        owned[n_owned++] = *p;
+        return true;
+    }
+};
+/* the end of every *_create: on failure `err` (unless the call set its own) and the set freed, else the set in *out */
+template <class S>
+static goldilocks_error_t finish_create(Call &k, bool ok, S *s, S **out, const char *err) {
+    const goldilocks_error_t r = k.finish();
+    if (!ok || r != GOLDILOCKS_SUCCESS) {
+        if (!ok) g_err = err;
+        delete s;
+        return GOLDILOCKS_FAILURE;
+    }
+    *out = s;
+    return GOLDILOCKS_SUCCESS;
+}
+/* The checks of a call on a set, each overload adding one: the set belongs to the calling device; the batch has fewer than 2^31
+ * elements; the caller passed scratch. */
+template <class S> static bool set_call(const S *s, int dev, const char *fn) {
+    if (s && s->dev == dev) return true;
+    g_err = std::string(fn) + ": the " + S::noun + " lives on another device";
+    return false;
+}
+template <class S> static bool set_call(const S *s, int dev, const char *fn, size_t n) {
+    if (!set_call(s, dev, fn)) return false;
+    if (n > (size_t)INT32_MAX) { g_err = std::string(fn) + ": n >= 2^31"; return false; }
+    return true;
+}
+template <class S> static bool set_call(const S *s, int dev, const char *fn, size_t n, const void *scratch) {
+    if (!set_call(s, dev, fn, n)) return false;
+    if (!scratch) { g_err = std::string(fn) + ": no scratch"; return false; }
+    return true;
+}
+/* the persistent kernel of a set's layout over n elements: make(std::true_type{}) / make(std::false_type{}) returns the functor of
+ * the flat / the compact kernel */
+template <class Make>
+static bool launch_layout(Ctx &c, bool flat, size_t n, cudaStream_t st, unsigned *counter, const Make &make) {
+    auto go = [&](auto f) {
+        int grid = 1;
+        return smp_grid<decltype(f)>(c, &grid) && launch_smp(c, f, n, grid, st, counter);
+    };
+    return flat ? go(make(std::true_type{})) : go(make(std::false_type{}));
+}
+/* the reference's (5,5,18) comb tables of `count` points (X448 and decaf peer sets), as affine niels */
+static void comb_tables(Call &k, const abi_pt *pts, niels *out, size_t count) {
+    LanePrecompute fp = {k.out<abi_niels>(COMB_ENTRIES * count), pts, k.out<niels>(16 * COMB_N * count)};
+    k.run(fp, COMB_N * count);
+    LaneNielsFromAbi fc = {out, fp.tables};
+    k.run(fc, COMB_ENTRIES * count);
+}
+/* the scratch of one call's ordering, carved from `base` (null: sizes only): sort keys and values in and out, CUB's temporary storage */
+struct OrderScratch { uint32_t *keys, *vals, *keys_s, *order; void *sort_tmp; size_t sort_bytes; };
+static size_t order_scratch(OrderScratch *s, void *base, size_t n) {
+    auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
+    const size_t words = al(sizeof(uint32_t) * n), sort_bytes = pair_sort_scratch_bytes(n);
+    if (s) {
+        char *p = (char *)base;
+        s->keys = (uint32_t *)p; s->vals = (uint32_t *)(p + words); s->keys_s = (uint32_t *)(p + 2 * words); s->order = (uint32_t *)(p + 3 * words);
+        s->sort_tmp = p + 4 * words; s->sort_bytes = sort_bytes;
+    }
+    return 4 * words + al(sort_bytes);
+}
+/* s.order = the elements sorted by set entry: keys (min(index[j], m), j) -> stable radix sort.  Decaf peer sets, point sets and
+ * key-set lookup order every call this way.  The sort is bracketed like a launch when profiling is on, so
+ * goldilocks_b200_profile_timeline shows its share of the call. */
+static bool set_order(Ctx &c, const uint32_t *index, uint32_t m, size_t n, const OrderScratch &s, cudaStream_t st, const char *what) {
+    LaneDecafPeerKeys fk = {s.keys, s.vals, index, m};
+    if (!launch(c, fk, n, st)) return false;
+    int key_bits = 1;
+    while (key_bits < 32 && (m >> key_bits)) key_bits++;   /* the bit length of m, the largest key */
+    cudaEvent_t a = nullptr, b = nullptr;
+    const bool prof = g_prof_on.load() != 0;
+    if (prof) a = prof_begin("pair_sort", st, &b);
+    const cudaError_t e = pair_sort(s.sort_tmp, s.sort_bytes, s.keys, s.keys_s, s.vals, s.order, n, key_bits, st);
+    if (prof) prof_end("pair_sort", st, a, b);
+    if (e != cudaSuccess) return fail(what, e);
+    return true;
+}
+static size_t order_scratch_bytes(size_t n) { return dev_ctx() ? order_scratch(nullptr, nullptr, n) : 0; }
+}  // extern "C++"
+
+// ---- key sets: per-key verification tables that outlive a call (SURVEY 8(f)4) ---------------------------------------
+struct goldilocks_b200_keyset_s : DeviceSet {
+    static constexpr const char *noun = "key set";
     uint8_t *pk;      /* m x 57 key bytes (the challenge hashes them) */
     int32_t *key_ok;  /* decode status per key */
     uint4 *ktabs;     /* m tables of KTAB_QUADS quads (10 columns x 9 rows), or of KSET_QUADS (flat: a column per digit position) */
@@ -1526,10 +1627,9 @@ goldilocks_error_t goldilocks_b200_keyset_create(goldilocks_b200_keyset **out, c
     if (!k.ok) return k.finish();
     const size_t mm = m ? m : 1;
     const bool flat = keyset_flat(mm);
-    goldilocks_b200_keyset_s *ks = new goldilocks_b200_keyset_s{k.c->dev, m, nullptr, nullptr, nullptr, flat, nullptr};
-    bool ok = cudaMalloc(&ks->pk, 57 * mm) == cudaSuccess && cudaMalloc(&ks->key_ok, sizeof(int32_t) * mm) == cudaSuccess &&
-              cudaMalloc(&ks->ktabs, mm * (flat ? KSET_QUADS : KTAB_QUADS) * sizeof(uint4)) == cudaSuccess &&
-              cudaMalloc(&ks->sorted, sizeof(uint32_t) * mm) == cudaSuccess;
+    goldilocks_b200_keyset_s *ks = new goldilocks_b200_keyset_s{{k.c->dev, m}, nullptr, nullptr, nullptr, flat, nullptr};
+    bool ok = ks->alloc(&ks->pk, 57 * mm) && ks->alloc(&ks->key_ok, mm) && ks->alloc(&ks->ktabs, mm * (flat ? KSET_QUADS : KTAB_QUADS)) &&
+              ks->alloc(&ks->sorted, mm);
     /* the bytes are on the host already: sort there (a byte order, not a hash order -- nobody can make the search longer) */
     std::vector<uint32_t> sorted(m);
     for (size_t i = 0; i < m; i++) sorted[i] = (uint32_t)i;
@@ -1542,24 +1642,9 @@ goldilocks_error_t goldilocks_b200_keyset_create(goldilocks_b200_keyset **out, c
         k.run(fd, m);
         keyset_tables(k, pts, ks->ktabs, m, flat);
     }
-    goldilocks_error_t r = k.finish();
-    if (!ok || r != GOLDILOCKS_SUCCESS) {
-        if (!ok) g_err = "goldilocks_b200_keyset_create: device allocation or copy failed";
-        cudaFree(ks->pk); cudaFree(ks->key_ok); cudaFree(ks->ktabs); cudaFree(ks->sorted);
-        delete ks;
-        return GOLDILOCKS_FAILURE;
-    }
-    *out = ks;
-    return GOLDILOCKS_SUCCESS;
+    return finish_create(k, ok, ks, out, "goldilocks_b200_keyset_create: device allocation or copy failed");
 }
-void goldilocks_b200_keyset_destroy(goldilocks_b200_keyset *ks) {
-    if (!ks) return;
-    int cur = 0;
-    const bool sw = cudaGetDevice(&cur) == cudaSuccess && cur != ks->dev && cudaSetDevice(ks->dev) == cudaSuccess;
-    cudaFree(ks->pk); cudaFree(ks->key_ok); cudaFree(ks->ktabs); cudaFree(ks->sorted);
-    if (sw) cudaSetDevice(cur);
-    delete ks;
-}
+void goldilocks_b200_keyset_destroy(goldilocks_b200_keyset *ks) { delete ks; }
 size_t goldilocks_b200_keyset_size(const goldilocks_b200_keyset *ks) { return ks ? ks->m : 0; }
 /* the index form on device buffers: challenges under the set's key bytes, the finish kernel of the set's layout, the sign check */
 static bool keyset_enqueue(Ctx &c, int32_t *status, const goldilocks_b200_keyset_s *ks, const uint32_t *key_index, const uint8_t *sig, const uint8_t *msg,
@@ -1567,14 +1652,10 @@ static bool keyset_enqueue(Ctx &c, int32_t *status, const goldilocks_b200_keyset
                            cudaStream_t st, unsigned *counter) {
     LaneEdVerifyScalars f2 = {chal, resp, sig, ks->pk, msg, off, prehashed, ctx, ctx_len, 0, key_index, (uint32_t)ks->m};
     if (!launch(c, f2, n, st)) return false;
-    int grid = 1;
-    if (ks->flat) {
-        SlotEdVerifyFinishKeysetFlat f3 = {aux, ks->key_ok, chal, resp, c.wide, ks->ktabs, key_index, (uint32_t)ks->m, sig};
-        if (!smp_grid<SlotEdVerifyFinishKeysetFlat>(c, &grid) || !launch_smp(c, f3, n, grid, st, counter)) return false;
-    } else {
-        SlotEdVerifyFinishKeyset f3 = {aux, ks->key_ok, chal, resp, c.wide, ks->ktabs, key_index, (uint32_t)ks->m, sig};
-        if (!smp_grid<SlotEdVerifyFinishKeyset>(c, &grid) || !launch_smp(c, f3, n, grid, st, counter)) return false;
-    }
+    if (!launch_layout(c, ks->flat, n, st, counter, [&](auto flat) {
+            return SlotEdVerifyFinishKeysetLayout<decltype(flat)::value>{aux, ks->key_ok, chal, resp, c.wide, ks->ktabs, key_index, (uint32_t)ks->m, sig};
+        }))
+        return false;
     LaneVerifySign fv = {status, aux, 1, n};
     return launch(c, fv, (n + VSIGN_BATCH - 1) / VSIGN_BATCH, st);
 }
@@ -1584,7 +1665,7 @@ goldilocks_error_t goldilocks_ed448_verify_keyset_batch(goldilocks_error_t *stat
     if (n == 0) return GOLDILOCKS_SUCCESS;
     Call k;
     if (!k.ok) return k.finish();
-    if (!ks || ks->dev != k.c->dev) { g_err = "goldilocks_ed448_verify_keyset_batch: the key set lives on another device"; return GOLDILOCKS_FAILURE; }
+    if (!set_call(ks, k.c->dev, "goldilocks_ed448_verify_keyset_batch")) return GOLDILOCKS_FAILURE;
     const size_t total = n ? msg_off[n] : 0;
     const size_t *doff = k.in(msg_off, n + 1);
     const uint8_t *dctx = k.in(context, context_len);
@@ -1599,8 +1680,8 @@ goldilocks_error_t goldilocks_ed448_verify_keyset_batch(goldilocks_error_t *stat
 }
 
 // ---- X448 peer sets: per-peer comb tables for key agreement with recurring public keys (slot_lanes.cuh SlotX448Peer) -------
-struct goldilocks_b200_x448_peerset_s {
-    int dev; size_t m;
+struct goldilocks_b200_x448_peerset_s : DeviceSet {
+    static constexpr const char *noun = "peer set";
     uint8_t *peers;     /* m x 56 u bytes: what the ladder reads for the peers that keep it */
     int32_t *table_ok;  /* per peer: SUCCESS = the comb table is valid (public) */
     niels *tables;      /* m tables of COMB_ENTRIES affine niels, 15 360 bytes each */
@@ -1611,44 +1692,25 @@ goldilocks_error_t goldilocks_b200_x448_peerset_create(goldilocks_b200_x448_peer
     Call k;
     if (!k.ok) return k.finish();
     const size_t mm = m ? m : 1;
-    goldilocks_b200_x448_peerset_s *ps = new goldilocks_b200_x448_peerset_s{k.c->dev, m, nullptr, nullptr, nullptr};
-    bool ok = m <= UINT32_MAX && cudaMalloc(&ps->peers, 56 * mm) == cudaSuccess && cudaMalloc(&ps->table_ok, sizeof(int32_t) * mm) == cudaSuccess &&
-              cudaMalloc(&ps->tables, mm * COMB_ENTRIES * sizeof(niels)) == cudaSuccess;
+    goldilocks_b200_x448_peerset_s *ps = new goldilocks_b200_x448_peerset_s{{k.c->dev, m}, nullptr, nullptr, nullptr};
+    bool ok = m <= UINT32_MAX && ps->alloc(&ps->peers, 56 * mm) && ps->alloc(&ps->table_ok, mm) && ps->alloc(&ps->tables, mm * COMB_ENTRIES);
     if (ok && m) {
         ok = cudaMemcpyAsync(ps->peers, peers, 56 * m, cudaMemcpyHostToDevice, k.c->stream) == cudaSuccess;
         abi_pt *pts = k.out<abi_pt>(m);
         LaneX448PeerLift fl = {pts, ps->table_ok, ps->peers};
         k.run(fl, m);
-        LanePrecompute fp = {k.out<abi_niels>(COMB_ENTRIES * m), pts, k.out<niels>(16 * COMB_N * m)};
-        k.run(fp, COMB_N * m);
-        LaneNielsFromAbi fc = {ps->tables, fp.tables};
-        k.run(fc, COMB_ENTRIES * m);
+        comb_tables(k, pts, ps->tables, m);
     }
-    goldilocks_error_t r = k.finish();
-    if (!ok || r != GOLDILOCKS_SUCCESS) {
-        if (!ok) g_err = "goldilocks_b200_x448_peerset_create: device allocation or copy failed";
-        cudaFree(ps->peers); cudaFree(ps->table_ok); cudaFree(ps->tables);
-        delete ps;
-        return GOLDILOCKS_FAILURE;
-    }
-    *out = ps;
-    return GOLDILOCKS_SUCCESS;
+    return finish_create(k, ok, ps, out, "goldilocks_b200_x448_peerset_create: device allocation or copy failed");
 }
-void goldilocks_b200_x448_peerset_destroy(goldilocks_b200_x448_peerset *ps) {
-    if (!ps) return;
-    int cur = 0;
-    const bool sw = cudaGetDevice(&cur) == cudaSuccess && cur != ps->dev && cudaSetDevice(ps->dev) == cudaSuccess;
-    cudaFree(ps->peers); cudaFree(ps->table_ok); cudaFree(ps->tables);
-    if (sw) cudaSetDevice(cur);
-    delete ps;
-}
+void goldilocks_b200_x448_peerset_destroy(goldilocks_b200_x448_peerset *ps) { delete ps; }
 size_t goldilocks_b200_x448_peerset_size(const goldilocks_b200_x448_peerset *ps) { return ps ? ps->m : 0; }
 goldilocks_error_t goldilocks_x448_peerset_batch(uint8_t *out, goldilocks_error_t *status, const goldilocks_b200_x448_peerset *ps, const uint32_t *peer_index,
                                                  const uint8_t *scalar, size_t n) {
     if (n == 0) return GOLDILOCKS_SUCCESS;
     Call k;
     if (!k.ok) return k.finish();
-    if (!ps || ps->dev != k.c->dev) { g_err = "goldilocks_x448_peerset_batch: the peer set lives on another device"; return GOLDILOCKS_FAILURE; }
+    if (!set_call(ps, k.c->dev, "goldilocks_x448_peerset_batch")) return GOLDILOCKS_FAILURE;
     SlotX448Peer f = {k.secret(k.out<uint8_t>(56 * n), 56 * n), k.out<int32_t>(n), ps->tables, ps->table_ok, ps->peers, k.in(peer_index, n),
                       k.secret(k.in(scalar, 56 * n), 56 * n), (uint32_t)ps->m};
     k.run_sm(f, n);
@@ -1658,44 +1720,16 @@ goldilocks_error_t goldilocks_x448_peerset_batch(uint8_t *out, goldilocks_error_
 }
 
 // ---- decaf peer sets: per-peer comb tables for goldilocks_448_direct_scalarmul against recurring points (slot_lanes.cuh SlotDecafPeer)
-struct goldilocks_b200_decaf_peerset_s {
-    int dev; size_t m;
+struct goldilocks_b200_decaf_peerset_s : DeviceSet {
+    static constexpr const char *noun = "peer set";
     int32_t *peer_ok;   /* m + 1 decode statuses (public); entry m, the base point with FAILURE, stands for every index >= m */
     niels *tables;      /* m + 1 tables of COMB_ENTRIES affine niels, 15 360 bytes each */
 };
-/* the scratch of one call, carved from `base` (null: sizes only): sort keys and values in and out, CUB's temporary storage */
-struct DecafPeerScratch { uint32_t *keys, *vals, *keys_s, *order; void *sort_tmp; size_t sort_bytes; };
-static size_t decaf_peer_scratch(DecafPeerScratch *s, void *base, size_t n) {
-    auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
-    const size_t words = al(sizeof(uint32_t) * n), sort_bytes = pair_sort_scratch_bytes(n);
-    if (s) {
-        char *p = (char *)base;
-        s->keys = (uint32_t *)p; s->vals = (uint32_t *)(p + words); s->keys_s = (uint32_t *)(p + 2 * words); s->order = (uint32_t *)(p + 3 * words);
-        s->sort_tmp = p + 4 * words; s->sort_bytes = sort_bytes;
-    }
-    return 4 * words + al(sort_bytes);
-}
-/* s.order = the elements sorted by set entry: keys (min(peer_index[j], m), j) -> stable radix sort.  Decaf peer sets and point sets
- * order every call this way.  The sort is bracketed like a launch when profiling is on, so goldilocks_b200_profile_timeline shows
- * its share of the call. */
-static bool peer_order(Ctx &c, const uint32_t *peer_index, uint32_t m, size_t n, const DecafPeerScratch &s, cudaStream_t st, const char *what) {
-    LaneDecafPeerKeys fk = {s.keys, s.vals, peer_index, m};
-    if (!launch(c, fk, n, st)) return false;
-    int key_bits = 1;
-    while (key_bits < 32 && (m >> key_bits)) key_bits++;   /* the bit length of m, the largest key */
-    cudaEvent_t a = nullptr, b = nullptr;
-    const bool prof = g_prof_on.load() != 0;
-    if (prof) a = prof_begin("pair_sort", st, &b);
-    const cudaError_t e = pair_sort(s.sort_tmp, s.sort_bytes, s.keys, s.keys_s, s.vals, s.order, n, key_bits, st);
-    if (prof) prof_end("pair_sort", st, a, b);
-    if (e != cudaSuccess) return fail(what, e);
-    return true;
-}
 /* the sort by peer, then the comb kernel over the elements in that order */
 static bool decaf_peer_enqueue(Ctx &c, uint8_t *scaled, int32_t *status, const goldilocks_b200_decaf_peerset_s *ps, const uint32_t *peer_index,
-                               const abi_sc *scalar, bool short_circuit, size_t n, const DecafPeerScratch &s, cudaStream_t st) {
+                               const abi_sc *scalar, bool short_circuit, size_t n, const OrderScratch &s, cudaStream_t st) {
     const uint32_t m = (uint32_t)ps->m;
-    if (!peer_order(c, peer_index, m, n, s, st, "pair_sort (decaf peer set)")) return false;
+    if (!set_order(c, peer_index, m, n, s, st, "pair_sort (decaf peer set)")) return false;
     SlotDecafPeer f = {scaled, status, ps->tables, ps->peer_ok, peer_index, s.order, scalar, m, short_circuit ? ~0u : 0u};
     return launch_slots(c, f, n, st);
 }
@@ -1706,49 +1740,30 @@ goldilocks_error_t goldilocks_b200_decaf_peerset_create(goldilocks_b200_decaf_pe
     if (!k.ok) return k.finish();
     if (m >= UINT32_MAX) { g_err = "goldilocks_b200_decaf_peerset_create: at most 2^32 - 2 peers"; return GOLDILOCKS_FAILURE; }
     const size_t mm = m + 1;
-    goldilocks_b200_decaf_peerset_s *ps = new goldilocks_b200_decaf_peerset_s{k.c->dev, m, nullptr, nullptr};
-    bool ok = cudaMalloc(&ps->peer_ok, sizeof(int32_t) * mm) == cudaSuccess && cudaMalloc(&ps->tables, mm * COMB_ENTRIES * sizeof(niels)) == cudaSuccess;
+    goldilocks_b200_decaf_peerset_s *ps = new goldilocks_b200_decaf_peerset_s{{k.c->dev, m}, nullptr, nullptr};
+    bool ok = ps->alloc(&ps->peer_ok, mm) && ps->alloc(&ps->tables, mm * COMB_ENTRIES);
     if (ok) {
         abi_pt *pts = k.out<abi_pt>(mm);
         LaneDecafPeerDecode fd = {pts, ps->peer_ok, k.in(peers, 56 * m), k.c->ft, (uint32_t)m, allow_identity ? 1u : 0u};
         k.run(fd, mm);
-        LanePrecompute fp = {k.out<abi_niels>(COMB_ENTRIES * mm), pts, k.out<niels>(16 * COMB_N * mm)};
-        k.run(fp, COMB_N * mm);
-        LaneNielsFromAbi fc = {ps->tables, fp.tables};
-        k.run(fc, COMB_ENTRIES * mm);
+        comb_tables(k, pts, ps->tables, mm);
     }
-    goldilocks_error_t r = k.finish();
-    if (!ok || r != GOLDILOCKS_SUCCESS) {
-        if (!ok) g_err = "goldilocks_b200_decaf_peerset_create: device allocation failed";
-        cudaFree(ps->peer_ok); cudaFree(ps->tables);
-        delete ps;
-        return GOLDILOCKS_FAILURE;
-    }
-    *out = ps;
-    return GOLDILOCKS_SUCCESS;
+    return finish_create(k, ok, ps, out, "goldilocks_b200_decaf_peerset_create: device allocation failed");
 }
-void goldilocks_b200_decaf_peerset_destroy(goldilocks_b200_decaf_peerset *ps) {
-    if (!ps) return;
-    int cur = 0;
-    const bool sw = cudaGetDevice(&cur) == cudaSuccess && cur != ps->dev && cudaSetDevice(ps->dev) == cudaSuccess;
-    cudaFree(ps->peer_ok); cudaFree(ps->tables);
-    if (sw) cudaSetDevice(cur);
-    delete ps;
-}
+void goldilocks_b200_decaf_peerset_destroy(goldilocks_b200_decaf_peerset *ps) { delete ps; }
 size_t goldilocks_b200_decaf_peerset_size(const goldilocks_b200_decaf_peerset *ps) { return ps ? ps->m : 0; }
 goldilocks_error_t goldilocks_448_direct_scalarmul_peerset_batch(uint8_t *scaled, goldilocks_error_t *status, const goldilocks_b200_decaf_peerset *ps,
                                                                  const uint32_t *peer_index, const hsc *scalar, goldilocks_bool_t short_circuit, size_t n) {
     if (n == 0) return GOLDILOCKS_SUCCESS;
     Call k;
     if (!k.ok) return k.finish();
-    if (!ps || ps->dev != k.c->dev) { g_err = "goldilocks_448_direct_scalarmul_peerset_batch: the peer set lives on another device"; return GOLDILOCKS_FAILURE; }
-    if (n > (size_t)INT32_MAX) { g_err = "goldilocks_448_direct_scalarmul_peerset_batch: n >= 2^31"; return GOLDILOCKS_FAILURE; }
+    if (!set_call(ps, k.c->dev, "goldilocks_448_direct_scalarmul_peerset_batch", n)) return GOLDILOCKS_FAILURE;
     uint8_t *dout = k.secret(k.in(scaled, 56 * n), 56 * n); /* short-circuited elements keep the caller's bytes */
     int32_t *dst = k.out<int32_t>(n);
     const uint32_t *didx = k.in(peer_index, n);
     const abi_sc *dsc = k.secret(k.in(S(scalar), n), n);
-    DecafPeerScratch s;
-    decaf_peer_scratch(&s, k.alloc(decaf_peer_scratch(nullptr, nullptr, n)), n);
+    OrderScratch s;
+    order_scratch(&s, k.alloc(order_scratch(nullptr, nullptr, n)), n);
     if (k.ok) k.ok = decaf_peer_enqueue(*k.c, dout, dst, ps, didx, dsc, short_circuit != 0, n, s, k.c->stream);
     k.fetch(scaled, dout, 56 * n);
     k.fetch((int32_t *)status, dst, n);
@@ -1756,23 +1771,19 @@ goldilocks_error_t goldilocks_448_direct_scalarmul_peerset_batch(uint8_t *scaled
 }
 
 // ---- point sets: key-set tables for goldilocks_448_base_double_scalarmul_non_secret against recurring points (slot_lanes.cuh SlotPointset)
-struct goldilocks_b200_pointset_s {
-    int dev; size_t m;
+struct goldilocks_b200_pointset_s : DeviceSet {
+    static constexpr const char *noun = "point set";
     uint4 *ktabs;   /* m + 1 key-set tables (KSET_QUADS each when flat, else KTAB_QUADS); table m, the identity's, stands for every index >= m */
     bool flat;
 };
 /* the sort by point (as decaf peer sets), then the point-set kernel of the set's layout over the elements in that order */
 static bool pointset_enqueue(Ctx &c, abi_pt *out, const goldilocks_b200_pointset_s *ps, const uint32_t *point_index, const abi_sc *scalar1,
-                             const abi_sc *scalar2, size_t n, const DecafPeerScratch &s, cudaStream_t st, unsigned *counter) {
+                             const abi_sc *scalar2, size_t n, const OrderScratch &s, cudaStream_t st, unsigned *counter) {
     const uint32_t m = (uint32_t)ps->m;
-    if (!peer_order(c, point_index, m, n, s, st, "pair_sort (point set)")) return false;
-    int grid = 1;
-    if (ps->flat) {
-        SlotPointset<true> f = {out, scalar1, scalar2, c.wide, ps->ktabs, point_index, s.order, m};
-        return smp_grid<SlotPointset<true>>(c, &grid) && launch_smp(c, f, n, grid, st, counter);
-    }
-    SlotPointset<false> f = {out, scalar1, scalar2, c.wide, ps->ktabs, point_index, s.order, m};
-    return smp_grid<SlotPointset<false>>(c, &grid) && launch_smp(c, f, n, grid, st, counter);
+    if (!set_order(c, point_index, m, n, s, st, "pair_sort (point set)")) return false;
+    return launch_layout(c, ps->flat, n, st, counter, [&](auto flat) {
+        return SlotPointset<decltype(flat)::value>{out, scalar1, scalar2, c.wide, ps->ktabs, point_index, s.order, m};
+    });
 }
 goldilocks_error_t goldilocks_b200_pointset_create(goldilocks_b200_pointset **out, const hpt *points, size_t m) {
     if (!out) return GOLDILOCKS_FAILURE;
@@ -1782,8 +1793,8 @@ goldilocks_error_t goldilocks_b200_pointset_create(goldilocks_b200_pointset **ou
     if (m >= UINT32_MAX) { g_err = "goldilocks_b200_pointset_create: at most 2^32 - 2 points"; return GOLDILOCKS_FAILURE; }
     const size_t mm = m + 1;
     const bool flat = keyset_flat(mm);
-    goldilocks_b200_pointset_s *ps = new goldilocks_b200_pointset_s{k.c->dev, m, nullptr, flat};
-    bool ok = cudaMalloc(&ps->ktabs, mm * (flat ? KSET_QUADS : KTAB_QUADS) * sizeof(uint4)) == cudaSuccess;
+    goldilocks_b200_pointset_s *ps = new goldilocks_b200_pointset_s{{k.c->dev, m}, nullptr, flat};
+    bool ok = ps->alloc(&ps->ktabs, mm * (flat ? KSET_QUADS : KTAB_QUADS));
     if (ok) {
         static const abi_pt identity = {{{0}}, {{1}}, {{1}}, {{0}}};
         abi_pt *pts = k.out<abi_pt>(mm);
@@ -1791,48 +1802,32 @@ goldilocks_error_t goldilocks_b200_pointset_create(goldilocks_b200_pointset **ou
              cudaMemcpyAsync(pts + m, &identity, sizeof(abi_pt), cudaMemcpyHostToDevice, k.c->stream) == cudaSuccess;
         if (ok) keyset_tables(k, pts, ps->ktabs, mm, flat);
     }
-    goldilocks_error_t r = k.finish();
-    if (!ok || r != GOLDILOCKS_SUCCESS) {
-        if (!ok) g_err = "goldilocks_b200_pointset_create: device allocation or copy failed";
-        cudaFree(ps->ktabs);
-        delete ps;
-        return GOLDILOCKS_FAILURE;
-    }
-    *out = ps;
-    return GOLDILOCKS_SUCCESS;
+    return finish_create(k, ok, ps, out, "goldilocks_b200_pointset_create: device allocation or copy failed");
 }
-void goldilocks_b200_pointset_destroy(goldilocks_b200_pointset *ps) {
-    if (!ps) return;
-    int cur = 0;
-    const bool sw = cudaGetDevice(&cur) == cudaSuccess && cur != ps->dev && cudaSetDevice(ps->dev) == cudaSuccess;
-    cudaFree(ps->ktabs);
-    if (sw) cudaSetDevice(cur);
-    delete ps;
-}
+void goldilocks_b200_pointset_destroy(goldilocks_b200_pointset *ps) { delete ps; }
 size_t goldilocks_b200_pointset_size(const goldilocks_b200_pointset *ps) { return ps ? ps->m : 0; }
 goldilocks_error_t goldilocks_448_base_double_scalarmul_non_secret_pointset_batch(hpt *out, const goldilocks_b200_pointset *ps, const uint32_t *point_index,
                                                                               const hsc *scalar1, const hsc *scalar2, size_t n) {
     if (n == 0) return GOLDILOCKS_SUCCESS;
     Call k;
     if (!k.ok) return k.finish();
-    if (!ps || ps->dev != k.c->dev) { g_err = "goldilocks_448_base_double_scalarmul_non_secret_pointset_batch: the point set lives on another device"; return GOLDILOCKS_FAILURE; }
-    if (n > (size_t)INT32_MAX) { g_err = "goldilocks_448_base_double_scalarmul_non_secret_pointset_batch: n >= 2^31"; return GOLDILOCKS_FAILURE; }
+    if (!set_call(ps, k.c->dev, "goldilocks_448_base_double_scalarmul_non_secret_pointset_batch", n)) return GOLDILOCKS_FAILURE;
     abi_pt *dout = k.out<abi_pt>(n);
     const uint32_t *didx = k.in(point_index, n);
     const abi_sc *ds1 = k.in(S(scalar1), n), *ds2 = k.in(S(scalar2), n);
-    DecafPeerScratch s;
-    decaf_peer_scratch(&s, k.alloc(decaf_peer_scratch(nullptr, nullptr, n)), n);
+    OrderScratch s;
+    order_scratch(&s, k.alloc(order_scratch(nullptr, nullptr, n)), n);
     if (k.ok) k.ok = pointset_enqueue(*k.c, dout, ps, didx, ds1, ds2, n, s, k.c->stream, nullptr);
     k.fetch(P(out), dout, n);
     return k.finish();
 }
 
 // ---- key-set lookup: verification by public-key bytes against a key set, the keys outside it through the ordinary path --------
-// Looked-up index per element (LaneKeysetLookup) -> the order of the decaf peer sets (hits grouped by key, the misses as one tail)
+// Looked-up index per element (LaneKeysetLookup) -> the sets' order (hits grouped by key, the misses as one tail)
 // -> the miss count, read back once -> the hits through the ordered key-set finish kernel, the misses packed and through verify_dev
 // unchanged -> every status scattered back to its element.
 struct KeysetLookupScratch {
-    DecafPeerScratch peer;
+    OrderScratch sort;
     uint32_t *idx, *hits;
     abi_sc *chal, *resp;
     verify_aux *aux;
@@ -1848,9 +1843,9 @@ static size_t keyset_lookup_scratch(KeysetLookupScratch *s, void *base, size_t n
     char *p = (char *)base;
     size_t used = 0;
     auto take = [&](size_t bytes) { void *r = p ? p + used : nullptr; used += al(bytes); return r; };
-    DecafPeerScratch peer;
-    void *pb = take(decaf_peer_scratch(nullptr, nullptr, n));
-    if (s) decaf_peer_scratch(&peer, pb, n);
+    OrderScratch sort;
+    void *pb = take(order_scratch(nullptr, nullptr, n));
+    if (s) order_scratch(&sort, pb, n);
     uint32_t *idx = (uint32_t *)take(sizeof(uint32_t) * n), *hits = (uint32_t *)take(sizeof(uint32_t));
     abi_sc *chal = (abi_sc *)take(sizeof(abi_sc) * n), *resp = (abi_sc *)take(sizeof(abi_sc) * n);
     verify_aux *aux = (verify_aux *)take(sizeof(verify_aux) * n);
@@ -1862,7 +1857,7 @@ static size_t keyset_lookup_scratch(KeysetLookupScratch *s, void *base, size_t n
     void *verify = take(verify_core_scratch_bytes(n));
     uint4 *slots = (uint4 *)take(verify_slot_bytes(g, n));
     uint8_t *msg2 = (uint8_t *)take(msg_bytes);
-    if (s) *s = {peer, idx, hits, chal, resp, aux, st, sig2, pk2, len, off2, scan_tmp, scan_bytes, verify, slots, msg2};
+    if (s) *s = {sort, idx, hits, chal, resp, aux, st, sig2, pk2, len, off2, scan_tmp, scan_bytes, verify, slots, msg2};
     return used;
 }
 /* the first half: looked-up indices into idx, the order, the number of hits on the host (synchronises st) */
@@ -1870,8 +1865,8 @@ static bool keyset_lookup_order(Ctx &c, uint32_t *idx, const goldilocks_b200_key
                                 cudaStream_t st, size_t *hits) {
     const uint32_t m = (uint32_t)ks->m;
     LaneKeysetLookup fl = {idx, pk, ks->pk, ks->sorted, m};
-    if (!launch(c, fl, n, st) || !peer_order(c, idx, m, n, s.peer, st, "pair_sort (key set lookup)")) return false;
-    LaneKeysetHits fh = {s.hits, s.peer.keys_s, m, n};
+    if (!launch(c, fl, n, st) || !set_order(c, idx, m, n, s.sort, st, "pair_sort (key set lookup)")) return false;
+    LaneKeysetHits fh = {s.hits, s.sort.keys_s, m, n};
     if (!launch(c, fh, n, st)) return false;
     uint32_t h = 0;
     CU(cudaMemcpyAsync(&h, s.hits, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
@@ -1886,28 +1881,24 @@ static bool keyset_lookup_verify(Ctx &c, int32_t *status, const goldilocks_b200_
     if (hits) {
         LaneEdVerifyScalars f2 = {s.chal, s.resp, sig, pk, msg, off, prehashed, ctx, ctx_len, 0};   /* a hit's key bytes are its set key's */
         if (!launch(c, f2, n, st)) return false;
-        int grid = 1;
-        if (ks->flat) {
-            SlotEdVerifyFinishKeysetOrdered<true> f3 = {s.aux, ks->key_ok, s.chal, s.resp, c.wide, ks->ktabs, idx, s.peer.order, sig};
-            if (!smp_grid<SlotEdVerifyFinishKeysetOrdered<true>>(c, &grid) || !launch_smp(c, f3, hits, grid, st, counter)) return false;
-        } else {
-            SlotEdVerifyFinishKeysetOrdered<false> f3 = {s.aux, ks->key_ok, s.chal, s.resp, c.wide, ks->ktabs, idx, s.peer.order, sig};
-            if (!smp_grid<SlotEdVerifyFinishKeysetOrdered<false>>(c, &grid) || !launch_smp(c, f3, hits, grid, st, counter)) return false;
-        }
+        if (!launch_layout(c, ks->flat, hits, st, counter, [&](auto flat) {
+                return SlotEdVerifyFinishKeysetOrdered<decltype(flat)::value>{s.aux, ks->key_ok, s.chal, s.resp, c.wide, ks->ktabs, idx, s.sort.order, sig};
+            }))
+            return false;
         LaneVerifySign fv = {s.st, s.aux, 1, hits};
         if (!launch(c, fv, (hits + VSIGN_BATCH - 1) / VSIGN_BATCH, st)) return false;
     }
     const size_t misses = n - hits;
     if (misses) {
-        LaneKeysetMissLengths fl = {s.len, off, s.peer.order, hits, misses};
+        LaneKeysetMissLengths fl = {s.len, off, s.sort.order, hits, misses};
         if (!launch(c, fl, misses + 1, st)) return false;
         CU(length_scan(s.scan_tmp, s.scan_bytes, s.len, s.off2, misses + 1, st));
-        LaneKeysetMissGather fg = {s.sig2, s.pk2, s.msg2, s.off2, sig, pk, msg, off, s.peer.order, hits};
+        LaneKeysetMissGather fg = {s.sig2, s.pk2, s.msg2, s.off2, sig, pk, msg, off, s.sort.order, hits};
         if (!launch(c, fg, misses, st)) return false;
         if (!verify_dev(c, s.st + hits, s.sig2, s.pk2, s.msg2, s.off2, prehashed, ctx, ctx_len, misses, s.verify, s.slots, grids, st, nullptr, side, side_evt))
             return false;
     }
-    LaneKeysetScatter fs = {status, s.st, s.peer.order};
+    LaneKeysetScatter fs = {status, s.st, s.sort.order};
     return launch(c, fs, n, st);
 }
 goldilocks_error_t goldilocks_ed448_verify_keyset_lookup_batch(goldilocks_error_t *status, uint32_t *key_index, const goldilocks_b200_keyset *ks, const uint8_t *signature,
@@ -1916,8 +1907,7 @@ goldilocks_error_t goldilocks_ed448_verify_keyset_lookup_batch(goldilocks_error_
     if (n == 0) return GOLDILOCKS_SUCCESS;
     Call k;
     if (!k.ok) return k.finish();
-    if (!ks || ks->dev != k.c->dev) { g_err = "goldilocks_ed448_verify_keyset_lookup_batch: the key set lives on another device"; return GOLDILOCKS_FAILURE; }
-    if (n > (size_t)INT32_MAX) { g_err = "goldilocks_ed448_verify_keyset_lookup_batch: n >= 2^31"; return GOLDILOCKS_FAILURE; }
+    if (!set_call(ks, k.c->dev, "goldilocks_ed448_verify_keyset_lookup_batch", n)) return GOLDILOCKS_FAILURE;
     /* the keys first, as goldilocks_ed448_verify_batch: the lookup, the sort and the read-back of the miss count run while the
      * signatures and messages still cross PCIe on the copy stream */
     const size_t total = msg_off[n];
@@ -1971,45 +1961,35 @@ goldilocks_error_t goldilocks_x448_peerset_batch_dev(uint8_t *out, goldilocks_er
     if (n == 0) return GOLDILOCKS_SUCCESS;
     Ctx *c = dev_ctx();
     if (!c) return GOLDILOCKS_FAILURE;
-    if (!ps || ps->dev != c->dev) { g_err = "goldilocks_x448_peerset_batch_dev: the peer set lives on another device"; return GOLDILOCKS_FAILURE; }
+    if (!set_call(ps, c->dev, "goldilocks_x448_peerset_batch_dev")) return GOLDILOCKS_FAILURE;
     SlotX448Peer f = {out, (int32_t *)status, ps->tables, ps->table_ok, ps->peers, peer_index, scalar, (uint32_t)ps->m};
     return launch_slots(*c, f, n, as_stream(stream)) ? GOLDILOCKS_SUCCESS : GOLDILOCKS_FAILURE;
 }
-size_t goldilocks_b200_decaf_peerset_scratch_bytes(size_t n) {
-    if (!dev_ctx()) return 0;
-    return decaf_peer_scratch(nullptr, nullptr, n);
-}
+size_t goldilocks_b200_decaf_peerset_scratch_bytes(size_t n) { return order_scratch_bytes(n); }
 goldilocks_error_t goldilocks_448_direct_scalarmul_peerset_batch_dev(uint8_t *scaled, goldilocks_error_t *status, const goldilocks_b200_decaf_peerset *ps,
                                                                      const uint32_t *peer_index, const hsc *scalar, goldilocks_bool_t short_circuit, size_t n,
                                                                      void *scratch, void *stream) {
     if (n == 0) return GOLDILOCKS_SUCCESS;
     Ctx *c = dev_ctx();
     if (!c) return GOLDILOCKS_FAILURE;
-    if (!ps || ps->dev != c->dev) { g_err = "goldilocks_448_direct_scalarmul_peerset_batch_dev: the peer set lives on another device"; return GOLDILOCKS_FAILURE; }
-    if (n > (size_t)INT32_MAX) { g_err = "goldilocks_448_direct_scalarmul_peerset_batch_dev: n >= 2^31"; return GOLDILOCKS_FAILURE; }
-    if (!scratch) { g_err = "goldilocks_448_direct_scalarmul_peerset_batch_dev: no scratch"; return GOLDILOCKS_FAILURE; }
+    if (!set_call(ps, c->dev, "goldilocks_448_direct_scalarmul_peerset_batch_dev", n, scratch)) return GOLDILOCKS_FAILURE;
     /* everything the call writes besides scaled / status lives in the caller's scratch: calls on different streams do not interfere */
-    DecafPeerScratch s;
-    decaf_peer_scratch(&s, scratch, n);
+    OrderScratch s;
+    order_scratch(&s, scratch, n);
     return decaf_peer_enqueue(*c, scaled, (int32_t *)status, ps, peer_index, S(scalar), short_circuit != 0, n, s, as_stream(stream)) ? GOLDILOCKS_SUCCESS
                                                                                                                                       : GOLDILOCKS_FAILURE;
 }
-size_t goldilocks_b200_pointset_scratch_bytes(size_t n) {
-    if (!dev_ctx()) return 0;
-    return decaf_peer_scratch(nullptr, nullptr, n);
-}
+size_t goldilocks_b200_pointset_scratch_bytes(size_t n) { return order_scratch_bytes(n); }
 goldilocks_error_t goldilocks_448_base_double_scalarmul_non_secret_pointset_batch_dev(hpt *out, const goldilocks_b200_pointset *ps, const uint32_t *point_index,
                                                                                   const hsc *scalar1, const hsc *scalar2, size_t n, void *scratch, void *stream) {
     if (n == 0) return GOLDILOCKS_SUCCESS;
     Ctx *c = dev_ctx();
     if (!c) return GOLDILOCKS_FAILURE;
-    if (!ps || ps->dev != c->dev) { g_err = "goldilocks_448_base_double_scalarmul_non_secret_pointset_batch_dev: the point set lives on another device"; return GOLDILOCKS_FAILURE; }
-    if (n > (size_t)INT32_MAX) { g_err = "goldilocks_448_base_double_scalarmul_non_secret_pointset_batch_dev: n >= 2^31"; return GOLDILOCKS_FAILURE; }
-    if (!scratch) { g_err = "goldilocks_448_base_double_scalarmul_non_secret_pointset_batch_dev: no scratch"; return GOLDILOCKS_FAILURE; }
+    if (!set_call(ps, c->dev, "goldilocks_448_base_double_scalarmul_non_secret_pointset_batch_dev", n, scratch)) return GOLDILOCKS_FAILURE;
     /* the sort lives in the caller's scratch and the kernel takes a fixed grid-stride assignment (no hand-out counter of the
      * context): calls on different streams do not interfere */
-    DecafPeerScratch s;
-    decaf_peer_scratch(&s, scratch, n);
+    OrderScratch s;
+    order_scratch(&s, scratch, n);
     return pointset_enqueue(*c, P(out), ps, point_index, S(scalar1), S(scalar2), n, s, as_stream(stream), GRID_STRIDE) ? GOLDILOCKS_SUCCESS : GOLDILOCKS_FAILURE;
 }
 size_t goldilocks_b200_keyset_scratch_bytes(size_t n, size_t msg_bytes) {
@@ -2024,9 +2004,7 @@ goldilocks_error_t goldilocks_ed448_verify_keyset_batch_dev(goldilocks_error_t *
     if (n == 0) return GOLDILOCKS_SUCCESS;
     Ctx *c = dev_ctx();
     if (!c) return GOLDILOCKS_FAILURE;
-    if (!ks || ks->dev != c->dev) { g_err = "goldilocks_ed448_verify_keyset_batch_dev: the key set lives on another device"; return GOLDILOCKS_FAILURE; }
-    if (n > (size_t)INT32_MAX) { g_err = "goldilocks_ed448_verify_keyset_batch_dev: n >= 2^31"; return GOLDILOCKS_FAILURE; }
-    if (!scratch) { g_err = "goldilocks_ed448_verify_keyset_batch_dev: no scratch"; return GOLDILOCKS_FAILURE; }
+    if (!set_call(ks, c->dev, "goldilocks_ed448_verify_keyset_batch_dev", n, scratch)) return GOLDILOCKS_FAILURE;
     VerifyGrids grids;
     if (!verify_grids(*c, &grids)) return GOLDILOCKS_FAILURE;
     KeysetLookupScratch s = {};
@@ -2041,9 +2019,7 @@ goldilocks_error_t goldilocks_ed448_verify_keyset_lookup_batch_dev(goldilocks_er
     if (n == 0) return GOLDILOCKS_SUCCESS;
     Ctx *c = dev_ctx();
     if (!c) return GOLDILOCKS_FAILURE;
-    if (!ks || ks->dev != c->dev) { g_err = "goldilocks_ed448_verify_keyset_lookup_batch_dev: the key set lives on another device"; return GOLDILOCKS_FAILURE; }
-    if (n > (size_t)INT32_MAX) { g_err = "goldilocks_ed448_verify_keyset_lookup_batch_dev: n >= 2^31"; return GOLDILOCKS_FAILURE; }
-    if (!scratch) { g_err = "goldilocks_ed448_verify_keyset_lookup_batch_dev: no scratch"; return GOLDILOCKS_FAILURE; }
+    if (!set_call(ks, c->dev, "goldilocks_ed448_verify_keyset_lookup_batch_dev", n, scratch)) return GOLDILOCKS_FAILURE;
     VerifyGrids grids;
     if (!verify_grids(*c, &grids)) return GOLDILOCKS_FAILURE;
     KeysetLookupScratch s = {};

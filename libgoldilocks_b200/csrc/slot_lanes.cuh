@@ -1,6 +1,7 @@
 // slot_lanes.cuh -- functors of the slot-machine kernels (slots.cuh): `operator()(i, base)` processes
 // element i with this lane's shared-memory slots starting at handle `base`.
 #pragma once
+#include <type_traits>
 #include "lanes.cuh"
 #include "slot_algos.cuh"
 #include "verify_plan.cuh"
@@ -335,6 +336,9 @@ struct SlotEdVerifyFinishKeyset { /* signature i under key key_index[i] of the s
         s_verify_accept_prep(aux + i, sb, sig + 114 * i, (gmask_t)key_ok[t]);
     }
 };
+/* the finish kernel of a set's layout, for host code that picks it with one flag (both keep their own kernel names) */
+template <bool FLAT>
+using SlotEdVerifyFinishKeysetLayout = std::conditional_t<FLAT, SlotEdVerifyFinishKeysetFlat, SlotEdVerifyFinishKeyset>;
 // Key-set lookup calls (goldilocks_ed448_verify_keyset_lookup_batch; DESIGN.md decision 23): lane j < hits verifies element
 // i = order[j] (the batch sorted by looked-up key, so the lanes of a warp read one or two tables) under key key_index[i] < m of a
 // set of either layout, with the evaluations of the two kernels above, and leaves its aux record at aux[j].
