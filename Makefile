@@ -1,6 +1,6 @@
 # Builds the product library (CUDA, sm_100a only) and the test-only artefacts.
 #   make lib       -> libgoldilocks_b200/libgoldilocks_b200.so   (the C ABI of include/goldilocks_b200.h)
-#   make hostsim   -> tests/hostsim/_hostsim.so, _hostsim_peerset.so, _hostsim_decaf_peerset.so, _hostsim_pointset.so, _hostsim_keyset_lookup.so (device math compiled for the host; tests only)
+#   make hostsim   -> tests/hostsim/_hostsim.so, _hostsim_peerset.so, _hostsim_decaf_peerset.so, _hostsim_pointset.so, _hostsim_keyset_lookup.so, _hostsim_peerset_lookup.so (device math compiled for the host; tests only)
 #   make oracle    -> oracle/liboracle.so (+ oracle/_ref/*.so with REF=<libgoldilocks source tree>; tests/bench baseline only)
 NVCC      ?= nvcc
 CXX       ?= g++
@@ -29,7 +29,8 @@ $(OBJDIR)/%.o: $(CSRC)/%.cu $(HDRS_$*) $(HDRS)
 $(LIB): $(OBJS)
 	$(NVCC) $(ARCH) -shared -cudart static -o $@ $(OBJS)
 
-hostsim: tests/hostsim/_hostsim.so tests/hostsim/_hostsim_peerset.so tests/hostsim/_hostsim_decaf_peerset.so tests/hostsim/_hostsim_pointset.so tests/hostsim/_hostsim_keyset_lookup.so
+hostsim: tests/hostsim/_hostsim.so tests/hostsim/_hostsim_peerset.so tests/hostsim/_hostsim_decaf_peerset.so tests/hostsim/_hostsim_pointset.so tests/hostsim/_hostsim_keyset_lookup.so \
+         tests/hostsim/_hostsim_peerset_lookup.so
 tests/hostsim/_hostsim.so: tests/hostsim/hostsim.cpp $(HDRS)
 	$(CXX) -std=c++17 -O2 -fPIC -shared -DGF_CHECK_BOUNDS -DGF_COUNT_OPS -o $@ $< -lpthread
 tests/hostsim/_hostsim_peerset.so: tests/hostsim/peerset.cpp $(HDRS)
@@ -40,10 +41,12 @@ tests/hostsim/_hostsim_pointset.so: tests/hostsim/pointset.cpp $(HDRS)
 	$(CXX) -std=c++17 -O2 -fPIC -shared -DGF_CHECK_BOUNDS -DGF_COUNT_OPS -o $@ $< -lpthread
 tests/hostsim/_hostsim_keyset_lookup.so: tests/hostsim/keyset_lookup.cpp tests/hostsim/hostsim.cpp $(HDRS)
 	$(CXX) -std=c++17 -O2 -fPIC -shared -DGF_CHECK_BOUNDS -DGF_COUNT_OPS -o $@ $< -lpthread
+tests/hostsim/_hostsim_peerset_lookup.so: tests/hostsim/peerset_lookup.cpp tests/hostsim/peerset.cpp $(HDRS)
+	$(CXX) -std=c++17 -O2 -fPIC -shared -DGF_CHECK_BOUNDS -DGF_COUNT_OPS -o $@ $< -lpthread
 
 oracle:
 	$(MAKE) -C oracle all
 
 clean:
-	rm -rf build $(LIB) tests/hostsim/_hostsim.so tests/hostsim/_hostsim_peerset.so tests/hostsim/_hostsim_decaf_peerset.so tests/hostsim/_hostsim_pointset.so tests/hostsim/_hostsim_keyset_lookup.so
+	rm -rf build $(LIB) tests/hostsim/_hostsim.so tests/hostsim/_hostsim_peerset.so tests/hostsim/_hostsim_decaf_peerset.so tests/hostsim/_hostsim_pointset.so tests/hostsim/_hostsim_keyset_lookup.so tests/hostsim/_hostsim_peerset_lookup.so
 	$(MAKE) -C oracle clean

@@ -280,13 +280,31 @@ GOLDILOCKS_B200_API goldilocks_error_t goldilocks_ed448_verify_keyset_lookup_bat
  * exactly what goldilocks_x448(out, peers[peer_index[i]], scalar + 56 i) returns; peer_index[i] >= m yields FAILURE and 56 zero
  * bytes.  Constant time in the scalars; the peer indices are public.  The handle belongs to the CUDA device that was current at
  * creation and is never sharded over goldilocks_b200_set_devices.  Order a batch by peer: the lanes of a
- * warp then read one table (with many peers in random order goldilocks_x448_batch's ladder is faster; DESIGN.md decision 20). */
+ * warp then read one table (with many peers in random order goldilocks_x448_batch's ladder is faster; DESIGN.md decision 20).
+ * goldilocks_x448_peerset_lookup_batch below takes the peers' bytes and orders the batch on the device. */
 typedef struct goldilocks_b200_x448_peerset_s goldilocks_b200_x448_peerset;
 GOLDILOCKS_B200_API goldilocks_error_t goldilocks_b200_x448_peerset_create(goldilocks_b200_x448_peerset **set, const uint8_t *peers /*m*56*/, size_t m);
 GOLDILOCKS_B200_API void goldilocks_b200_x448_peerset_destroy(goldilocks_b200_x448_peerset *set);
 GOLDILOCKS_B200_API size_t goldilocks_b200_x448_peerset_size(const goldilocks_b200_x448_peerset *set);
 GOLDILOCKS_B200_API goldilocks_error_t goldilocks_x448_peerset_batch(uint8_t *out /*n*56*/, goldilocks_error_t *status, const goldilocks_b200_x448_peerset *set,
                                                                      const uint32_t *peer_index /*n*/, const uint8_t *scalar /*n*56*/, size_t n);
+/* X448 against a peer set by the peer's bytes (our extension; DESIGN.md decision 24): the arguments of goldilocks_x448_batch plus a
+ * peer set, for a caller that holds each peer's 56 public bytes rather than its index in the set.
+ *   Results: out[i], status[i] are exactly what goldilocks_x448(out, base + 56 i, scalar + 56 i) returns, for every i and any 56 bytes.
+ *   Lookup: by raw bytes.  peer_index (may be NULL) receives, per element, the lowest set index whose 56 bytes equal base + 56 i, or m
+ *   when there is none.  A u of the set encoded differently (u + p) misses and takes the ladder; its result is still goldilocks_x448's.
+ *   Duplicate peers are allowed, an empty set is valid (every element misses), n = 0 succeeds, n < 2^31.  The search runs over the
+ *   set's peers in byte order (kept by goldilocks_b200_x448_peerset_create, 4 bytes per peer), so its cost does not depend on which
+ *   peers the set holds.
+ *   Work: the call orders the batch by looked-up peer on the device (a radix sort of the indices, never of the scalars), so the lanes
+ *   of a warp read one table whatever order the caller used; hits on peers with a comb table run the comb, every other element the
+ *   ladder, in the same launch.
+ *   Timing: constant time in the scalars; the bytes, the indices and the order are public.
+ *   Devices: the handle belongs to the CUDA device that was current at creation (another device gets FAILURE) and is never sharded
+ *   over goldilocks_b200_set_devices. */
+GOLDILOCKS_B200_API goldilocks_error_t goldilocks_x448_peerset_lookup_batch(uint8_t *out /*n*56*/, goldilocks_error_t *status, uint32_t *peer_index /*n, or NULL*/,
+                                                                            const goldilocks_b200_x448_peerset *set, const uint8_t *base /*n*56*/,
+                                                                            const uint8_t *scalar /*n*56*/, size_t n);
 /* Decaf peer sets (our extension): the same idea for goldilocks_448_direct_scalarmul, the decaf Diffie-Hellman.  A set of m
  * peer encodings is decoded once under allow_identity, and each peer gets the reference's (5,5,18) comb table (15 KB per peer
  * in HBM), so a multiplication against it costs a comb instead of a decode and a window multiplication.  scaled[i], status[i]
@@ -379,6 +397,16 @@ GOLDILOCKS_B200_API goldilocks_error_t goldilocks_ed448_verify_rlc_batch_dev(gol
 GOLDILOCKS_B200_API goldilocks_error_t goldilocks_x448_batch_dev(uint8_t *out, goldilocks_error_t *status, const uint8_t *base, const uint8_t *scalar, size_t n, void *stream);
 GOLDILOCKS_B200_API goldilocks_error_t goldilocks_x448_peerset_batch_dev(uint8_t *out, goldilocks_error_t *status, const goldilocks_b200_x448_peerset *set,
                                                                          const uint32_t *peer_index, const uint8_t *scalar, size_t n, void *stream);
+/* scratch of a device-resident X448 peer-set lookup call: the looked-up indices, the sort keys, the order and the sort's temporary
+ * storage, about 20 bytes per element.  It holds public data only (indices and order), so it needs no wipe; the secrets stay in
+ * out and scalar.  Returns 0 without a usable GPU. */
+GOLDILOCKS_B200_API size_t goldilocks_b200_x448_peerset_scratch_bytes(size_t n);
+/* device-pointer form of goldilocks_x448_peerset_lookup_batch; scratch >= goldilocks_b200_x448_peerset_scratch_bytes(n).  Fully
+ * asynchronous on `stream`: unlike goldilocks_ed448_verify_keyset_lookup_batch_dev it never synchronises it.  It writes only into
+ * scratch, out, status and peer_index, so calls in flight on different streams with different scratch buffers are independent. */
+GOLDILOCKS_B200_API goldilocks_error_t goldilocks_x448_peerset_lookup_batch_dev(uint8_t *out, goldilocks_error_t *status, uint32_t *peer_index /*or NULL*/,
+                                                                                const goldilocks_b200_x448_peerset *set, const uint8_t *base, const uint8_t *scalar,
+                                                                                size_t n, void *scratch, void *stream);
 /* scratch of a device-resident decaf peer-set call: the sort keys, the order and the sort's temporary storage, about 16 bytes
  * per element.  The call writes only there and into scaled / status, so calls in flight on different streams with different
  * scratch buffers are independent.  Returns 0 without a usable GPU. */

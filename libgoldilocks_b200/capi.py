@@ -365,6 +365,16 @@ class BatchLib:
         self._call("goldilocks_x448_peerset_batch", out, st, handle, peer_index, scalar, _Z(len(scalar)))
         return out, st
 
+    def x448_peerset_lookup(self, handle, base, scalar, return_index=False):
+        """(out (n,56) u8, status int32[n]) of X448 of scalar i against base i ((n,56) u8), exactly goldilocks_x448's; peers found in
+        the set by their bytes use its tables, the rest the ladder.  With return_index: (out, status, peer_index uint32[n]), the
+        lowest set index whose 56 bytes equal base[i], or m"""
+        base, scalar = _u8(base, 56), _u8(scalar, 56)
+        out = np.empty_like(scalar); st = np.zeros(len(scalar), np.int32)
+        idx = np.zeros(len(scalar), np.uint32) if return_index else None
+        self._call("goldilocks_x448_peerset_lookup_batch", out, st, idx, handle, base, scalar, _Z(len(scalar)))
+        return (out, st, idx) if return_index else (out, st)
+
     # ---- decaf peer sets: per-peer comb tables for direct_scalarmul against recurring points ----
     def decaf_peerset_create(self, encodings, allow_identity=False):
         """handle for m peer encodings ((m,56) u8) decoded under allow_identity; free it with decaf_peerset_destroy"""

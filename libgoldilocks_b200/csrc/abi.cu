@@ -1685,6 +1685,7 @@ struct goldilocks_b200_x448_peerset_s : DeviceSet {
     uint8_t *peers;     /* m x 56 u bytes: what the ladder reads for the peers that keep it */
     int32_t *table_ok;  /* per peer: SUCCESS = the comb table is valid (public) */
     niels *tables;      /* m tables of COMB_ENTRIES affine niels, 15 360 bytes each */
+    uint32_t *sorted;   /* the m indices ordered by peer bytes (memcmp), ties by index: the lookup calls' binary search (LaneX448PeerLookup) */
 };
 goldilocks_error_t goldilocks_b200_x448_peerset_create(goldilocks_b200_x448_peerset **out, const uint8_t *peers, size_t m) {
     if (!out) return GOLDILOCKS_FAILURE;
@@ -1692,14 +1693,21 @@ goldilocks_error_t goldilocks_b200_x448_peerset_create(goldilocks_b200_x448_peer
     Call k;
     if (!k.ok) return k.finish();
     const size_t mm = m ? m : 1;
-    goldilocks_b200_x448_peerset_s *ps = new goldilocks_b200_x448_peerset_s{{k.c->dev, m}, nullptr, nullptr, nullptr};
-    bool ok = m <= UINT32_MAX && ps->alloc(&ps->peers, 56 * mm) && ps->alloc(&ps->table_ok, mm) && ps->alloc(&ps->tables, mm * COMB_ENTRIES);
+    goldilocks_b200_x448_peerset_s *ps = new goldilocks_b200_x448_peerset_s{{k.c->dev, m}, nullptr, nullptr, nullptr, nullptr};
+    bool ok = m <= UINT32_MAX && ps->alloc(&ps->peers, 56 * mm) && ps->alloc(&ps->table_ok, mm) && ps->alloc(&ps->tables, mm * COMB_ENTRIES) &&
+              ps->alloc(&ps->sorted, mm);
+    std::vector<uint32_t> sorted;   /* lives until finish_create has synchronised the copy from it */
     if (ok && m) {
         ok = cudaMemcpyAsync(ps->peers, peers, 56 * m, cudaMemcpyHostToDevice, k.c->stream) == cudaSuccess;
         abi_pt *pts = k.out<abi_pt>(m);
         LaneX448PeerLift fl = {pts, ps->table_ok, ps->peers};
         k.run(fl, m);
         comb_tables(k, pts, ps->tables, m);
+        /* the byte order for the lookup calls, sorted on the host while the lift and the tables run (as goldilocks_b200_keyset_create) */
+        sorted.resize(m);
+        for (size_t i = 0; i < m; i++) sorted[i] = (uint32_t)i;
+        std::stable_sort(sorted.begin(), sorted.end(), [peers](uint32_t a, uint32_t b) { return memcmp(peers + 56 * (size_t)a, peers + 56 * (size_t)b, 56) < 0; });
+        ok = ok && cudaMemcpyAsync(ps->sorted, sorted.data(), sizeof(uint32_t) * m, cudaMemcpyHostToDevice, k.c->stream) == cudaSuccess;
     }
     return finish_create(k, ok, ps, out, "goldilocks_b200_x448_peerset_create: device allocation or copy failed");
 }
@@ -1716,6 +1724,43 @@ goldilocks_error_t goldilocks_x448_peerset_batch(uint8_t *out, goldilocks_error_
     k.run_sm(f, n);
     k.fetch(out, f.out, 56 * n);
     k.fetch((int32_t *)status, f.status, n);
+    return k.finish();
+}
+
+/* X448 against the set by the peers' bytes: looked-up indices into idx (LaneX448PeerLookup), the batch ordered by them (hits grouped
+ * by peer, the misses as one tail), then one kernel in which the hits with a table run its comb and everything else the ladder.
+ * No read-back: the misses need no packing, so the call stays asynchronous. */
+static size_t x448_peer_lookup_scratch(OrderScratch *s, uint32_t **idx, void *base, size_t n) {
+    const size_t order_bytes = order_scratch(s, base, n);
+    if (idx) *idx = (uint32_t *)((char *)base + order_bytes);
+    return order_bytes + ((sizeof(uint32_t) * n + 255) & ~(size_t)255);
+}
+static bool x448_peer_lookup_enqueue(Ctx &c, uint8_t *out, int32_t *status, uint32_t *idx, const goldilocks_b200_x448_peerset_s *ps, const uint8_t *base,
+                                     const uint8_t *scalar, size_t n, const OrderScratch &s, cudaStream_t st) {
+    const uint32_t m = (uint32_t)ps->m;
+    LaneX448PeerLookup fl = {idx, base, ps->peers, ps->sorted, m};
+    if (!launch(c, fl, n, st) || !set_order(c, idx, m, n, s, st, "pair_sort (X448 peer set lookup)")) return false;
+    SlotX448PeerLookup f = {out, status, ps->tables, ps->table_ok, idx, s.order, base, scalar, m};
+    return launch_slots(c, f, n, st);
+}
+goldilocks_error_t goldilocks_x448_peerset_lookup_batch(uint8_t *out, goldilocks_error_t *status, uint32_t *peer_index, const goldilocks_b200_x448_peerset *ps,
+                                                        const uint8_t *base, const uint8_t *scalar, size_t n) {
+    if (n == 0) return GOLDILOCKS_SUCCESS;
+    Call k;
+    if (!k.ok) return k.finish();
+    if (!set_call(ps, k.c->dev, "goldilocks_x448_peerset_lookup_batch", n)) return GOLDILOCKS_FAILURE;
+    uint8_t *dout = k.secret(k.out<uint8_t>(56 * n), 56 * n);
+    int32_t *dst = k.out<int32_t>(n);
+    const uint8_t *dbase = k.in(base, 56 * n);
+    const uint8_t *dsc = k.secret(k.in(scalar, 56 * n), 56 * n);
+    OrderScratch s = {};
+    uint32_t *idx = nullptr;
+    void *scratch = k.alloc(x448_peer_lookup_scratch(nullptr, nullptr, nullptr, n));
+    if (k.ok) x448_peer_lookup_scratch(&s, &idx, scratch, n);
+    if (k.ok) k.ok = x448_peer_lookup_enqueue(*k.c, dout, dst, idx, ps, dbase, dsc, n, s, k.c->stream);
+    k.fetch(out, dout, 56 * n);
+    k.fetch((int32_t *)status, dst, n);
+    if (peer_index) k.fetch(peer_index, idx, n);
     return k.finish();
 }
 
@@ -1964,6 +2009,21 @@ goldilocks_error_t goldilocks_x448_peerset_batch_dev(uint8_t *out, goldilocks_er
     if (!set_call(ps, c->dev, "goldilocks_x448_peerset_batch_dev")) return GOLDILOCKS_FAILURE;
     SlotX448Peer f = {out, (int32_t *)status, ps->tables, ps->table_ok, ps->peers, peer_index, scalar, (uint32_t)ps->m};
     return launch_slots(*c, f, n, as_stream(stream)) ? GOLDILOCKS_SUCCESS : GOLDILOCKS_FAILURE;
+}
+size_t goldilocks_b200_x448_peerset_scratch_bytes(size_t n) { return dev_ctx() ? x448_peer_lookup_scratch(nullptr, nullptr, nullptr, n) : 0; }
+goldilocks_error_t goldilocks_x448_peerset_lookup_batch_dev(uint8_t *out, goldilocks_error_t *status, uint32_t *peer_index, const goldilocks_b200_x448_peerset *ps,
+                                                            const uint8_t *base, const uint8_t *scalar, size_t n, void *scratch, void *stream) {
+    if (n == 0) return GOLDILOCKS_SUCCESS;
+    Ctx *c = dev_ctx();
+    if (!c) return GOLDILOCKS_FAILURE;
+    if (!set_call(ps, c->dev, "goldilocks_x448_peerset_lookup_batch_dev", n, scratch)) return GOLDILOCKS_FAILURE;
+    /* everything the call writes besides out / status / peer_index lives in the caller's scratch: calls on different streams do not
+     * interfere, and nothing waits for the stream */
+    OrderScratch s;
+    uint32_t *idx = nullptr;
+    x448_peer_lookup_scratch(&s, &idx, scratch, n);
+    return x448_peer_lookup_enqueue(*c, out, (int32_t *)status, peer_index ? peer_index : idx, ps, base, scalar, n, s, as_stream(stream)) ? GOLDILOCKS_SUCCESS
+                                                                                                                                        : GOLDILOCKS_FAILURE;
 }
 size_t goldilocks_b200_decaf_peerset_scratch_bytes(size_t n) { return order_scratch_bytes(n); }
 goldilocks_error_t goldilocks_448_direct_scalarmul_peerset_batch_dev(uint8_t *scaled, goldilocks_error_t *status, const goldilocks_b200_decaf_peerset *ps,

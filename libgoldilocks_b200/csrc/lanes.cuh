@@ -638,28 +638,33 @@ struct LaneVerifySign {
         }
     }
 };
-// ---- key-set lookup (goldilocks_ed448_verify_keyset_lookup_batch; DESIGN.md decision 23).  Public data only, variable time.
-GD int key57_cmp(const uint8_t *a, const uint8_t *b) { /* memcmp order of two 57-byte keys */
-    for (int k = 0; k < 57; k++)
+// ---- set lookup by bytes (goldilocks_ed448_verify_keyset_lookup_batch, DESIGN.md decision 23; goldilocks_x448_peerset_lookup_batch,
+// decision 24).  Public data only, variable time.
+template <int W>
+GD int key_cmp(const uint8_t *a, const uint8_t *b) { /* memcmp order of two W-byte keys */
+    for (int k = 0; k < W; k++)
         if (a[k] != b[k]) return a[k] < b[k] ? -1 : 1;
     return 0;
 }
-// Lane j: key_index[j] = the lowest index of the set whose 57 bytes equal pk j, or m.  `sorted` holds the set's indices ordered by
-// key bytes, ties by index (made on the host at creation), so the lower bound of pk j in it is its lowest equal index.  A byte
+// Lane j: key_index[j] = the lowest index of the set whose W bytes equal key j, or m.  `sorted` holds the set's indices ordered by
+// key bytes, ties by index (made on the host at creation), so the lower bound of key j in it is its lowest equal index.  A byte
 // order rather than a hash order: ceil(log2 m) + 1 comparisons whatever keys the set holds.
-struct LaneKeysetLookup {
+template <int W>
+struct LaneSetLookup {
     uint32_t *key_index; const uint8_t *pk, *set_pk; const uint32_t *sorted; uint32_t m;
     GDM void operator()(size_t j) const {
-        const uint8_t *q = pk + 57 * j;
+        const uint8_t *q = pk + W * j;
         uint32_t lo = 0, hi = m;
         while (lo < hi) {
             const uint32_t mid = lo + (hi - lo) / 2;
-            if (key57_cmp(set_pk + 57 * (size_t)sorted[mid], q) < 0) lo = mid + 1;
+            if (key_cmp<W>(set_pk + W * (size_t)sorted[mid], q) < 0) lo = mid + 1;
             else hi = mid;
         }
-        key_index[j] = (lo < m && key57_cmp(set_pk + 57 * (size_t)sorted[lo], q) == 0) ? sorted[lo] : m;
+        key_index[j] = (lo < m && key_cmp<W>(set_pk + W * (size_t)sorted[lo], q) == 0) ? sorted[lo] : m;
     }
 };
+using LaneKeysetLookup = LaneSetLookup<57>;    /* Ed448 public keys of a key set */
+using LaneX448PeerLookup = LaneSetLookup<56>;  /* u-coordinates of an X448 peer set */
 // *hits = the number of sort keys below m (keys_s: the looked-up indices, clamped to m and sorted; LaneDecafPeerKeys).  One lane
 // writes: the first miss, or the last lane when there is none.
 struct LaneKeysetHits {

@@ -45,6 +45,7 @@ cudaError_t launch_lanes(const F &f, size_t n, cudaStream_t s) {
 #endif
 template <> struct slot_min_blocks<SlotX448> { static constexpr int value = 4; };
 template <> struct slot_min_blocks<SlotX448Peer> { static constexpr int value = 4; };
+template <> struct slot_min_blocks<SlotX448PeerLookup> { static constexpr int value = 4; };
 template <> struct slot_min_blocks<SlotNielsDebug> { static constexpr int value = 4; };
 template <> struct slot_min_blocks<SlotComb> { static constexpr int value = SLOT7_MIN_BLOCKS; };
 template <> struct slot_min_blocks<SlotX448DerivePk> { static constexpr int value = SLOT7_MIN_BLOCKS; };
@@ -114,9 +115,9 @@ cudaError_t launch_sm_persist(const F &f, size_t n, int grid, cudaStream_t s, un
     X(LaneEdSecretScalar) X(LaneEdSignExpand) X(LaneEdSignNonce) X(LaneEdSignFinish)   \
     X(LaneEdVerifyDecode) X(LaneEdVerifyScalars) X(LaneVerifySign) X(LaneVerifyHalf) X(LaneKeysetNormalize) X(LaneBuildTables) X(LaneBuildWide) \
     X(LaneRlcDecode) X(LaneRlcZ) X(LaneRlcWeights) X(LaneRlcLate) X(LaneRlcKeyScalars) X(LaneRlcDigits) X(LaneRlcBucketRuns) X(LaneRlcSegments) X(LaneRlcNodes) X(LaneRlcWindows) X(LaneRlcTotal) X(LaneRlcVerdict) X(LaneRlcPackPlan) X(LaneRlcPack) X(LaneRlcUnpack) X(LanePtNiels) \
-    X(LaneKeysetLookup) X(LaneKeysetHits) X(LaneKeysetMissLengths) X(LaneKeysetMissGather) X(LaneKeysetScatter)
+    X(LaneKeysetLookup) X(LaneX448PeerLookup) X(LaneKeysetHits) X(LaneKeysetMissLengths) X(LaneKeysetMissGather) X(LaneKeysetScatter)
 
-#define LANES_SM(X) X(SlotNielsDebug) X(SlotX448) X(SlotX448Peer) X(SlotComb) X(SlotCombTable) X(SlotDecafPeer) X(SlotX448DerivePk) X(SlotEdDerivePk) X(SlotEdSignR) X(SlotRlcBucket)
+#define LANES_SM(X) X(SlotNielsDebug) X(SlotX448) X(SlotX448Peer) X(SlotX448PeerLookup) X(SlotComb) X(SlotCombTable) X(SlotDecafPeer) X(SlotX448DerivePk) X(SlotEdDerivePk) X(SlotEdSignR) X(SlotRlcBucket)
 #define INSTANTIATE_SM(F) template cudaError_t launch_sm<F>(const F &, size_t, cudaStream_t);
 #define DECLARE_SM(F) extern INSTANTIATE_SM(F)
 #define LANES_SMP(X) X(SlotEdVerifyFinish) X(SlotEdVerifyFinishShared) X(SlotKeyChain) X(SlotKeyColumns) X(SlotKeysetTables) X(SlotKeysetChain) X(SlotKeysetColumns) X(SlotEdVerifyFinishKeyset) X(SlotEdVerifyFinishKeysetFlat) X(SlotPointset<true>) X(SlotPointset<false>) X(SlotEdVerifyFinishKeysetOrdered<true>) X(SlotEdVerifyFinishKeysetOrdered<false>) X(SlotBaseDoubleScalarmul) X(SlotScalarmul) X(SlotDoubleScalarmul) X(SlotDualScalarmul) X(SlotDirectScalarmul)

@@ -447,6 +447,21 @@ struct LaneX448PeerLift {
         table_ok[i] = ST_OK(ok);
     }
 };
+// The comb half of an X448 against a peer with a table: the scalar words ws clamped exactly as the ladder clamps them
+// (SlotX448DerivePk), k / 8 through table t of the set, and the fraction num / den = (y^2, x^2) of the result.
+GD void s_x448_peer_comb(sref num, sref den, uint32_t ws[14], sref sb, const niels *tables, uint32_t t) {
+    ws[0] &= ~3u;
+    ws[13] |= 0x80000000u;
+    sc s, h;
+    ByteAtWords at = {ws};
+    sc_decode_long(s, at, 56);
+    sc_halve(h, s);
+    sc_halve(s, h);
+    sc_halve(h, s);                                      /* k / 8 */
+    s_comb_scalarmul_table(sb, tables + (size_t)COMB_ENTRIES * t, h);
+    s_sqr(num, s_slot(sb, 1));
+    s_sqr(den, s_slot(sb, 0));
+}
 // Element i = goldilocks_x448(peers[peer_index[i]], scalar i): the comb over the peer's table or the ladder, by the peer's
 // public flag.  Both leave a fraction num / den -- (y^2, x^2) of the comb result (goldilocks.c:1104-1115 u = (y/x)^2), the
 // ladder's (x2, z2) -- and meet in ONE x448_finish, because its inversion is shared across the block (s_block_invert4) and
@@ -467,20 +482,39 @@ struct SlotX448Peer {
             s_st(num, z);
             s_st(den, z);
         } else if (table_ok[t]) {
-            ws[0] &= ~3u;
-            ws[13] |= 0x80000000u;                       /* clamped exactly as the ladder clamps (SlotX448DerivePk) */
-            sc s, h;
-            ByteAtWords at = {ws};
-            sc_decode_long(s, at, 56);
-            sc_halve(h, s);
-            sc_halve(s, h);
-            sc_halve(h, s);                              /* k / 8 */
-            s_comb_scalarmul_table(sb, tables + (size_t)COMB_ENTRIES * t, h);
-            s_sqr(num, s_slot(sb, 1));
-            s_sqr(den, s_slot(sb, 0));
+            s_x448_peer_comb(num, den, ws, sb, tables, t);
         } else {
             uint32_t wu[14];
             words_load56(wu, peers + 56 * (size_t)t);
+            x448_ladder_xz(num, den, wu, ws, sb);
+        }
+        const gmask_t nz = x448_finish(wo, sb, num, den);
+        if (!live) return;
+        words_store56(out + 56 * i, wo);
+        status[i] = ST_OK(nz);
+    }
+};
+// X448 against a peer set by the peer's bytes (goldilocks_x448_peerset_lookup_batch; DESIGN.md decision 24).  Lane j handles
+// element i = order[j] (the batch sorted by looked-up peer, LaneDecafPeerKeys: hits grouped by peer, the misses as one tail) in
+// place, with t = peer_index[i] (LaneX448PeerLookup: the lowest set index with base i's bytes, or m).  A hit on a peer with a
+// table runs its comb; every other element -- a miss, or a peer that keeps the ladder -- runs the ladder on its own base bytes,
+// which on a hit are the set's.  Both meet in the one x448_finish every lane has to reach, as in SlotX448Peer.
+struct SlotX448PeerLookup {
+    static constexpr int NSLOTS = 7;
+    static_assert(COMB_NSLOTS == NSLOTS && X448_NSLOTS == NSLOTS, "the comb and the ladder share the slots");
+    uint8_t *out; int32_t *status; const niels *tables; const int32_t *table_ok;
+    const uint32_t *peer_index, *order; const uint8_t *base, *scalar; uint32_t n_peers;
+    GDM void operator()(size_t j, sref sb, bool live) const {
+        const size_t i = order[j];
+        const uint32_t t = peer_index[i];
+        uint32_t ws[14], wo[14];
+        words_load56(ws, scalar + 56 * i);
+        sref num = s_slot(sb, 6), den = s_slot(sb, 5);
+        if (t < n_peers && table_ok[t]) {
+            s_x448_peer_comb(num, den, ws, sb, tables, t);
+        } else {
+            uint32_t wu[14];
+            words_load56(wu, base + 56 * i);
             x448_ladder_xz(num, den, wu, ws, sb);
         }
         const gmask_t nz = x448_finish(wo, sb, num, den);

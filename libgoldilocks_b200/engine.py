@@ -116,6 +116,19 @@ class DeviceEngine:
         self._call("goldilocks_x448_peerset_batch_dev", self._p(out), self._p(status), handle, self._p(peer_index), self._p(scalar),
                    _Z(status.numel()), self._stream())
 
+    def x448_peerset_scratch_bytes(self, n):
+        f = self.lib.goldilocks_b200_x448_peerset_scratch_bytes
+        f.restype = _Z
+        f.argtypes = [_Z]
+        return int(f(n))
+
+    def x448_peerset_lookup(self, out, status, peer_index, handle, base, scalar, scratch):
+        """goldilocks_x448_peerset_lookup_batch_dev: X448 of scalar i against base i, peers found in a set made by capi
+        x448_peerset_create by their bytes; peer_index (int32 tensor read as uint32, or None) receives the looked-up indices;
+        `scratch` holds x448_peerset_scratch_bytes(n).  Asynchronous on the current stream."""
+        self._call("goldilocks_x448_peerset_lookup_batch_dev", self._p(out), self._p(status), self._p(peer_index), handle, self._p(base), self._p(scalar),
+                   _Z(status.numel()), self._p(scratch), self._stream())
+
     def decaf_peerset_scratch_bytes(self, n):
         f = self.lib.goldilocks_b200_decaf_peerset_scratch_bytes
         f.restype = _Z

@@ -40,12 +40,12 @@ AUDITED = ["SlotX448", "SlotComb", "SlotCombTable", "SlotX448DerivePk", "SlotEdD
            "SlotDualScalarmul", "SlotDirectScalarmul", "LaneEdSignExpand", "LaneEdSignNonce", "LaneEdSignFinish", "LaneEdSecretScalar", "LaneEdSkToX448"]
 # secret-handling kernels of entry points the reference's API does not have (our extensions), reported as their own group,
 # one summary line per extension
-AUDITED_EXTENSIONS = ["SlotX448Peer", "SlotDecafPeer"]
-EXTENSION_NAMES = {"SlotX448Peer": "X448 peer-set", "SlotDecafPeer": "decaf peer-set"}
+AUDITED_EXTENSIONS = ["SlotX448Peer", "SlotX448PeerLookup", "SlotDecafPeer"]
+EXTENSION_NAMES = {"SlotX448Peer": "X448 peer-set", "SlotX448PeerLookup": "X448 peer-set lookup", "SlotDecafPeer": "decaf peer-set"}
 
 NEGATIVE_CONTROL = "SlotBaseDoubleScalarmul"
 
-NO_DEST = {"STG", "STS", "STL", "ST", "BRA", "BSSY", "BSYNC", "CALL", "EXIT", "RET", "NOP", "BAR", "RED", "WARPSYNC", "MEMBAR", "ERRBAR", "DEPBAR", "YIELD", "BMOV",
+NO_DEST = {"STG", "STS", "STL", "ST", "BRA", "BSSY", "BSYNC", "BREAK", "CALL", "EXIT", "RET", "NOP", "BAR", "RED", "WARPSYNC", "MEMBAR", "ERRBAR", "DEPBAR", "YIELD", "BMOV",
            "NANOSLEEP", "CCTL", "UBLKCP", "SYNCS"}
 PRED_ONLY_DEST = {"ISETP", "UISETP", "PLOP3", "UPLOP3", "FSETP", "DSETP", "PSETP", "UPSETP"}
 KNOWN = NO_DEST | PRED_ONLY_DEST | {"ATOMG", "CS2R", "FLO", "IADD3", "IMAD", "LDC", "LDCU", "LDG", "LDL", "LDS", "LEA", "LOP3", "MOV", "POPC", "PRMT", "S2R", "S2UR", "SEL", "SHF",
@@ -401,7 +401,8 @@ def audit_kernel(name, functor, ins_list, layout, verbose=False, trace=None):
                     st.dyn = (st.dyn[0] or tt, st.dyn[1] | pp)
         elif i.base in ("S2R", "S2UR", "CS2R"):
             t, p = guard_t, frozenset()
-        if record and (i.base in ("BRA", "EXIT", "RET") or i.base == "CALL"):
+        # BREAK: a predicated exit from a convergence region (BSSY ... BSYNC) -- control flow like a branch
+        if record and (i.base in ("BRA", "BREAK", "EXIT", "RET") or i.base == "CALL"):
             preds = [o.lstrip("!") for o in i.operands if is_pred(o)] + ([i.guard] if i.guard else [])
             preds = [q for q in preds if q not in ("PT", "UPT")]
             if preds:

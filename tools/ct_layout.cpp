@@ -31,6 +31,9 @@ int main() {
     K(SlotX448); FLD(SlotX448, out, "out"); FLD(SlotX448, status, "out"); FLD(SlotX448, base, "public"); FLD(SlotX448, scalar, "secret");
     K(SlotX448Peer); FLD(SlotX448Peer, out, "out"); FLD(SlotX448Peer, status, "out"); FLD(SlotX448Peer, tables, "public"); FLD(SlotX448Peer, table_ok, "public");
     FLD(SlotX448Peer, peers, "public"); FLD(SlotX448Peer, peer_index, "public"); FLD(SlotX448Peer, scalar, "secret"); FLD(SlotX448Peer, n_peers, "value");
+    K(SlotX448PeerLookup); FLD(SlotX448PeerLookup, out, "out"); FLD(SlotX448PeerLookup, status, "out"); FLD(SlotX448PeerLookup, tables, "public");
+    FLD(SlotX448PeerLookup, table_ok, "public"); FLD(SlotX448PeerLookup, peer_index, "public"); FLD(SlotX448PeerLookup, order, "public");
+    FLD(SlotX448PeerLookup, base, "public"); FLD(SlotX448PeerLookup, scalar, "secret"); FLD(SlotX448PeerLookup, n_peers, "value");
     K(SlotDecafPeer); FLD(SlotDecafPeer, scaled, "out"); FLD(SlotDecafPeer, status, "out"); FLD(SlotDecafPeer, tables, "public"); FLD(SlotDecafPeer, peer_ok, "public");
     FLD(SlotDecafPeer, peer_index, "public"); FLD(SlotDecafPeer, order, "public"); FLD(SlotDecafPeer, scalar, "secret"); FLD(SlotDecafPeer, n_peers, "value");
     FLD(SlotDecafPeer, short_circuit, "value");
